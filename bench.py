@@ -397,6 +397,28 @@ def measure_h2d_rate(torch, nbytes=1 << 30):
         return None
 
 
+DUMP_BUDGET_BYTES = 64 << 20
+
+
+def dump_outputs(directory, arrays):
+    """--dump-outputs: each array as DIR/<name>.npy in float64, so that two builds run with the same arguments (and
+    therefore the same seeded inputs) can be compared output for output. An array larger than its share of the 64 MB
+    budget is replaced by a fixed, seeded sample of its rows."""
+    os.makedirs(directory, exist_ok=True)
+    share = DUMP_BUDGET_BYTES // max(len(arrays), 1)
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64)
+        if a.nbytes > share:
+            rows = max(1, share // (a.nbytes // a.shape[0]))
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], rows, replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
+def log_array(log):
+    """Program.iteration_log() as an (iterations x 8) array, columns in the order of its keys."""
+    return np.array([list(row.values()) for row in log])
+
+
 def hbm_peak():
     try:
         peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))
@@ -405,8 +427,9 @@ def hbm_peak():
         return 6534.8, "B200_PROFILING.md fallback 6534.8 GB/s"
 
 
-def batched_bench(proc, args, w, cpu_leg):
-    """BASELINE config 3 on this process' share of the programs; returns the JSON dict on rank 0, None elsewhere."""
+def batched_bench(proc, args, w, steps, warmup, cpu_leg, outputs=None):
+    """BASELINE config 3 on this process' share of the programs; returns the JSON dict on rank 0, None elsewhere.
+    `outputs` (a dict) receives y of the timed solve, all programs."""
     from conex_b200.binding import Batch
     from conex_b200.workloads import add_cones, small_multicone_problem
     torch, dev, L, world, rank = proc.torch, proc.dev, proc.L, proc.world, proc.rank
@@ -426,57 +449,75 @@ def batched_bench(proc, args, w, cpu_leg):
     del programs
     setup_s = time.perf_counter() - t_setup
 
-    cfg = dev.default_config()
-    # warm-up solve (W >= 3 untimed Newton steps: one full solve is ~17), then the timed solve
-    batch.maximize(b, cfg)
+    # W warm-up + K timed lock steps in one solve, as the dense path times its Newton steps; without final centering
+    # every program takes a full Newton step in each of them
+    total = warmup + steps
+    cfg = dev.default_config(max_iterations=total, final_centering_steps=0, inv_sqrt_mu_max=1e12)
     proc.barrier()
     sampler = ClockSampler(proc.local_rank)
     sampler.start()
     launches0 = L.CONEXB200_LaunchCount()
-    t0 = time.perf_counter()
-    solved, y = batch.maximize(b, cfg)
+    _, y = batch.maximize(b, cfg)
     torch.cuda.synchronize()
-    e2e_wall = time.perf_counter() - t0
     launches = L.CONEXB200_LaunchCount() - launches0
     clocks = sampler.stop()
-    its, by, cx, _ = batch.results()
     step_ms = batch.step_milliseconds()
-    lock_steps = len(step_ms)
+    assert len(step_ms) == total, f"expected {total} lock steps, ran {len(step_ms)}"
+    timed = step_ms[warmup:]
+    its = batch.results()[0]
+    if outputs is not None:
+        if world > 1:
+            parts = [None] * world
+            proc.dist.all_gather_object(parts, y)
+            y = np.concatenate(parts)
+        outputs["y"] = y
+
+    # whole-solve throughput: a cold-start solve with the DEFAULT configuration, run to termination
+    proc.barrier()
+    t0 = time.perf_counter()
+    solved, _ = batch.maximize(b, dev.default_config())
+    torch.cuda.synchronize()
+    e2e_wall = time.perf_counter() - t0
+    solve_steps = len(batch.step_milliseconds())
     dev_ms = batch.milliseconds()
-    dev_ms, e2e_ms, mean_step_ms = proc.max_over_ranks([dev_ms, e2e_wall * 1e3, float(step_ms.mean())])
-    program_steps, nsolved, nprog = proc.sum_over_ranks([float(its.sum()), float(solved.sum()), float(hi - lo)])
+    timed_ms = float(timed.sum())
+    dev_ms, e2e_ms, timed_ms = proc.max_over_ranks([dev_ms, e2e_wall * 1e3, timed_ms])
+    program_steps, nsolved, nprog = proc.sum_over_ranks([float(np.clip(its - warmup, 0, steps).sum()),
+                                                         float(solved.sum()), float(hi - lo)])
     nsolved, nprog = int(nsolved), int(nprog)
     del batch
     proc.release()
     if rank != 0:
         return None
+    mean_step_ms = timed_ms / steps
     flops = batched_flops_per_program_step() * program_steps
     bytes_ = batched_bytes_per_program_step() * program_steps
     peak, peak_src = hbm_peak()
     line = {
-        "metric": METRIC, "value": mean_step_ms, "unit": UNIT, "n_gpus": world, "steps": lock_steps,
-        "warmup": lock_steps, "ms_per_step": mean_step_ms, "higher_is_better": False, "scaling": "strong",
+        "metric": METRIC, "value": mean_step_ms, "unit": UNIT, "n_gpus": world, "steps": steps,
+        "warmup": warmup, "ms_per_step": mean_step_ms, "higher_is_better": False, "scaling": "strong",
         "vs_baseline": None, "dtype": "f64", "data": "synthetic",
         "config": {"workload": w["name"], "programs": nprog, "m": 40,
                    "path": "CONEXB200_BatchMaximize: all programs advance one Newton step per launch set",
-                   "l2": "a full solve (cone data 1.6 GB per step) separates repeats",
+                   "l2": "cone data 1.6 GB per step vs 126 MB L2: no flush",
                    "multi_gpu": (f"programs partitioned over {world} ranks, no collective" if world > 1 else "n/a"),
-                   "step": "one lock-step Newton step of the whole batch (mean over the solve; programs that "
-                           "have terminated are masked out of later steps)"},
-        "solve_ms": dev_ms, "programs_per_s": nprog / (dev_ms * 1e-3), "programs_solved": nsolved,
-        "program_steps": program_steps,
-        "step_tflops_fp64": flops / (dev_ms * 1e-3) / 1e12,
+                   "step": "one lock-step Newton step of the whole batch (mean over the K timed steps that follow W "
+                           "warm-up steps of one solve without final centering)"},
+        "step_ms_per_step": [round(float(v), 4) for v in timed],
+        "solve_ms": dev_ms, "solve_lock_steps": solve_steps, "programs_per_s": nprog / (dev_ms * 1e-3),
+        "programs_solved": nsolved, "program_steps": program_steps,
+        "step_tflops_fp64": flops / (timed_ms * 1e-3) / 1e12,
         "roofline": {"bound": "hbm", "kernel": "whole lock step of the batch: PsdSchurMma2Kernel (DMMA, 66 % pipe-active under "
                                                "ncu, profiles/r02_m_c3_schur_ncu_full.txt) + the eigen-bound / step kernels",
-                     "achieved": bytes_ / (dev_ms * 1e-3) / 1e9, "peak": peak * world, "unit": "GB/s",
-                     "frac": bytes_ / (dev_ms * 1e-3) / 1e9 / (peak * world), "peak_source": peak_src,
-                     "note": "whole-solve time, all kernels; the same work is 2 flop/byte-balanced: "
-                             f"{flops / (dev_ms * 1e-3) / 1e12:.2f} TFLOP/s FP64 vs {proc.peak_tf:.1f} TFLOP/s cuBLAS DGEMM",
+                     "achieved": bytes_ / (timed_ms * 1e-3) / 1e9, "peak": peak * world, "unit": "GB/s",
+                     "frac": bytes_ / (timed_ms * 1e-3) / 1e9 / (peak * world), "peak_source": peak_src,
+                     "note": "time of the timed lock steps, all kernels; the same work is 2 flop/byte-balanced: "
+                             f"{flops / (timed_ms * 1e-3) / 1e12:.2f} TFLOP/s FP64 vs {proc.peak_tf:.1f} TFLOP/s cuBLAS DGEMM",
                      "traffic": None},
-        "e2e": {"value": e2e_ms / max(lock_steps, 1), "unit": UNIT, "solve_ms": e2e_ms,
-                "h2d_bytes_per_step": 8.0 * 40 * nprog / max(lock_steps, 1) + 8.0 * 6 * nprog,
-                "d2h_bytes_per_step": 8.0 * 40 * nprog / max(lock_steps, 1) + 8.0 * (2 * 6 * 4 + 6) * nprog,
-                "note": "CONEXB200_BatchMaximize from host b to host y (wall clock / lock steps)"},
+        "e2e": {"value": e2e_ms / max(solve_steps, 1), "unit": UNIT, "solve_ms": e2e_ms,
+                "h2d_bytes_per_step": 8.0 * 40 * nprog / max(solve_steps, 1) + 8.0 * 6 * nprog,
+                "d2h_bytes_per_step": 8.0 * 40 * nprog / max(solve_steps, 1) + 8.0 * (2 * 6 * 4 + 6) * nprog,
+                "note": "default-configuration CONEXB200_BatchMaximize from host b to host y (wall clock / lock steps)"},
         "gpu_launches": int(launches), "clocks": clocks, "setup_s": setup_s,
     }
     if cpu_leg:
@@ -494,9 +535,13 @@ def run_b200_batched(args):
         proc.L.cxb_set_small_cone_threads(args.small_cone_threads)
     if args.small_fused_launches >= 0:
         proc.L.cxb_set_small_fused_launches(args.small_fused_launches)
-    line = batched_bench(proc, args, workload_shape(args), cpu_leg=not args.no_cpu_baseline)
+    outputs = {} if args.dump_outputs else None
+    line = batched_bench(proc, args, workload_shape(args), args.steps, args.warmup, cpu_leg=not args.no_cpu_baseline,
+                         outputs=outputs)
     if line is not None:
         print(json.dumps(line))
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
     proc.close()
 
 
@@ -554,6 +599,7 @@ def run_b200_structured(args):
     torch.cuda.synchronize()
     wall = time.perf_counter() - t0
     launches = L.CONEXB200_LaunchCount() - launches0
+    outputs = {"y": y, "iteration_log": log_array(P.iteration_log())} if args.dump_outputs else None
     assert L.CONEXB200_ConstraintIsEntrySparse(P.h, cid.value) == 1
     its = P.status()["num_iterations"]
     ms = np.zeros(1)
@@ -618,6 +664,8 @@ def run_b200_structured(args):
         "final": {"by": log[-1]["by"], "cx": log[-1]["cx"], "mu": log[-1]["mu"]},
     }
     print(json.dumps(line))
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
 
 
 def arrow_flops(blocks, private, shared, n):
@@ -661,9 +709,11 @@ def run_b200_sparse(args):
         b = P.feasible_objective()
         cfg = dev.default_config(max_iterations=total, final_centering_steps=0, inv_sqrt_mu_max=1e12)
         launches0 = L.CONEXB200_LaunchCount()
-        P.maximize(b, cfg)
+        _, y = P.maximize(b, cfg)
         torch.cuda.synchronize()
         launches = L.CONEXB200_LaunchCount() - launches0
+        if name == "auto" and args.dump_outputs:
+            outputs = {"y": y, "iteration_log": log_array(P.iteration_log())}
         its = P.status()["num_iterations"]
         assert its == total, f"expected {total} Newton steps, ran {its}"
         ms = np.zeros(1)
@@ -718,6 +768,8 @@ def run_b200_sparse(args):
     if not args.no_cpu_baseline:
         line["cpu_baseline"] = cpu_baseline_sparse(w)
     print(json.dumps(line))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
 
 
 def cpu_baseline_sparse(w):
@@ -844,8 +896,9 @@ def executed_assembly_flops(form, n, m):
     return 3.0 * (m + 1) * n ** 3 + float(m) * (m + 1) * n ** 2
 
 
-def dense_bench(proc, args, w, steps, warmup, full_solve, cpu_leg):
-    """One dense-LMI workload (c1 / c2 / c4 / c5) on all ranks; returns the JSON dict on rank 0, None elsewhere."""
+def dense_bench(proc, args, w, steps, warmup, full_solve, cpu_leg, outputs=None):
+    """One dense-LMI workload (c1 / c2 / c4 / c5) on all ranks; returns the JSON dict on rank 0, None elsewhere.
+    `outputs` (a dict) receives y and the iteration log of the timed solve."""
     torch, dist, dev, L, world, rank = proc.torch, proc.dist, proc.dev, proc.L, proc.world, proc.rank
     n, m = w["n"], w["m"]
     fl = algorithmic_flops(n, m)
@@ -897,6 +950,9 @@ def dense_bench(proc, args, w, steps, warmup, full_solve, cpu_leg):
     timed = np.array(step_ms[warmup:])
     ph_timed = np.array(phases[warmup:]).mean(axis=0)
     log = P.iteration_log()
+    if outputs is not None:
+        outputs["y"] = y
+        outputs["iteration_log"] = log_array(log)
     form = L.CONEXB200_GetAssemblyForm(P.h, 0)
     shard = np.zeros(4)
     has_shard = L.CONEXB200_GetShardPhaseMilliseconds(P.h, 0, shard.ctypes.data_as(C.POINTER(C.c_double))) == 1
@@ -1040,23 +1096,31 @@ def run_b200(args):
     if args.gram_config >= -1:
         proc.L.cxb_set_gram_gemm_config(args.gram_config)
     w = workload_shape(args)
+    outputs = {} if args.dump_outputs else None
     line = dense_bench(proc, args, w, args.steps, args.warmup, full_solve=not args.no_full_solve,
-                       cpu_leg=not args.no_cpu_baseline and proc.rank == 0 and proc.world == 1)
+                       cpu_leg=not args.no_cpu_baseline and proc.rank == 0 and proc.world == 1, outputs=outputs)
     if args.workload == "c2" and not args.no_extra and not args.n and not args.m:
         # The other two shapes the north star quotes scaling on ride along in the same JSON line, so that the driver's
         # 1/2/4/8-GPU runs carry them: C5 (n = 1000, m = 20000; multi-GPU Cholesky on) and C3 (4096 small programs).
         # (a failure of a secondary block must not take the main line with it; every rank runs the same code on the
         # same shapes, so an exception is raised on all of them or on none)
+        # The outputs of a block go into the dump only when the block has returned a result.
+        c5_out = {} if outputs is not None else None
         try:
             c5w = workload_shape(argparse.Namespace(workload="c5", n=0, m=0, programs=0))
-            c5 = compact(dense_bench(proc, args, c5w, 2, 1, full_solve=False, cpu_leg=False))
+            c5 = compact(dense_bench(proc, args, c5w, 2, 1, full_solve=False, cpu_leg=False, outputs=c5_out))
             if c5 is not None and "error" not in c5:
-                c5["note"] = "1 warm-up + 2 timed Newton steps (a step is 1.3-14 s at this shape)"
+                c5["note"] = "1 warm-up + 2 timed Newton steps whatever --steps / --warmup ask (a step is 1.3-14 s at this shape)"
+                if outputs is not None:
+                    outputs.update({"c5_" + k: v for k, v in c5_out.items()})
         except Exception as e:  # noqa: BLE001
             c5 = {"error": f"{type(e).__name__}: {e}"}
+        c3_out = {} if outputs is not None else None
         try:
             c3w = workload_shape(argparse.Namespace(workload="c3", n=0, m=0, programs=0))
-            c3 = compact(batched_bench(proc, args, c3w, cpu_leg=False))
+            c3 = compact(batched_bench(proc, args, c3w, args.steps, args.warmup, cpu_leg=False, outputs=c3_out))
+            if outputs is not None:
+                outputs.update({"c3_" + k: v for k, v in c3_out.items()})
         except Exception as e:  # noqa: BLE001
             c3 = {"error": f"{type(e).__name__}: {e}"}
         if line is not None:
@@ -1064,14 +1128,17 @@ def run_b200(args):
             line["c3"] = c3
     if line is not None:
         print(json.dumps(line))
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
     proc.close()
 
 
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=5,
+                    help="timed Newton steps (c3: lock steps of the batch); the C5 block of the c2 line always times 2")
+    ap.add_argument("--warmup", type=int, default=3, help="untimed Newton steps before them (at least 3 on the B200 arm)")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="c2", choices=sorted(WORKLOADS),
                     help="BASELINE.json configuration (c2 = MaxCut n=2000, the headline)")
@@ -1095,7 +1162,12 @@ def main():
     ap.add_argument("--replicated-cholesky", action="store_true",
                     help="N > 1: factor the Schur complement on every rank instead of across the ranks")
     ap.add_argument("--cholesky-block", type=int, default=0, help="N > 1: block-column width (<= 512)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="B200 arm: after the timed steps, write what the timed solve returned (y, the iteration log; "
+                         "c2 also the C5 / C3 blocks as c5_*, c3_*) as DIR/<name>.npy in float64")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the B200 arm")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference(args)
