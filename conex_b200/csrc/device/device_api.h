@@ -19,15 +19,27 @@ int DgemmEx(cudaStream_t stream, int config, int splits, bool transA, bool trans
             double beta, double* C, long ldc, long sC, int batch, bool lower_only, bool mirror,
             int diag_off = 0);
 
-// Structured variant: tri bit 0 = op(B) is lower triangular (op(B)[k, c] = 0 for k < c), bit 1 = op(A)
-// is upper triangular (op(A)[r, k] = 0 for k < r) — k-tiles inside the zero part are skipped, the
-// stored zeros cover the rest; pack = the (square, lower_only) result is written as packed 64 x 64
+// What a structured GEMM knows about its operands (square, lower_only results; k-tiles inside the zero parts
+// are skipped, stored zeros cover the rest; always the 64 x 64 x 16 tile of configuration 2, no split-K):
+enum GemmStructure : int {
+  kGeneral = 0,
+  // C = alpha S B (A, B untransposed, beta = 0), S = tril(A, -1) + diag(A) / 2, B lower triangular with stored zeros
+  // above its diagonal. Only the lower triangle of A is ever part of the result (entries above it are selected
+  // away, not multiplied), so A may hold anything there. C is lower triangular; its diagonal tiles are stored
+  // whole, the strict upper part as exact zeros.
+  kHalfLowerTimesLower = 1,
+  // C = alpha (A^T B + B^T A) (transA, B untransposed, lda == ldb), A and B lower triangular with stored zeros
+  // above their diagonals inside the diagonal tiles; the diagonal tiles of C are computed whole.
+  kSyr2kLower = 2,
+};
+
+// Structured variant: see GemmStructure; pack = the (square, lower_only) result is written as packed 64 x 64
 // lower tiles, PackedSymmetricSize(n) doubles per matrix (stride sC), off-diagonal tiles scaled by
 // sqrt(2) so that the plain dot product of two packed symmetric matrices is their trace inner product.
 int DgemmStructured(cudaStream_t stream, int config, int splits, bool transA, bool transB, int M, int N,
                     int K, double alpha, const double* A, long lda, long sA, const double* B, long ldb,
                     long sB, double beta, double* C, long ldc, long sC, int batch, bool lower_only,
-                    bool mirror, int diag_off, int tri, bool pack);
+                    bool mirror, int diag_off, GemmStructure structure, bool pack);
 long PackedSymmetricSize(int n);
 
 // cholesky.cu: factors the block column [j0, j0 + w) x rows [j0, m) in place (w <= 512)

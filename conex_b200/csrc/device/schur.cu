@@ -42,14 +42,16 @@ __global__ void CopyLowerKernel(int n, const double* __restrict__ W, double* L) 
 
 // ---- symmetric form -----------------------------------------------------------------------------------
 // With W = L L^T:  H_ij = tr(A_i W A_j W) = <L^T A_i L, L^T A_j L>, so the Schur complement is the Gram
-// matrix of the scaled matrices S_i = L^T A_i L ("form W^{1/2} A_i W^{1/2}, then a SYRK-style Gram"):
-//   K1  T_i = A_i L            L lower triangular: k-tiles above the diagonal skipped   (n^3 flop)
-//       S_i = L^T T_i          symmetric: lower tiles only, L^T upper triangular        (n^3 / 3 flop)
+// matrix of the scaled matrices S_i = L^T A_i L ("form W^{1/2} A_i W^{1/2}, then a SYRK-style Gram").
+// K1 forms S_i in n^3 flops, as LAPACK's dsygst does, from A_i = V_i + V_i^T with V_i = tril(A_i, -1) + diag(A_i) / 2:
+//   K1  Y_i = V_i L            lower x lower = lower: lower tiles only, into dT             (n^3 / 3 flop)
+//       S_i = L^T Y_i + Y_i^T L  symmetric: lower tiles only, both products in one k loop (2 n^3 / 3 flop)
 //           stored as packed 64 x 64 lower tiles with sqrt(2)-scaled off-diagonal tiles, so that the
 //           plain dot product of two packed matrices is their trace inner product (K = 0.54 n^2)
 //   K2  Haug = X^T X (lower)   X = [S_0 .. S_{m-1}, L^T C L, I]: one DMMA SYRK-shaped GEMM
-// Rows m and m+1 of Haug are AQc_j = <L^T C L, S_j> and AW_j = tr(S_j) as before. Executed flops:
-// 1.33 m n^3 + 0.54 m^2 n^2 against 3 m n^3 + m^2 n^2 of the W A_i W form (4 m n^3 + m^2 n^2 dense).
+// K1 reads the lower triangle of A_i and C only. Rows m and m+1 of Haug are AQc_j = <L^T C L, S_j> and
+// AW_j = tr(S_j) as before. Executed flops: 1.0 m n^3 + 0.54 m^2 n^2 against 3 m n^3 + m^2 n^2 of the W A_i W form
+// (4 m n^3 + m^2 n^2 dense).
 // dL: n*n scratch for the factor; d_info[0] != 0 reports a W that is not numerically positive definite
 // (the caller then falls back to cxb_schur_dense_lmi). dX: (m + 2) * cxb_packed_symmetric_size(n).
 extern "C" size_t cxb_packed_symmetric_size(int n) { return (size_t)cxb::PackedSymmetricSize(n); }
@@ -77,10 +79,10 @@ extern "C" int cxb_schur_dense_lmi_sym_scale(void* stream, int n, int m, const d
   for (int p0 = 0; p0 < total; p0 += panel) {
     const int pb = (panel < total - p0) ? panel : (total - p0);
     rc = DgemmStructured(s, -1, 1, false, false, n, n, n, 1.0, dAall + (long)p0 * nn, n, nn, dL, n, 0, 0.0, dT,
-                         n, nn, pb, false, false, 0, /*tri=*/1, false);
+                         n, nn, pb, true, false, 0, kHalfLowerTimesLower, false);
     if (rc) return rc;
     rc = DgemmStructured(s, -1, 1, true, false, n, n, n, 1.0, dL, n, 0, dT, n, nn, 0.0, dX + (long)p0 * kp, n,
-                         kp, pb, true, false, 0, /*tri=*/2, /*pack=*/true);
+                         kp, pb, true, false, 0, kSyr2kLower, /*pack=*/true);
     if (rc) return rc;
   }
   // row m + 1 of the Gram: the packed identity, AW_j = tr(S_j) = <I, S_j>
