@@ -6,20 +6,25 @@
 // Factorisation, two levels of blocking:
 //   outer block column of kOuter = 512 columns:
 //     for each inner block of kNB = 128 columns inside it
-//       1. PotrfDiagKernel  — one CTA factors the 128 x 128 diagonal block in shared memory
-//                             (column scale + rank-1 update per step, fixed thread->(row, column
-//                             group) map, no integer division in the loop);
+//       1. PotrfDiagBlockedKernel — one CTA factors the 128 x 128 diagonal block in shared memory,
+//                             in 32 x 32 sub-blocks (warp-shuffle factor of the diagonal part,
+//                             substitution for the rows below, register-tiled rank-32 update);
 //       2. TrsmPanelKernel  — X L11^T = A21 by true substitution (no explicit inverses: H becomes
 //                             very ill conditioned late in the IPM). One thread per row keeps 32
 //                             accumulators in registers; L11 is streamed through shared memory in
 //                             32-column slabs and read as 16-byte broadcasts;
 //       3. DMMA update of the rest of the outer block column (lower trapezoid, K = 128);
 //     DMMA SYRK of everything to the right with K = 512 (gemm.cu) — where the flops are.
+// Above 3 x 512 columns the outer loop runs with a look-ahead of one block column: panel J + 1 is
+// factored on a high-priority side stream while panel J updates the rest of the trailing matrix.
 // A non-positive pivot sets *info = 1 + column (Eigen::LLT::info() != Success in the reference).
 //
-// Solves: one launch per 128-column block and direction. Every CTA redundantly solves the small
-// diagonal system (4 x (32 x 32 warp-shuffle substitution + block update) in shared memory) and then
-// applies the block's update to its own rows, so no second launch or inter-CTA flag is needed.
+// Solves: one launch per sweep and right-hand side, a wavefront over the 128-row blocks whose
+// hand-off between CTAs is the solution vector itself, polled against a sentinel (see "triangular
+// solves" below).
+//
+// The LDL^T (K4) reuses the panel solve and the DMMA updates; its diagonal blocks are factored by
+// LdltDiagKernel, a signed rank-1 variant (L S L^T, S = diag(+-1)).
 // All global->shared staging keeps 8 loads in flight per thread (latency, not bandwidth, is the
 // limit of these small kernels).
 #include <algorithm>
@@ -53,23 +58,19 @@ __device__ __forceinline__ void BatchedCopy(int total, int tid, int nthreads, Lo
 }
 
 // ---- 1. diagonal block ---------------------------------------------------------------------------
-// Factor the nb x nb (nb <= 128) block at H (ld) in place; lower triangle. One CTA of 512 threads.
-// Thread t owns row r = t % 128 and the columns c with c % 4 == t / 128.
-//
-// SIGNED = true factors a symmetric indefinite block as L S L^T with S = diag(+-1) ("signed
-// Cholesky" = LDL^T with D = S and the columns of L scaled by sqrt|d|): pivots with |d| <= 1e-9 are
-// replaced by +-1e-9 like Eigen::RLDLT (RLDLT.h:378-389) and reported through info[1]; it never fails.
-template <bool SIGNED>
-__global__ void __launch_bounds__(512) PotrfDiagKernel(int nb, double* H, long ld, int col0,
-                                                       int* info, double* signs) {
+// Signed factorisation of the nb x nb (nb <= 128) block at H (ld) in place, lower triangle: a symmetric
+// indefinite block becomes L S L^T with S = diag(+-1) ("signed Cholesky" = LDL^T with D = S and the
+// columns of L scaled by sqrt|d|), S stored to signs[col0 ..]. Pivots with |d| <= 1e-9 are replaced by
+// +-1e-9 like Eigen::RLDLT (RLDLT.h:378-389) and reported through info[1]; it never fails.
+// One CTA of 512 threads, column scale + rank-1 update per step: thread t owns row r = t % 128 and the
+// columns c with c % 4 == t / 128.
+__global__ void __launch_bounds__(512) LdltDiagKernel(int nb, double* H, long ld, int col0, int* info,
+                                                      double* signs) {
   extern __shared__ double s[];  // s[c * P + r], P = 129
   constexpr int P = kNB + 1;
-  __shared__ int failed;
   const int tid = threadIdx.x;
   const int r = tid & (kNB - 1);
   const int cg = tid >> 7;  // 0..3
-  if (!SIGNED && *info != 0) return;  // an earlier block already failed
-  if (tid == 0) failed = 0;
   BatchedCopy<8>(
       kNB * kNB, tid, 512,
       [&](int e) {
@@ -80,49 +81,39 @@ __global__ void __launch_bounds__(512) PotrfDiagKernel(int nb, double* H, long l
   __syncthreads();
   for (int j = 0; j < nb; j++) {
     double d = s[j * P + j];
-    double sign = 1.0;
-    if (SIGNED) {
-      if (!(fabs(d) > 1e-9)) {
-        d = (d < 0) ? -1e-9 : 1e-9;
-        if (tid == 0) info[1] = 1;  // regularization_used
-      }
-      sign = (d < 0) ? -1.0 : 1.0;
-      if (tid == 0) signs[col0 + j] = sign;
-      d = fabs(d);
-    } else if (!(d > 0.0)) {  // every thread sees the same d: uniform branch
-      if (tid == 0) {
-        failed = 1;
-        *info = col0 + j + 1;
-      }
-      break;
+    if (!(fabs(d) > 1e-9)) {
+      d = (d < 0) ? -1e-9 : 1e-9;
+      if (tid == 0) info[1] = 1;  // regularization_used
     }
+    const double sign = (d < 0) ? -1.0 : 1.0;
+    if (tid == 0) signs[col0 + j] = sign;
+    d = fabs(d);
     const double rd = sqrt(d);
     const double inv = 1.0 / rd;
     // l[r] for this thread's row (pre-scale value is still in s[j][r] until the barrier below);
-    // signed: column j of L is sign * a_j / sqrt|d| and the update is sign * (a_r a_c / |d|)
+    // column j of L is sign * a_j / sqrt|d| and the update is sign * (a_r a_c / |d|)
     const double lr = (r > j && r < nb) ? s[j * P + r] * inv : 0.0;
     // trailing update of my row: s[c][r] -= l[r] * l[c] for j < c <= r, c in my column group
     if (r > j && r < nb) {
       int c = j + 1 + ((cg - (j + 1)) & 3);  // first c > j with c % 4 == cg
-      const double slr = SIGNED ? sign * lr : lr;
+      const double slr = sign * lr;
       for (; c <= r; c += 4) s[c * P + r] -= slr * (s[j * P + c] * inv);
     }
     __syncthreads();  // all reads of the unscaled column j are done
     if (cg == 0 && r < nb) {
       if (r == j) s[j * P + j] = rd;
-      if (r > j) s[j * P + r] = SIGNED ? sign * lr : lr;
+      if (r > j) s[j * P + r] = sign * lr;
     }
     __syncthreads();
   }
   __syncthreads();
-  if (failed) return;
   if (r < nb) {
     for (int c = cg; c <= r; c += 4) H[(long)c * ld + r] = s[c * P + r];
   }
 }
 
-// Plain Cholesky of the same block, blocked 32 x 32 inside the CTA (the rank-1 kernel above spends two
-// barriers per column: 132 us per 128 x 128 block, 40 % of the whole factorisation at m = 10^4):
+// Cholesky of the diagonal block, blocked 32 x 32 inside the CTA (a rank-1 kernel like the one above
+// spends two barriers per column: 132 us per 128 x 128 block, 40 % of the whole factorisation at m = 10^4):
 //   for each 32-column sub-block: warp 0 factors the 32 x 32 diagonal part in registers (lane = row,
 //   column entries exchanged by shuffles); one thread per row below solves its 32 entries by
 //   substitution in registers; all 512 threads apply the rank-32 update to the rest of the block
@@ -300,6 +291,20 @@ __global__ void __launch_bounds__(kNB) TrsmPanelKernel(int nb, const double* __r
 }
 
 // ---- triangular solves -------------------------------------------------------------------------------
+// One launch per sweep and right-hand side: a wavefront over the 128-row blocks. The CTA with ticket i owns
+// block row i of the sweep: it streams its own part of L exactly once, consuming each earlier solution block
+// as soon as its owner has stored it, then solves its 128 x 128 diagonal block and stores x_i. Tickets come
+// from an atomic counter, so a CTA only ever waits for CTAs that started before it: no co-residency
+// assumption, no deadlock when m / 128 exceeds the number of SMs.
+// The solution itself is the hand-off: the output vector is pre-filled with a sentinel (a quiet NaN with a
+// payload no computation produces) and every consuming WARP polls the 32 (forward) / 128 (backward) solution
+// entries it needs with relaxed gpu-scope loads until none is the sentinel: one L2 round trip, no flag, no
+// fence (each entry is a single 64-bit store, so seeing it is seeing all of it) and no CTA barrier between
+// the producer's store and the consumer's FMAs. (A release/acquire flag per block costs about 5 us of
+// barriers, fence and spin per hand-off, and that chain of m / 128 hand-offs, not bandwidth, set the pace:
+// profiles/r01_m_*.) The right-hand side is read from a separate array. The diagonal blocks are solved by
+// true substitution, with the reciprocal of the diagonal folded into the rows beforehand so that the
+// 32-step chain is shuffle + FMA only. Summation order is fixed: results are deterministic.
 // Loads the nb x nb lower block L (ld) into shared memory, sl[c * P + r] = L[r][c], and the
 // reciprocals of its diagonal into srd.
 template <int P>
@@ -317,394 +322,6 @@ __device__ __forceinline__ void LoadLowerBlock(double* sl, double* srd, const do
   }
 }
 
-// Forward: x_k = L_kk^{-1} b_k (in shared memory sx[k * kNB + r]), all right-hand sides. 256 threads.
-template <int P>
-__device__ __forceinline__ void SolveLowerBlock(const double* sl, const double* srd, double* sx, int nb,
-                                                int nrhs) {
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  for (int b0 = 0; b0 < nb; b0 += 32) {
-    const int bw = min(32, nb - b0);
-    if (warp < nrhs) {  // one warp per right-hand side solves the 32 x 32 diagonal sub-block
-      double v = (lane < bw) ? sx[warp * kNB + b0 + lane] : 0.0;
-      for (int j = 0; j < bw; j++) {
-        const double xj = __shfl_sync(0xffffffffu, v, j) * srd[b0 + j];
-        if (lane == j) v = xj;
-        if (lane > j && lane < bw) v -= sl[(b0 + j) * P + b0 + lane] * xj;
-      }
-      if (lane < bw) sx[warp * kNB + b0 + lane] = v;
-    }
-    __syncthreads();
-    // rows below the sub-block: b[r] -= sum_j L[r][b0 + j] x_j
-    for (int e = tid; e < (nb - b0 - bw) * nrhs; e += blockDim.x) {
-      const int r = b0 + bw + e % (nb - b0 - bw), k = e / (nb - b0 - bw);
-      double a = 0;
-      for (int j = 0; j < bw; j++) a += sl[(b0 + j) * P + r] * sx[k * kNB + b0 + j];
-      sx[k * kNB + r] -= a;
-    }
-    __syncthreads();
-  }
-}
-
-// Backward: x_k = L_kk^{-T} z_k.
-template <int P>
-__device__ __forceinline__ void SolveLowerTransposedBlock(const double* sl, const double* srd, double* sx,
-                                                          int nb, int nrhs) {
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int nblk = (nb + 31) / 32;
-  for (int bi = nblk - 1; bi >= 0; bi--) {
-    const int b0 = bi * 32;
-    const int bw = min(32, nb - b0);
-    if (warp < nrhs) {
-      double v = (lane < bw) ? sx[warp * kNB + b0 + lane] : 0.0;
-      for (int j = bw - 1; j >= 0; j--) {
-        const double xj = __shfl_sync(0xffffffffu, v, j) * srd[b0 + j];
-        if (lane == j) v = xj;
-        // x[r] -= L[j][r] x_j for r < j  (L^T[r][j] = L[j][r] = sl[r * P + j])
-        if (lane < j) v -= sl[(b0 + lane) * P + b0 + j] * xj;
-      }
-      if (lane < bw) sx[warp * kNB + b0 + lane] = v;
-    }
-    __syncthreads();
-    // rows above the sub-block: z[r] -= sum_j L[b0 + j][r] x_j, r < b0
-    for (int e = tid; e < b0 * nrhs; e += blockDim.x) {
-      const int r = e % b0, k = e / b0;
-      double a = 0;
-      for (int j = 0; j < bw; j++) a += sl[r * P + b0 + j] * sx[k * kNB + b0 + j];
-      sx[k * kNB + r] -= a;
-    }
-    __syncthreads();
-  }
-}
-
-constexpr int kFwdRows = 64;  // rows per CTA in the forward update (4 column groups of 32 each)
-
-// One forward step: every CTA solves block k (redundantly) from the working vector X, CTA 0 stores
-// the solved block into Out (a different array: other CTAs may still be reading the unsolved block
-// from X), then each CTA updates its 64 rows below: x[r] -= L[r, kblock] x_k. Thread (r, g) sums
-// the 32 columns of group g with all loads in flight; the 4 partials are added in a fixed order.
-__global__ void __launch_bounds__(256) TrsvFwdStepKernel(int m, int j0, int nb,
-                                                         const double* __restrict__ L, long ld,
-                                                         double* X, long ldx, double* Out, long ldo,
-                                                         int nrhs) {
-  constexpr int P = kNB + 1;
-  extern __shared__ double s[];
-  double* sl = s;
-  double* sx = s + kNB * P;           // kMaxRhs x kNB
-  double* srd = sx + kMaxRhs * kNB;   // kNB
-  double* sp = srd + kNB;             // partial sums: kMaxRhs x 4 x kFwdRows
-  const int tid = threadIdx.x;
-  LoadLowerBlock<P>(sl, srd, L + (long)j0 * ld + j0, ld, nb);
-  for (int e = tid; e < kNB * nrhs; e += 256) {
-    const int r = e & (kNB - 1), k = e >> 7;
-    sx[k * kNB + r] = (r < nb) ? X[(long)k * ldx + j0 + r] : 0.0;
-  }
-  __syncthreads();
-  SolveLowerBlock<P>(sl, srd, sx, nb, nrhs);
-  if (blockIdx.x == 0) {
-    for (int e = tid; e < nb * nrhs; e += 256) Out[(long)(e / nb) * ldo + j0 + e % nb] = sx[(e / nb) * kNB + e % nb];
-  }
-  const int rl = tid & (kFwdRows - 1), g = tid >> 6;
-  const int r = j0 + nb + blockIdx.x * kFwdRows + rl;
-  double acc[kMaxRhs] = {0, 0, 0, 0};
-  if (r < m) {
-    const double* Lr = L + (long)(j0 + g * 32) * ld + r;
-    double l[32];
-#pragma unroll
-    for (int c = 0; c < 32; c++) l[c] = (g * 32 + c < nb) ? Lr[(long)c * ld] : 0.0;
-#pragma unroll
-    for (int c = 0; c < 32; c++) {
-#pragma unroll
-      for (int k = 0; k < kMaxRhs; k++) {
-        if (k < nrhs) acc[k] += l[c] * sx[k * kNB + g * 32 + c];
-      }
-    }
-  }
-#pragma unroll
-  for (int k = 0; k < kMaxRhs; k++) {
-    if (k < nrhs) sp[(k * 4 + g) * kFwdRows + rl] = acc[k];
-  }
-  __syncthreads();
-  if (g == 0 && r < m) {
-#pragma unroll
-    for (int k = 0; k < kMaxRhs; k++) {
-      if (k < nrhs) {
-        const double t = ((sp[(k * 4 + 0) * kFwdRows + rl] + sp[(k * 4 + 1) * kFwdRows + rl]) +
-                          sp[(k * 4 + 2) * kFwdRows + rl]) + sp[(k * 4 + 3) * kFwdRows + rl];
-        X[(long)k * ldx + r] -= t;
-      }
-    }
-  }
-}
-
-// One backward step: every CTA solves block k with L_kk^T from the working vector X, CTA 0 stores
-// x_k into Out, then each CTA updates its 32 entries c < j0 (one warp per 4 columns of L, all four
-// columns' loads in flight): x[c] -= L[kblock rows, c]^T x_k.
-__global__ void __launch_bounds__(256) TrsvBwdStepKernel(int j0, int nb, const double* __restrict__ L,
-                                                         long ld, double* X, long ldx, double* Out,
-                                                         long ldo, int nrhs) {
-  constexpr int P = kNB + 1;
-  extern __shared__ double s[];
-  double* sl = s;
-  double* sx = s + kNB * P;
-  double* srd = sx + kMaxRhs * kNB;
-  const int tid = threadIdx.x, lane = tid & 31;
-  LoadLowerBlock<P>(sl, srd, L + (long)j0 * ld + j0, ld, nb);
-  for (int e = tid; e < kNB * nrhs; e += 256) {
-    const int r = e & (kNB - 1), k = e >> 7;
-    sx[k * kNB + r] = (r < nb) ? X[(long)k * ldx + j0 + r] : 0.0;
-  }
-  __syncthreads();
-  SolveLowerTransposedBlock<P>(sl, srd, sx, nb, nrhs);
-  if (blockIdx.x == 0) {
-    for (int e = tid; e < nb * nrhs; e += 256) Out[(long)(e / nb) * ldo + j0 + e % nb] = sx[(e / nb) * kNB + e % nb];
-  }
-  const int cbase = (blockIdx.x * 8 + (tid >> 5)) * 4;
-  double l[4][4];
-#pragma unroll
-  for (int q = 0; q < 4; q++) {
-    const int c = cbase + q;
-#pragma unroll
-    for (int i = 0; i < 4; i++) {
-      const int r = lane + 32 * i;
-      l[q][i] = (c < j0 && r < nb) ? L[(long)c * ld + j0 + r] : 0.0;
-    }
-  }
-#pragma unroll
-  for (int q = 0; q < 4; q++) {
-    const int c = cbase + q;
-#pragma unroll
-    for (int k = 0; k < kMaxRhs; k++) {
-      if (k < nrhs) {
-        double a = 0;
-#pragma unroll
-        for (int i = 0; i < 4; i++) a += l[q][i] * sx[k * kNB + lane + 32 * i];
-        const double v = WarpSum(a);
-        if (lane == 0 && c < j0) X[(long)k * ldx + c] -= v;
-      }
-    }
-  }
-}
-
-// ---- single-launch sweeps (wavefront over block rows) ------------------------------------------------
-// One launch per direction instead of one per 128-column block (the stepwise kernels above reach
-// 0.2 TB/s at m = 10^4: 2 x 79 launches of ~26 us whose every CTA re-solves the diagonal block).
-// CTA with ticket i owns block row i of the sweep: it streams its own part of L exactly once,
-// consuming each earlier solution block x_k as soon as its owner publishes it (release/acquire flag
-// in global memory), then solves its 128 x 128 diagonal block by substitution and publishes x_i.
-// Tickets come from an atomic counter, so a CTA only ever waits for CTAs that started before it:
-// no co-residency assumption, no deadlock when m / 128 exceeds the number of SMs. Summation order is
-// fixed (independent of timing): results are deterministic. One right-hand side per launch.
-__device__ __forceinline__ void WaitFlag(const int* flag) {
-  if (threadIdx.x == 0) {
-    int v;
-    do {
-      asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(flag) : "memory");
-    } while (v == 0);
-  }
-  __syncthreads();
-}
-// Call after a __syncthreads() that follows the block's global writes.
-__device__ __forceinline__ void SetFlag(int* flag) {
-  if (threadIdx.x == 0) {
-    __threadfence();
-    asm volatile("st.release.gpu.global.s32 [%0], %1;" ::"l"(flag), "r"(1) : "memory");
-  }
-}
-
-// x (one right-hand side, sx[0..127]) <- L_kk^{-1} x by 32 x 32 warp-shuffle substitutions (warp 0, its
-// row of the sub-block in registers) and block updates by all threads. Rows >= nb are padded
-// (sl = 0, srd = 0) and come out as 0.
-template <int P>
-__device__ __forceinline__ void SolveLowerBlock1(const double* sl, const double* srd, double* sx) {
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-#pragma unroll 1
-  for (int b0 = 0; b0 < kNB; b0 += 32) {
-    if (warp == 0) {
-      double lrow[32];
-#pragma unroll
-      for (int j = 0; j < 32; j++) lrow[j] = sl[(b0 + j) * P + b0 + lane];  // L[b0 + lane][b0 + j]
-      double v = sx[b0 + lane];
-      const double rd = srd[b0 + lane];
-#pragma unroll
-      for (int j = 0; j < 32; j++) {
-        const double xj = __shfl_sync(0xffffffffu, v * rd, j);
-        if (lane == j) v = xj;
-        if (lane > j) v -= lrow[j] * xj;
-      }
-      sx[b0 + lane] = v;
-    }
-    __syncthreads();
-    // rows below the sub-block: 4 threads per row, 8 columns each, fixed-order combination
-    const int rows = kNB - b0 - 32;
-    if (tid < rows * 4) {
-      const int r = b0 + 32 + (tid >> 2), q = tid & 3;
-      double a = 0;
-#pragma unroll
-      for (int j = 0; j < 8; j++) a += sl[(b0 + q * 8 + j) * P + r] * sx[b0 + q * 8 + j];
-      a += __shfl_xor_sync(0xffffffffu, a, 1);
-      a += __shfl_xor_sync(0xffffffffu, a, 2);
-      if (q == 0) sx[r] -= a;
-    }
-    __syncthreads();
-  }
-}
-
-// x <- L_kk^{-T} x, same organisation from the bottom up.
-template <int P>
-__device__ __forceinline__ void SolveLowerTransposedBlock1(const double* sl, const double* srd, double* sx) {
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-#pragma unroll 1
-  for (int b0 = kNB - 32; b0 >= 0; b0 -= 32) {
-    if (warp == 0) {
-      double lcol[32];
-#pragma unroll
-      for (int j = 0; j < 32; j++) lcol[j] = sl[(b0 + lane) * P + b0 + j];  // L[b0 + j][b0 + lane]
-      double v = sx[b0 + lane];
-      const double rd = srd[b0 + lane];
-#pragma unroll
-      for (int j = 31; j >= 0; j--) {
-        const double xj = __shfl_sync(0xffffffffu, v * rd, j);
-        if (lane == j) v = xj;
-        if (lane < j) v -= lcol[j] * xj;
-      }
-      sx[b0 + lane] = v;
-    }
-    __syncthreads();
-    // entries above the sub-block: z[r] -= sum_j L[b0 + j][r] x_j for r < b0
-    if (tid < b0 * 4) {
-      const int r = tid >> 2, q = tid & 3;
-      double a = 0;
-#pragma unroll
-      for (int j = 0; j < 8; j++) a += sl[r * P + b0 + q * 8 + j] * sx[b0 + q * 8 + j];
-      a += __shfl_xor_sync(0xffffffffu, a, 1);
-      a += __shfl_xor_sync(0xffffffffu, a, 2);
-      if (q == 0) sx[r] -= a;
-    }
-    __syncthreads();
-  }
-}
-
-// sync[0]: ticket counter, sync[1 + k]: block k solved. Both zero at launch.
-__global__ void __launch_bounds__(512) TrsvFwdWaveKernel(int m, const double* __restrict__ L, long ld,
-                                                         double* X, int* sync) {
-  constexpr int P = kNB + 1;
-  extern __shared__ double s[];
-  double* sl = s;
-  double* sx = s + kNB * P;   // kNB
-  double* srd = sx + kNB;     // kNB
-  double* sp = srd + kNB;     // 4 x kNB partial sums
-  double* sxk = sp + 4 * kNB; // 2 x kNB: solution block being consumed
-  __shared__ int s_block;
-  const int tid = threadIdx.x;
-  if (tid == 0) s_block = atomicAdd(&sync[0], 1);
-  __syncthreads();
-  const int i = s_block;
-  int* flags = sync + 1;
-  const int r0 = i * kNB;
-  const int nb = min(kNB, m - r0);
-  LoadLowerBlock<P>(sl, srd, L + (long)r0 * ld + r0, ld, nb);
-  const int rl = tid & (kNB - 1), g = tid >> 7;  // row of the strip, column group (32 of every 128)
-  const bool active = rl < nb;
-  const int r = r0 + rl;
-  double acc = 0;
-  for (int kb = 0; kb < i; kb++) {
-    const double* Lr = L + (long)(kb * kNB + g * 32) * ld + r;
-    double l[32];
-#pragma unroll
-    for (int c = 0; c < 32; c++) l[c] = active ? __ldcs(Lr + (long)c * ld) : 0.0;  // read exactly once
-    WaitFlag(flags + kb);
-    // x_kb goes through shared memory: one coalesced L2 read per CTA. (Every thread fetching its 32
-    // values itself put 512 requests per CTA and step on the same few L2 sectors — with ~150 CTAs in
-    // lock step that hot spot, not the substitution chain, set the pace.) Double-buffered: the
-    // barrier inside the next WaitFlag separates these reads from the write after next.
-    double* xs = sxk + (kb & 1) * kNB;
-    if (tid < kNB) xs[tid] = __ldcg(X + kb * kNB + tid);  // L2: written by another SM
-    __syncthreads();
-#pragma unroll
-    for (int c = 0; c < 32; c++) acc += l[c] * xs[g * 32 + c];
-  }
-  sp[g * kNB + rl] = acc;
-  __syncthreads();
-  if (g == 0) sx[rl] = active ? X[r] - (((sp[rl] + sp[kNB + rl]) + sp[2 * kNB + rl]) + sp[3 * kNB + rl]) : 0.0;
-  __syncthreads();
-  SolveLowerBlock1<P>(sl, srd, sx);
-  if (tid < nb) X[r0 + tid] = sx[tid];
-  __syncthreads();
-  SetFlag(flags + i);
-}
-
-__global__ void __launch_bounds__(512) TrsvBwdWaveKernel(int m, const double* __restrict__ L, long ld,
-                                                         double* X, int* sync) {
-  constexpr int P = kNB + 1;
-  extern __shared__ double s[];
-  double* sl = s;
-  double* sx = s + kNB * P;
-  double* srd = sx + kNB;
-  double* sp = srd + kNB;  // kNB column sums
-  double* sxk = sp + 4 * kNB;
-  __shared__ int s_block;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if (tid == 0) s_block = atomicAdd(&sync[0], 1);
-  __syncthreads();
-  const int nblk = (m + kNB - 1) / kNB;
-  const int i = nblk - 1 - s_block;
-  int* flags = sync + 1;
-  const int c0 = i * kNB;
-  const int nb = min(kNB, m - c0);
-  LoadLowerBlock<P>(sl, srd, L + (long)c0 * ld + c0, ld, nb);
-  // warp w owns the columns c0 + 8 w .. c0 + 8 w + 7 of L; lanes run down the rows of a block
-  double acc[8];
-#pragma unroll
-  for (int q = 0; q < 8; q++) acc[q] = 0;
-  for (int kb = nblk - 1; kb > i; kb--) {
-    const int rb = kb * kNB;
-    const int nrows = min(kNB, m - rb);
-    double l[8][4];
-#pragma unroll
-    for (int q = 0; q < 8; q++) {
-      const int cw = warp * 8 + q;
-      const double* Lc = L + (long)(c0 + cw) * ld + rb + lane;
-#pragma unroll
-      for (int p = 0; p < 4; p++) l[q][p] = (cw < nb && lane + 32 * p < nrows) ? __ldcs(Lc + 32 * p) : 0.0;
-    }
-    WaitFlag(flags + kb);
-    double* xs = sxk + (kb & 1) * kNB;  // see the forward kernel
-    if (tid < kNB) xs[tid] = (tid < nrows) ? __ldcg(X + rb + tid) : 0.0;
-    __syncthreads();
-    double xv[4];
-#pragma unroll
-    for (int p = 0; p < 4; p++) xv[p] = xs[lane + 32 * p];
-#pragma unroll
-    for (int q = 0; q < 8; q++) {
-#pragma unroll
-      for (int p = 0; p < 4; p++) acc[q] += l[q][p] * xv[p];
-    }
-  }
-#pragma unroll
-  for (int q = 0; q < 8; q++) {
-    const double v = WarpSum(acc[q]);
-    if (lane == 0) sp[warp * 8 + q] = v;
-  }
-  __syncthreads();
-  if (tid < kNB) sx[tid] = (tid < nb) ? X[c0 + tid] - sp[tid] : 0.0;
-  __syncthreads();
-  SolveLowerTransposedBlock1<P>(sl, srd, sx);
-  if (tid < nb) X[c0 + tid] = sx[tid];
-  __syncthreads();
-  SetFlag(flags + i);
-}
-
-// ---- single-launch sweeps, second version: the solution itself is the hand-off -----------------------
-// The flag version above spends per 128-row block: st X, barrier, fence, st.release flag | ld.acquire spin by one
-// thread, barrier, L2 read of x, barrier, 32 FMAs, two more barriers — about 5 us on top of the diagonal solve,
-// and that chain of m / 128 hand-offs, not bandwidth, sets the pace (profiles/r01_m_*). Here the output vector is
-// pre-filled with a sentinel (a quiet NaN with a payload no computation produces) and every consuming WARP polls the
-// 32 (forward) / 128 (backward) solution entries it needs with relaxed gpu-scope loads until none is the sentinel:
-// one L2 round trip, no flag, no fence (each entry is a single 64-bit store, so seeing it is seeing all of it) and
-// no CTA barrier between the producer's store and the consumer's FMAs. The right-hand side is read from a
-// separate array. The diagonal blocks are solved by the same true substitution, with the reciprocal of the
-// diagonal folded into the rows beforehand so that the 32-step chain is shuffle + FMA only.
-// Summation order is fixed, tickets as above: deterministic, no co-residency assumption.
 constexpr unsigned long long kSentinelBits = 0x7FF8DEADBEEF0001ull;
 __device__ __forceinline__ bool IsSentinel(double v) {
   return static_cast<unsigned long long>(__double_as_longlong(v)) == kSentinelBits;
@@ -1006,28 +623,14 @@ __global__ void ApplySignsKernel(int N, int nrhs, const double* __restrict__ sig
 
 constexpr size_t kDiagSmem = sizeof(double) * kNB * (kNB + 1);
 constexpr size_t kTrsmSmem = sizeof(double) * (kNB * kNB + kNB * 32 + 32);
-constexpr size_t kTrsvSmem =
-    sizeof(double) * (kNB * (kNB + 1) + kMaxRhs * kNB + kNB + kMaxRhs * 4 * kFwdRows);
 constexpr size_t kWaveSmem = sizeof(double) * (kNB * (kNB + 1) + 8 * kNB);
-// 2: single-launch sweeps whose hand-off is the solution itself (default); 0: single-launch sweeps with
-// release/acquire flags; 1: one launch per block. The earlier schemes are kept for A/B measurements through
-// cxb_set_trsv_mode.
-int g_trsv_mode = 2;
-// 0: blocked diagonal kernel (default); 1: rank-1 kernel (the earlier one; A/B through cxb_set_potrf_mode)
-int g_potrf_mode = 0;
-int g_potrf_lookahead = 1;  // bit 1 of cxb_set_potrf_mode clears it (sequential schedule, A/B)
 
 void ConfigureOnce() {
   static std::atomic<unsigned long long> configured{0};
   if (!FirstUseOnCurrentDevice(configured)) return;
-  cudaFuncSetAttribute(PotrfDiagKernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kDiagSmem);
-  cudaFuncSetAttribute(PotrfDiagKernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kDiagSmem);
+  cudaFuncSetAttribute(LdltDiagKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kDiagSmem);
   cudaFuncSetAttribute(PotrfDiagBlockedKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kDiagSmem);
   cudaFuncSetAttribute(TrsmPanelKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTrsmSmem);
-  cudaFuncSetAttribute(TrsvFwdStepKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTrsvSmem);
-  cudaFuncSetAttribute(TrsvBwdStepKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTrsvSmem);
-  cudaFuncSetAttribute(TrsvFwdWaveKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWaveSmem);
-  cudaFuncSetAttribute(TrsvBwdWaveKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWaveSmem);
   cudaFuncSetAttribute(TrsvFwdPollKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWaveSmem);
   cudaFuncSetAttribute(TrsvBwdPollKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWaveSmem);
 }
@@ -1041,12 +644,7 @@ int PotrfBlockColumn(cudaStream_t s, int m, int j0, int w, double* H, long ldh, 
   for (int i0 = j0; i0 < j0 + w; i0 += kNB) {
     const int nb = min(kNB, j0 + w - i0);
     double* Hii = H + (long)i0 * ldh + i0;
-    CountLaunch();
-    if (g_potrf_mode == 0) {
-      PotrfDiagBlockedKernel<<<1, 512, kDiagSmem, s>>>(nb, Hii, ldh, i0, info);
-    } else {
-      PotrfDiagKernel<false><<<1, 512, kDiagSmem, s>>>(nb, Hii, ldh, i0, info, nullptr);
-    }
+    CountLaunch(); PotrfDiagBlockedKernel<<<1, 512, kDiagSmem, s>>>(nb, Hii, ldh, i0, info);
     const int rows = m - i0 - nb;
     if (rows <= 0) continue;
     double* A21 = Hii + nb;
@@ -1074,30 +672,7 @@ size_t cxb_potrf_worksize(int m) {
 }
 
 namespace {
-// Per host thread: a high-priority side stream and two events for the look-ahead below (a Program is
-// single-threaded; programs driven from different threads get their own).
-struct LookAhead {
-  cudaStream_t side = nullptr;
-  cudaEvent_t updated = nullptr, factored = nullptr;
-  int device = -1;
-  bool Prepare() {
-    int current = 0;
-    if (cudaGetDevice(&current) != cudaSuccess) return false;
-    if (side && device == current) return true;
-    if (side) {  // the thread moved to another device: streams and events belong to the old one
-      cudaStreamDestroy(side);
-      cudaEventDestroy(updated);
-      cudaEventDestroy(factored);
-      side = nullptr;
-    }
-    device = current;
-    int lo = 0, hi = 0;
-    cudaDeviceGetStreamPriorityRange(&lo, &hi);
-    if (cudaStreamCreateWithPriority(&side, cudaStreamNonBlocking, hi) != cudaSuccess) return false;
-    return cudaEventCreateWithFlags(&updated, cudaEventDisableTiming) == cudaSuccess &&
-           cudaEventCreateWithFlags(&factored, cudaEventDisableTiming) == cudaSuccess;
-  }
-};
+// Side stream of the Cholesky's look-ahead below, separate from the LU's.
 thread_local LookAhead t_lookahead;
 
 // Right-looking factorisation with a look-ahead of one outer block column: after panel J the update
@@ -1148,7 +723,7 @@ int cxb_potrf_lower(void* stream, int m, double* dH, long ldh, double* d_work, i
   CountLaunch(); ResetInfoKernel<<<1, 1, 0, s>>>(d_info);
   // below three outer block columns there is nothing to overlap; the legacy default stream cannot
   // run concurrently with a side stream's work ordering-wise in a useful way either
-  if (g_potrf_lookahead && m > 3 * kOuter) return PotrfLookAhead(s, m, dH, ldh, d_info);
+  if (m > 3 * kOuter) return PotrfLookAhead(s, m, dH, ldh, d_info);
   for (int j0 = 0; j0 < m; j0 += kOuter) {
     const int w = min(kOuter, m - j0);
     int rc = PotrfBlockColumn(s, m, j0, w, dH, ldh, d_info);
@@ -1205,32 +780,19 @@ int cxb_trsv_lower(void* stream, int m, const double* dL, long ldl, double* dx, 
   if (m <= 0) return 0;
   ConfigureOnce();
   const int nblk = (m + kNB - 1) / kNB;
-  if (g_trsv_mode == 2) {
-    // out-of-place sweep into a sentinel-filled scratch vector (+ the ticket behind it), copied back
-    double* Z = nullptr;
-    if (cudaMallocAsync(&Z, sizeof(double) * ((size_t)m + 2), s) != cudaSuccess) return (int)cudaErrorMemoryAllocation;
-    int* ticket = reinterpret_cast<int*>(Z + m);
-    CountLaunch(); WaveInitKernel<<<(m + 255) / 256, 256, 0, s>>>(Z, m, ticket, 1);
-    CountLaunch();
-    if (transposed) {
-      TrsvBwdPollKernel<<<nblk, 512, kWaveSmem, s>>>(m, dL, ldl, dx, Z, ticket);
-    } else {
-      TrsvFwdPollKernel<<<nblk, 512, kWaveSmem, s>>>(m, dL, ldl, dx, Z, ticket);
-    }
-    cudaMemcpyAsync(dx, Z, sizeof(double) * (size_t)m, cudaMemcpyDeviceToDevice, s);
-    cudaFreeAsync(Z, s);
-    return LaunchStatus();
-  }
-  int* sync = nullptr;
-  if (cudaMallocAsync(&sync, sizeof(int) * ((size_t)nblk + 1), s) != cudaSuccess) return (int)cudaErrorMemoryAllocation;
-  cudaMemsetAsync(sync, 0, sizeof(int) * ((size_t)nblk + 1), s);
+  // out-of-place sweep into a sentinel-filled scratch vector (+ the ticket behind it), copied back
+  double* Z = nullptr;
+  if (cudaMallocAsync(&Z, sizeof(double) * ((size_t)m + 2), s) != cudaSuccess) return (int)cudaErrorMemoryAllocation;
+  int* ticket = reinterpret_cast<int*>(Z + m);
+  CountLaunch(); WaveInitKernel<<<(m + 255) / 256, 256, 0, s>>>(Z, m, ticket, 1);
   CountLaunch();
   if (transposed) {
-    TrsvBwdWaveKernel<<<nblk, 512, kWaveSmem, s>>>(m, dL, ldl, dx, sync);
+    TrsvBwdPollKernel<<<nblk, 512, kWaveSmem, s>>>(m, dL, ldl, dx, Z, ticket);
   } else {
-    TrsvFwdWaveKernel<<<nblk, 512, kWaveSmem, s>>>(m, dL, ldl, dx, sync);
+    TrsvFwdPollKernel<<<nblk, 512, kWaveSmem, s>>>(m, dL, ldl, dx, Z, ticket);
   }
-  cudaFreeAsync(sync, s);
+  cudaMemcpyAsync(dx, Z, sizeof(double) * (size_t)m, cudaMemcpyDeviceToDevice, s);
+  cudaFreeAsync(Z, s);
   return LaunchStatus();
 }
 
@@ -1263,72 +825,24 @@ static int PotrsLowerImpl(cudaStream_t s, int m, const double* dL, long ldl, dou
   if (nrhs > kMaxRhs) return -1;
   ConfigureOnce();
   const int nblk = (m + kNB - 1) / kNB;
-  if (g_trsv_mode == 2) {
-    // forward: dX (b) -> Z (z); backward: Z -> dX. Both outputs are sentinel-filled right before their sweep.
-    const size_t mz = (size_t)m * nrhs;
-    double* Z = nullptr;
-    if (cudaMallocAsync(&Z, sizeof(double) * (mz + (size_t)nrhs + 1), s) != cudaSuccess) return (int)cudaErrorMemoryAllocation;
-    int* tickets = reinterpret_cast<int*>(Z + mz);  // 2 * nrhs ints
-    CountLaunch(); WaveInitKernel<<<(unsigned)((std::max<size_t>(mz, 2 * (size_t)nrhs) + 255) / 256), 256, 0, s>>>(Z, (long)mz, tickets, 2 * nrhs);
-    for (int k = 0; k < nrhs; k++) {
-      CountLaunch(); TrsvFwdPollKernel<<<nblk, 512, kWaveSmem, s>>>(m, dL, ldl, dX + (long)k * ldx, Z + (size_t)k * m, tickets + 2 * k);
-    }
-    if (signs) {
-      CountLaunch(); ApplySignsKernel<<<(m + 255) / 256, 256, 0, s>>>(m, nrhs, signs, Z, m);
-    }
-    for (int k = 0; k < nrhs; k++) {
-      CountLaunch(); WaveInitKernel<<<(m + 255) / 256, 256, 0, s>>>(dX + (long)k * ldx, m, nullptr, 0);
-      CountLaunch(); TrsvBwdPollKernel<<<nblk, 512, kWaveSmem, s>>>(m, dL, ldl, Z + (size_t)k * m, dX + (long)k * ldx, tickets + 2 * k + 1);
-    }
-    cudaFreeAsync(Z, s);
-    return LaunchStatus();
-  }
-  if (g_trsv_mode == 0) {
-    // one ticket counter + nblk flags per sweep and right-hand side, zeroed once
-    const size_t per = (size_t)nblk + 1;
-    int* sync = nullptr;
-    if (cudaMallocAsync(&sync, sizeof(int) * per * 2 * nrhs, s) != cudaSuccess) return (int)cudaErrorMemoryAllocation;
-    cudaMemsetAsync(sync, 0, sizeof(int) * per * 2 * nrhs, s);
-    for (int k = 0; k < nrhs; k++) {
-      CountLaunch(); TrsvFwdWaveKernel<<<nblk, 512, kWaveSmem, s>>>(m, dL, ldl, dX + (long)k * ldx, sync + per * (2 * k));
-    }
-    if (signs) {
-      CountLaunch(); ApplySignsKernel<<<(m + 255) / 256, 256, 0, s>>>(m, nrhs, signs, dX, ldx);
-    }
-    for (int k = 0; k < nrhs; k++) {
-      CountLaunch(); TrsvBwdWaveKernel<<<nblk, 512, kWaveSmem, s>>>(m, dL, ldl, dX + (long)k * ldx, sync + per * (2 * k + 1));
-    }
-    cudaFreeAsync(sync, s);
-    return LaunchStatus();
-  }
-  // z (the forward solution) is collected in a scratch array while dX is the working vector; the
-  // backward sweep then works in the scratch array and collects x in dX.
+  // forward: dX (b) -> Z (z); backward: Z -> dX. Both outputs are sentinel-filled right before their sweep.
+  const size_t mz = (size_t)m * nrhs;
   double* Z = nullptr;
-  if (cudaMallocAsync(&Z, sizeof(double) * (size_t)m * nrhs, s) != cudaSuccess) return (int)cudaErrorMemoryAllocation;
-  // forward: L z = b
-  for (int k = 0; k < nblk; k++) {
-    const int j0 = k * kNB, nb = min(kNB, m - j0);
-    const int rows = m - j0 - nb;
-    const int grid = rows > 0 ? (rows + kFwdRows - 1) / kFwdRows : 1;
-    CountLaunch(); TrsvFwdStepKernel<<<grid, 256, kTrsvSmem, s>>>(m, j0, nb, dL, ldl, dX, ldx, Z, m, nrhs);
+  if (cudaMallocAsync(&Z, sizeof(double) * (mz + (size_t)nrhs + 1), s) != cudaSuccess) return (int)cudaErrorMemoryAllocation;
+  int* tickets = reinterpret_cast<int*>(Z + mz);  // 2 * nrhs ints
+  CountLaunch(); WaveInitKernel<<<(unsigned)((std::max<size_t>(mz, 2 * (size_t)nrhs) + 255) / 256), 256, 0, s>>>(Z, (long)mz, tickets, 2 * nrhs);
+  for (int k = 0; k < nrhs; k++) {
+    CountLaunch(); TrsvFwdPollKernel<<<nblk, 512, kWaveSmem, s>>>(m, dL, ldl, dX + (long)k * ldx, Z + (size_t)k * m, tickets + 2 * k);
   }
   if (signs) {
     CountLaunch(); ApplySignsKernel<<<(m + 255) / 256, 256, 0, s>>>(m, nrhs, signs, Z, m);
   }
-  // backward: L^T x = z
-  for (int k = nblk - 1; k >= 0; k--) {
-    const int j0 = k * kNB, nb = min(kNB, m - j0);
-    const int grid = j0 > 0 ? (j0 + 31) / 32 : 1;
-    CountLaunch(); TrsvBwdStepKernel<<<grid, 256, kTrsvSmem, s>>>(j0, nb, dL, ldl, Z, m, dX, ldx, nrhs);
+  for (int k = 0; k < nrhs; k++) {
+    CountLaunch(); WaveInitKernel<<<(m + 255) / 256, 256, 0, s>>>(dX + (long)k * ldx, m, nullptr, 0);
+    CountLaunch(); TrsvBwdPollKernel<<<nblk, 512, kWaveSmem, s>>>(m, dL, ldl, Z + (size_t)k * m, dX + (long)k * ldx, tickets + 2 * k + 1);
   }
   cudaFreeAsync(Z, s);
   return LaunchStatus();
-}
-
-void cxb_set_trsv_mode(int mode) { g_trsv_mode = mode; }
-void cxb_set_potrf_mode(int mode) {
-  g_potrf_mode = mode & 1;
-  g_potrf_lookahead = (mode & 2) ? 0 : 1;
 }
 
 int cxb_potrs_lower(void* stream, int m, const double* dL, long ldl, double* dX, long ldx, int nrhs) {
@@ -1353,7 +867,7 @@ int cxb_ldlt_lower(void* stream, int N, double* dK, long ldk, double* d_signs, d
   for (int i0 = 0; i0 < N; i0 += kNB) {
     const int nb = min(kNB, N - i0);
     double* Kii = dK + (long)i0 * ldk + i0;
-    CountLaunch(); PotrfDiagKernel<true><<<1, 512, kDiagSmem, s>>>(nb, Kii, ldk, i0, d_info, d_signs);
+    CountLaunch(); LdltDiagKernel<<<1, 512, kDiagSmem, s>>>(nb, Kii, ldk, i0, d_info, d_signs);
     const int rows = N - i0 - nb;
     if (rows <= 0) continue;
     double* A21 = Kii + nb;
@@ -1382,7 +896,7 @@ int cxb_ldlt_partial(void* stream, int rows, int cols, double* dF, long ld, doub
   for (int i0 = 0; i0 < cols; i0 += kNB) {
     const int nb = min(kNB, cols - i0);
     double* Kii = dF + (long)i0 * ld + i0;
-    CountLaunch(); PotrfDiagKernel<true><<<1, 512, kDiagSmem, s>>>(nb, Kii, ld, i0, d_info, d_signs);
+    CountLaunch(); LdltDiagKernel<<<1, 512, kDiagSmem, s>>>(nb, Kii, ld, i0, d_info, d_signs);
     const int below = rows - i0 - nb;
     if (below <= 0) continue;
     double* A21 = Kii + nb;

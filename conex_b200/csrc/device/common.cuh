@@ -35,6 +35,33 @@ inline bool FirstUseOnCurrentDevice(std::atomic<unsigned long long>& mask) {
   return true;
 }
 
+// A high-priority side stream and two events for a look-ahead schedule: the next panel is factored on
+// the side stream while the main stream applies the current one to the rest of the matrix. Meant to be
+// held per host thread (a Program is single-threaded; programs driven from different threads get their
+// own). Prepare() creates them on first use and re-creates them when the thread's current device changes.
+struct LookAhead {
+  cudaStream_t side = nullptr;
+  cudaEvent_t updated = nullptr, factored = nullptr;
+  int device = -1;
+  bool Prepare() {
+    int current = 0;
+    if (cudaGetDevice(&current) != cudaSuccess) return false;
+    if (side && device == current) return true;
+    if (side) {  // the thread moved to another device: streams and events belong to the old one
+      cudaStreamDestroy(side);
+      cudaEventDestroy(updated);
+      cudaEventDestroy(factored);
+      side = nullptr;
+    }
+    device = current;
+    int lo = 0, hi = 0;
+    cudaDeviceGetStreamPriorityRange(&lo, &hi);
+    if (cudaStreamCreateWithPriority(&side, cudaStreamNonBlocking, hi) != cudaSuccess) return false;
+    return cudaEventCreateWithFlags(&updated, cudaEventDisableTiming) == cudaSuccess &&
+           cudaEventCreateWithFlags(&factored, cudaEventDisableTiming) == cudaSuccess;
+  }
+};
+
 // ---- cp.async (LDGSTS) -------------------------------------------------------------------
 // 16-byte copy with zero fill of the bytes beyond src_bytes (0, 8 or 16).
 __device__ __forceinline__ void CpAsync16(void* smem, const void* gmem, int src_bytes) {

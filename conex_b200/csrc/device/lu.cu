@@ -376,31 +376,8 @@ __global__ void ResetInfoKernel2(int* info) { *info = 0; }
 }  // namespace
 
 namespace {
-// Per host thread: a high-priority side stream for the look-ahead of LuFactor (see cholesky.cu for the same scheme).
-struct LuLookAhead {
-  cudaStream_t side = nullptr;
-  cudaEvent_t updated = nullptr, factored = nullptr;
-  int device = -1;
-  bool Prepare() {
-    int current = 0;
-    if (cudaGetDevice(&current) != cudaSuccess) return false;
-    if (side && device == current) return true;
-    if (side) {
-      cudaStreamDestroy(side);
-      cudaEventDestroy(updated);
-      cudaEventDestroy(factored);
-      side = nullptr;
-    }
-    device = current;
-    int lo = 0, hi = 0;
-    cudaDeviceGetStreamPriorityRange(&lo, &hi);
-    if (cudaStreamCreateWithPriority(&side, cudaStreamNonBlocking, hi) != cudaSuccess) return false;
-    return cudaEventCreateWithFlags(&updated, cudaEventDisableTiming) == cudaSuccess &&
-           cudaEventCreateWithFlags(&factored, cudaEventDisableTiming) == cudaSuccess;
-  }
-};
-thread_local LuLookAhead t_lu_lookahead;
-int g_lu_lookahead = 1;  // cxb_set_lu_mode(0): sequential schedule (A/B)
+// Side stream of LuFactor's look-ahead, separate from the Cholesky's.
+thread_local LookAhead t_lu_lookahead;
 
 void LaunchPanel(cudaStream_t s, int n, int j0, int nb, double* A, long lda, int* ipiv, int* info) {
   // sub-panel width by what fits on chip: 8 columns up to 3200 rows, 4 up to 6400, else the global-memory kernel
@@ -437,8 +414,8 @@ int ApplyPanel(cudaStream_t s, int n, int j0, int nb, double* A, long lda, const
 int LuFactor(cudaStream_t s, int n, double* A, long lda, int* ipiv, int* info) {
   ConfigureOnce();
   CountLaunch(); ResetInfoKernel2<<<1, 1, 0, s>>>(info);
-  LuLookAhead& la = t_lu_lookahead;
-  const bool ahead = g_lu_lookahead && n > 4 * kLuNB && la.Prepare();
+  LookAhead& la = t_lu_lookahead;
+  const bool ahead = n > 4 * kLuNB && la.Prepare();
   LaunchPanel(s, n, 0, min(kLuNB, n), A, lda, ipiv, info);
   for (int j0 = 0; j0 < n; j0 += kLuNB) {
     const int nb = min(kLuNB, n - j0);
@@ -529,8 +506,6 @@ int PadeExpm(cudaStream_t s, int n, const double* X, double* out, double* work, 
 using namespace cxb;
 
 extern "C" {
-
-void cxb_set_lu_mode(int lookahead) { g_lu_lookahead = lookahead; }
 
 size_t cxb_geodesic_worksize(int n) { return (size_t)4 * n * n; }
 

@@ -135,15 +135,6 @@ int cxb_front_backward(void* stream, int p, int sk, const double* dL21, long ld,
 /* ---- K5: triangular solves with the Cholesky factor (block_triangular_operations.cc:114-182):
  * X <- L^{-T} L^{-1} X for nrhs right-hand sides (columns of dX, leading dimension ldx). */
 int cxb_potrs_lower(void* stream, int m, const double* dL, long ldl, double* dX, long ldx, int nrhs);
-/* 0 (default): each sweep is ONE launch — a wavefront over the 128-row blocks, L streamed exactly once,
- * solution blocks handed from CTA to CTA through release/acquire flags; 1: one launch per block and
- * direction (the earlier scheme). Process-wide; for A/B measurements only. */
-void cxb_set_trsv_mode(int mode);
-/* 0 (default): the 128 x 128 diagonal blocks of the factorisation are factored by the blocked kernel
- * (32-wide sub-blocks, warp-shuffle factor); 1: by the rank-1 kernel with two barriers per column.
- * Adding 2 turns the look-ahead off (orders above 1536 factor panel J + 1 on a high-priority side
- * stream while panel J updates the rest of the trailing matrix). Process-wide; for A/B measurements. */
-void cxb_set_potrf_mode(int mode);
 
 /* ---- K4: diagonally pivoted, regularised LDL^T (block_triangular_operations.cc:315-349 +
  * Eigen::RLDLT, RLDLT.h:297-431) for KKT systems with equality constraints.
@@ -242,8 +233,6 @@ int cxb_pade_expm(void* stream, int n, const double* d_X, double* d_out, double*
 /* Partial-pivot LU solve A X = B (A n x n destroyed, B n x nrhs overwritten by X). */
 int cxb_lu_solve(void* stream, int n, double* dA, long lda, int nrhs, double* dB, long ldb,
                  int* d_ipiv, int* d_info);
-/* A/B switch of the LU factorisation's schedule: 1 (default) = look-ahead of one panel on a side stream, 0 = sequential. */
-void cxb_set_lu_mode(int lookahead);
 
 /* ---- small vector / matrix helpers used by the host loop -------------------------------------*/
 /* W <- I (psd_constraint.cc:92-95) */

@@ -1,8 +1,8 @@
 #!/usr/bin/env python
 """Iteration logs of BASELINE config 1 (n = 50, m = 100): oracle (BLAS and plain-loop summation) and the
-device with both triangular-solve schemes, side by side — how far the per-step trajectory is determined
-at all (see tests/test_gpu_solve.py::oracle_trajectory_horizon)."""
-import ctypes as C
+device, side by side — how far the per-step trajectory is determined at all
+(see tests/test_gpu_solve.py::oracle_trajectory_horizon). Then the accuracy of the device's Cholesky and
+solve against an extended-precision reference on ill-conditioned matrices."""
 import os
 import sys
 
@@ -14,31 +14,17 @@ from harness import oracle, random_dense_lmi  # noqa: E402
 mats, Cm = random_dense_lmi(50, 100, 1)
 ora = oracle()
 dev = devlib.product()
-dev.lib.cxb_set_trsv_mode.argtypes = [C.c_int]
-dev.lib.cxb_set_trsv_mode.restype = None
-dev.lib.cxb_set_potrf_mode.argtypes = [C.c_int]
-dev.lib.cxb_set_potrf_mode.restype = None
-
-
-def modes(trsv, potrf):
-    dev.lib.cxb_set_trsv_mode(trsv)
-    dev.lib.cxb_set_potrf_mode(potrf)
-
 
 logs = {}
 for name, L, setup in (("oracle/blas", ora, lambda: ora.lib.ORACLE_ForcePlainLoops(0)),
                        ("oracle/loops", ora, lambda: ora.lib.ORACLE_ForcePlainLoops(1)),
-                       ("dev wave+blocked", dev, lambda: modes(0, 0)),
-                       ("dev step+blocked", dev, lambda: modes(1, 0)),
-                       ("dev wave+rank1", dev, lambda: modes(0, 1)),
-                       ("dev step+rank1", dev, lambda: modes(1, 1))):
+                       ("device", dev, lambda: None)):
     setup()
     P = L.program()
     P.add_dense_lmi(mats, Cm)
     P.maximize(P.feasible_objective(), L.default_config(prepare_dual_variables=1))
     logs[name] = P.iteration_log()
 ora.lib.ORACLE_ForcePlainLoops(0)
-modes(0, 0)
 names = list(logs)
 print("step " + " ".join(f"{n:>28s}" for n in names))
 for i in range(max(len(v) for v in logs.values())):
@@ -66,7 +52,6 @@ def reference_cholesky(H):
     return Lx
 
 
-vp = C.c_void_p
 for m, cond in ((100, 1e4), (100, 1e10), (300, 1e10), (1000, 1e8)):
     rng = np.random.default_rng(m)
     Q, _ = np.linalg.qr(rng.standard_normal((m, m)))
@@ -79,17 +64,13 @@ for m, cond in ((100, 1e4), (100, 1e10), (300, 1e10), (1000, 1e8)):
     xref = np.linalg.solve(H, b)
     line = [f"m={m} cond={cond:.0e}: LAPACK |L-Lx|={np.abs(np.linalg.cholesky(H) - Lx).max():.2e} "
             f"x-err {np.abs(xref - xtrue).max():.2e}"]
-    for potrf in (0, 1):
-        for trsv in (0, 1):
-            modes(trsv, potrf)
-            dH = devlib.to_dev(np.tril(H))
-            info = devlib.izeros(1)
-            assert dev.lib.cxb_potrf_lower(None, m, devlib.ptr(dH), m, None, devlib.ptr(info)) == 0
-            Ld = np.tril(devlib.from_dev(dH))
-            dx = devlib.to_dev(b)
-            assert dev.lib.cxb_potrs_lower(None, m, devlib.ptr(dH), m, devlib.ptr(dx), m, 1) == 0
-            xd = devlib.from_dev(dx)
-            line.append(f"potrf{potrf}/trsv{trsv}: info={int(info.cpu()[0])} |L-Lx|={np.abs(Ld - Lx).max():.2e} "
-                        f"x-err {np.abs(xd - xtrue).max():.2e}")
+    dH = devlib.to_dev(np.tril(H))
+    info = devlib.izeros(1)
+    assert dev.lib.cxb_potrf_lower(None, m, devlib.ptr(dH), m, None, devlib.ptr(info)) == 0
+    Ld = np.tril(devlib.from_dev(dH))
+    dx = devlib.to_dev(b)
+    assert dev.lib.cxb_potrs_lower(None, m, devlib.ptr(dH), m, devlib.ptr(dx), m, 1) == 0
+    xd = devlib.from_dev(dx)
+    line.append(f"device: info={int(info.cpu()[0])} |L-Lx|={np.abs(Ld - Lx).max():.2e} "
+                f"x-err {np.abs(xd - xtrue).max():.2e}")
     print(" | ".join(line))
-modes(0, 0)

@@ -20,10 +20,6 @@ import conex_b200.binding as dev  # noqa: E402
 import torch  # noqa: E402
 
 L = dev.product().lib
-L.cxb_set_trsv_mode.argtypes = [C.c_int]
-L.cxb_set_trsv_mode.restype = None
-L.cxb_set_potrf_mode.argtypes = [C.c_int]
-L.cxb_set_potrf_mode.restype = None
 vp = C.c_void_p
 f64 = dict(dtype=torch.float64, device="cuda")
 
@@ -90,26 +86,17 @@ def prof_chol(s, reps, out, sizes):
             Hwork.copy_(H)
 
         medc, bestc = timed(copy_only, reps)
-        variants = ((3, "rank-1 diagonal kernel, sequential"), (2, "blocked diagonal kernel, sequential"),
-                    (0, "blocked diagonal kernel + look-ahead (default)"))
-        for mode, name in (variants if reps > 1 else variants[-1:]):
-            L.cxb_set_potrf_mode(mode)
-            medf, bestf = timed(factor, reps)
-            assert int(info.cpu()[0]) == 0
-            t = bestf - bestc
-            out.append(dict(kernel=f"K3 cxb_potrf_lower ({name})", shape=f"m = {m}", ms=t,
-                            algorithmic_flops=m ** 3 / 3.0, TFLOPs=m ** 3 / 3.0 / (t * 1e-3) / 1e12))
-        L.cxb_set_potrf_mode(0)
+        medf, bestf = timed(factor, reps)
+        assert int(info.cpu()[0]) == 0
+        t = bestf - bestc
+        out.append(dict(kernel="K3 cxb_potrf_lower", shape=f"m = {m}", ms=t,
+                        algorithmic_flops=m ** 3 / 3.0, TFLOPs=m ** 3 / 3.0 / (t * 1e-3) / 1e12))
         x = torch.rand(m, **f64)
         reps_solve = max(reps, 5 if reps > 1 else 1) * (4 if reps > 1 else 1)
-        for mode, name, launches in ((1, "one launch per block", 2 * ((m + 127) // 128)), (0, "wavefront, flags", 2),
-                                     (2, "wavefront, solution polled (default)", 4)):
-            L.cxb_set_trsv_mode(mode)
-            med, best = timed(lambda: L.cxb_potrs_lower(vp(s), m, vp(Hwork.data_ptr()), ld, vp(x.data_ptr()), m, 1), reps_solve)
-            out.append(dict(kernel=f"K5 cxb_potrs_lower ({name})", shape=f"m = {m}, 1 rhs", ms=med, best_ms=best,
-                            algorithmic_bytes=8.0 * m * m, GBps=8.0 * m * m / (best * 1e-3) / 1e9,
-                            launches=launches))
-        L.cxb_set_trsv_mode(2)
+        med, best = timed(lambda: L.cxb_potrs_lower(vp(s), m, vp(Hwork.data_ptr()), ld, vp(x.data_ptr()), m, 1), reps_solve)
+        # launches: sentinel fill + forward sweep, sentinel fill + backward sweep
+        out.append(dict(kernel="K5 cxb_potrs_lower", shape=f"m = {m}, 1 rhs", ms=med, best_ms=best,
+                        algorithmic_bytes=8.0 * m * m, GBps=8.0 * m * m / (best * 1e-3) / 1e9, launches=4))
         del H, Hwork, x
         torch.cuda.empty_cache()
 
