@@ -323,7 +323,13 @@ class Conex:
 class ConexBatch:
     """Many structurally identical `Conex` programs solved in lock step on one GPU
     (CONEXB200_CreateBatch / CONEXB200_BatchMaximize, include/conex_b200.h). No counterpart in the
-    reference, which solves such programs one after the other."""
+    reference, which solves such programs one after the other.
+
+    The programs may combine LP, second-order and dense LMI cones on all variables with equality
+    constraints (e.g. the lb == ub rows of AddLinearInequalities, on any subset of the variables);
+    every program must have the same constraints in the same order. With equality constraints the
+    KKT systems are factored by a batched regularised LDL^T, and iterative refinement, or a line
+    search on programs of LP cones and equalities only, is refused."""
 
     def __init__(self, programs):
         self.count = len(programs)

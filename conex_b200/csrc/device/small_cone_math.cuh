@@ -1139,5 +1139,103 @@ CXB_HD void SmallPotrs(T& t, int N, const double* L, long ld, double* x, double*
   t.par(N, [&](int i) { x[i] = sx[i]; });
 }
 
+// =================================================================================================
+// Small KKT system with equality multipliers (N = variables + multipliers, symmetric indefinite): the regularised
+// LDL^T of Eigen::RLDLT (RLDLT.h:297-431) as L S L^T, S = diag(+-1), |D|^{1/2} folded into L — the arithmetic of
+// cxb_sym_permute_lower + cxb_ldlt_lower (cholesky.cu, LdltDiagKernel) for one program, in shared memory.
+// =================================================================================================
+// The pivot that Eigen::RLDLT's left-looking algorithm takes at step k is the largest |d| among positions k.. of
+// the CURRENT arrangement (lowest position on ties), swapped to position k; those entries are still the original
+// diagonal, so the whole order follows from diag(K) (host RldltPivotOrder, cone_program.cc). A selection with
+// swaps, not a stable sort. One warp: a shuffle arg-max per step. sd: the N |d| (shared, permuted in place);
+// at[i]: original index at position i.
+template <class W>
+CXB_HD void RldltPivotOrder(W& w, int N, double* sd, int* at) {
+  for (int k = 0; k + 1 < N; k++) {
+    double v;
+    const int p = k + w.argmax_first(N - k, [&](int i) { return sd[k + i]; }, &v);
+    if (p != k) {
+      w.single([&]() {
+        const double d = sd[k];
+        sd[k] = sd[p];
+        sd[p] = d;
+        const int a = at[k];
+        at[k] = at[p];
+        at[p] = a;
+      });
+    }
+  }
+}
+
+// A pivot with |d| <= 1e-9 is used as -1e-9 when d < 0 and as +1e-9 otherwise (RLDLT.h:378-389).
+CXB_HD double RegularisedPivot(double d) { return (fabs(d) > 1e-9) ? d : ((d < 0) ? -1e-9 : 1e-9); }
+
+// K (N x N, lower triangle read, ld ldk) is not modified. Writes the lower triangle of L (ldl), perm[i] = original
+// index at pivot position i and signs = S; returns 1 when some pivot was regularised, else 0 (it never fails).
+// sH: N*N doubles, sd: N doubles, at: N ints, all shared.
+template <class T>
+CXB_HD int SmallLdlt(T& t, int N, const double* K, long ldk, double* L, long ldl, int* perm, double* signs,
+                     double* sH, double* sd, int* at) {
+  t.par(N, [&](int i) {
+    sd[i] = fabs(K[(long)i * ldk + i]);
+    at[i] = i;
+  });
+  t.warp0([&](auto& w) { RldltPivotOrder(w, N, sd, at); });
+  // P K P^T from the lower triangle of K, the permutation fused into the load
+  const Divider by_N(N);
+  t.par(N * N, [&](int e) {
+    const int c = by_N.quot(e), r = e - c * N;
+    if (r >= c) {
+      const int i = at[r], j = at[c];
+      sH[e] = (i >= j) ? K[(long)j * ldk + i] : K[(long)i * ldk + j];
+    }
+  });
+  int regularised = 0;
+  for (int j = 0; j < N; j++) {
+    // the diagonal keeps the (unregularised) pivot until the end, as in SmallPotrf
+    double d = sH[j * N + j];
+    if (!(fabs(d) > 1e-9)) regularised = 1;
+    d = RegularisedPivot(d);
+    const double sign = (d < 0) ? -1.0 : 1.0;
+    const double inv = 1.0 / sqrt(fabs(d));
+    // column j of L = sign a_j / sqrt|d|; the update of entry (r, c) is sign a_r a_c / |d| = L_rj (sign L_cj)
+    t.par(N - j - 1, [&](int i) { sH[j * N + j + 1 + i] *= sign * inv; });
+    const int w = N - j - 1;
+    t.par2(
+        w, w, [&](int i) { return sH[j * N + j + 1 + i]; },
+        [&](int i, int c, double lr) {
+          if (i >= c) sH[(j + 1 + c) * N + j + 1 + i] -= lr * (sign * sH[j * N + j + 1 + c]);
+        });
+  }
+  t.par(N * N, [&](int e) {
+    const int c = by_N.quot(e), r = e - c * N;
+    if (r > c) L[(long)c * ldl + r] = sH[e];
+    if (r == c) {
+      const double d = RegularisedPivot(sH[e]);
+      L[(long)c * ldl + r] = sqrt(fabs(d));
+      signs[r] = (d < 0) ? -1.0 : 1.0;
+      perm[r] = at[r];
+    }
+  });
+  return regularised;
+}
+
+// x <- P^T L^{-T} S L^{-1} P x with the factors of SmallLdlt. sx: N doubles shared.
+template <class T>
+CXB_HD void SmallLdltSolve(T& t, int N, const double* L, long ld, const int* perm, const double* signs, double* x,
+                           double* sx) {
+  t.par(N, [&](int i) { sx[i] = x[perm[i]]; });
+  for (int j = 0; j < N; j++) {
+    const double xj = sx[j] / L[(long)j * ld + j];
+    t.par(N - j - 1, [&](int i) { sx[j + 1 + i] -= L[(long)j * ld + j + 1 + i] * xj; });
+  }
+  t.par(N, [&](int j) { sx[j] = signs[j] * (sx[j] / L[(long)j * ld + j]); });
+  for (int j = N - 1; j >= 0; j--) {
+    const double s = t.sum(N - j - 1, [&](int i) { return L[(long)j * ld + j + 1 + i] * sx[j + 1 + i]; });
+    t.single([&]() { sx[j] = (sx[j] - s) / L[(long)j * ld + j]; });
+  }
+  t.par(N, [&](int i) { x[perm[i]] = sx[i]; });
+}
+
 }  // namespace small
 }  // namespace cxb

@@ -354,6 +354,41 @@ __global__ void __launch_bounds__(kThreads) PotrsKernel(int batch, long per, int
   small::SmallPotrs(t, N, L + p * lstride, ldl, X + p * xstride, base + 64);
 }
 
+// Shared memory (doubles) of the regularised LDL^T: the permuted copy, the |diagonal| and the pivot order (ints).
+__host__ __device__ inline long LdltSmemDoubles(int N) { return (long)N * N + N + (N + 1) / 2; }
+
+template <bool WARP>
+__global__ void __launch_bounds__(kThreads) LdltKernel(int batch, long per, int N, const double* K, long ldk,
+                                                       long kstride, double* L, long ldl, long lstride, int* perm,
+                                                       long pstride, double* signs, long sstride, int* info,
+                                                       const int* active) {
+  extern __shared__ double sm[];
+  int p;
+  double* base;
+  if (!Slot<WARP>(batch, per, sm, active, &p, &base)) return;
+  auto t = TeamOf<WARP>::Make(base);
+  double* sH = base + 64;
+  const int regularised = small::SmallLdlt(t, N, K + p * kstride, ldk, L + p * lstride, ldl, perm + p * pstride,
+                                           signs + p * sstride, sH, sH + (long)N * N,
+                                           reinterpret_cast<int*>(sH + (long)N * N + N));
+  // written here rather than inside SmallLdlt: a pointer live across the whole factorisation was spilled
+  t.single([&]() { info[p] = regularised; });
+}
+
+template <bool WARP>
+__global__ void __launch_bounds__(kThreads) LdltSolveKernel(int batch, long per, int N, const double* L, long ldl,
+                                                            long lstride, const int* perm, long pstride,
+                                                            const double* signs, long sstride, double* X,
+                                                            long xstride, const int* active) {
+  extern __shared__ double sm[];
+  int p;
+  double* base;
+  if (!Slot<WARP>(batch, per, sm, active, &p, &base)) return;
+  auto t = TeamOf<WARP>::Make(base);
+  small::SmallLdltSolve(t, N, L + p * lstride, ldl, perm + p * pstride, signs + p * sstride, X + p * xstride,
+                        base + 64);
+}
+
 __global__ void LincombKernel(int n, const double* a, const double* x, long xs, const double* b,
                               const double* y, long ys, const double* c, const double* z, long zs,
                               double* out, long os, const int* active) {
@@ -778,6 +813,44 @@ int cxb_small_potrs(void* stream, int batch, int N, const double* dL, long ldl, 
     if (rc) return rc;
     CountLaunch(); PotrsKernel<false><<<g.grid, g.threads, g.smem, AsStream(stream)>>>(batch, g.per, N, dL, ldl, lstride, dX,
                                                                                     xstride, d_active);
+  }
+  return LaunchStatus();
+}
+
+int cxb_small_ldlt(void* stream, int batch, int N, const double* dK, long ldk, long kstride, double* dL, long ldl,
+                   long lstride, int* d_perm, long pstride, double* d_signs, long sstride, int* d_info,
+                   const int* d_active) {
+  if (batch <= 0 || N <= 0) return 0;
+  const Geometry g = MakeGeometry(batch, sizeof(double) * (64 + (size_t)LdltSmemDoubles(N)));
+  if (g.warp) {
+    int rc = EnsureSmem(LdltKernel<true>, g.smem);
+    if (rc) return rc;
+    CountLaunch(); LdltKernel<true><<<g.grid, g.threads, g.smem, AsStream(stream)>>>(
+        batch, g.per, N, dK, ldk, kstride, dL, ldl, lstride, d_perm, pstride, d_signs, sstride, d_info, d_active);
+  } else {
+    int rc = EnsureSmem(LdltKernel<false>, g.smem);
+    if (rc) return rc;
+    CountLaunch(); LdltKernel<false><<<g.grid, g.threads, g.smem, AsStream(stream)>>>(
+        batch, g.per, N, dK, ldk, kstride, dL, ldl, lstride, d_perm, pstride, d_signs, sstride, d_info, d_active);
+  }
+  return LaunchStatus();
+}
+
+int cxb_small_ldlt_solve(void* stream, int batch, int N, const double* dL, long ldl, long lstride, const int* d_perm,
+                         long pstride, const double* d_signs, long sstride, double* dX, long xstride,
+                         const int* d_active) {
+  if (batch <= 0 || N <= 0) return 0;
+  const Geometry g = MakeGeometry(batch, sizeof(double) * (64 + (size_t)N), /*chain_only=*/true);
+  if (g.warp) {
+    int rc = EnsureSmem(LdltSolveKernel<true>, g.smem);
+    if (rc) return rc;
+    CountLaunch(); LdltSolveKernel<true><<<g.grid, g.threads, g.smem, AsStream(stream)>>>(
+        batch, g.per, N, dL, ldl, lstride, d_perm, pstride, d_signs, sstride, dX, xstride, d_active);
+  } else {
+    int rc = EnsureSmem(LdltSolveKernel<false>, g.smem);
+    if (rc) return rc;
+    CountLaunch(); LdltSolveKernel<false><<<g.grid, g.threads, g.smem, AsStream(stream)>>>(
+        batch, g.per, N, dL, ldl, lstride, d_perm, pstride, d_signs, sstride, dX, xstride, d_active);
   }
   return LaunchStatus();
 }

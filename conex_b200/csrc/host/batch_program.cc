@@ -7,6 +7,7 @@
 #include "../../../include/conex_b200_device.h"
 #include "dense_lmi_constraint.h"
 #include "divergence.h"
+#include "equality_constraint.h"
 #include "small_cone_constraint.h"
 
 namespace conex {
@@ -22,6 +23,13 @@ struct ConeSlot {
   int rank = 0;
 };
 
+// An equality block A y[variables] = b: rank 0, no launches of its own. Its multipliers are the KKT unknowns
+// m + offset .. m + offset + rows - 1; its rows of H, AQc and AW are constant and written once per batch.
+struct EqualitySlot {
+  int rows = 0, offset = 0;
+  std::vector<int> variables;  // the columns of A
+};
+
 size_t Align4(size_t n) { return (n + 3) & ~static_cast<size_t>(3); }
 
 }  // namespace
@@ -30,15 +38,21 @@ struct BatchProgram::Impl {
   DeviceContext ctx;
   std::vector<ConeSlot> cones;
   std::vector<cxb_small_cone> descs;  // the descriptors of `cones`, contiguous, for the fused launches
-  int B = 0, m = 0;
+  std::vector<EqualitySlot> equalities;
+  std::vector<int> slot_of;  // constraint number -> index into `cones`, or -1 for an equality block
+  // N = m + multipliers: the order of the KKT systems (reference constraint_manager.h:42-48)
+  int B = 0, m = 0, N = 0, multipliers = 0;
   long ldh = 0;
   size_t vstride = 0;
   // per-program Newton system and vectors
   DeviceBuffer<double> H, AW, AQc, scal, b, y, y2;
+  // with multipliers: the factors of the regularised LDL^T (H itself is kept, its equality rows are constant)
+  DeviceBuffer<double> L, signs;
+  DeviceBuffer<int> perm;
   // per-program scalars exchanged with the host each phase
   DeviceBuffer<double> coef;   // 3 x B coefficient arrays | B c_weights | B step sizes
   DeviceBuffer<double> out;    // cone outputs: B x ncones x 4, then B x 4 dots/scalars
-  DeviceBuffer<int> info;      // B Cholesky flags | B Padé flags
+  DeviceBuffer<int> info;      // B Cholesky flags | B Padé flags (| B regularisation flags of the LDL^T)
   DeviceBuffer<int> mask;      // B active | B mu-update
   PinnedBuffer<double> hcoef, hout;
   PinnedBuffer<int> hinfo, hmask;
@@ -64,11 +78,31 @@ struct BatchProgram::Impl {
   void Assemble(const int* active) {
     bool first = true;
     for (auto& c : cones) {
-      DeviceCheck(cxb_small_schur(s(), B, &c.desc, H.get(), ldh, ldh * m, AW.get(), AQc.get(), vstride,
+      DeviceCheck(cxb_small_schur(s(), B, &c.desc, H.get(), ldh, ldh * N, AW.get(), AQc.get(), vstride,
                                   scal.get(), 2, first ? 0 : 1, active),
                   "cxb_small_schur");
       first = false;
     }
+  }
+  // The KKT factor and solve: Cholesky without multipliers, the regularised LDL^T with them, which never fails
+  // (kkt_solver.cc:172-199: the input decides).
+  void Factor(const int* active) {
+    if (multipliers == 0) {
+      DeviceCheck(cxb_small_potrf(s(), B, N, H.get(), ldh, ldh * N, info.get(), active), "cxb_small_potrf");
+      return;
+    }
+    DeviceCheck(cxb_small_ldlt(s(), B, N, H.get(), ldh, ldh * N, L.get(), ldh, ldh * N, perm.get(), N, signs.get(),
+                               N, info.get() + 2 * static_cast<size_t>(B), active),
+                "cxb_small_ldlt");
+  }
+  void Solve(double* x, const int* active) {
+    if (multipliers == 0) {
+      DeviceCheck(cxb_small_potrs(s(), B, N, H.get(), ldh, ldh * N, x, vstride, active), "cxb_small_potrs");
+      return;
+    }
+    DeviceCheck(cxb_small_ldlt_solve(s(), B, N, L.get(), ldh, ldh * N, perm.get(), N, signs.get(), N, x, vstride,
+                                     active),
+                "cxb_small_ldlt_solve");
   }
 };
 
@@ -80,18 +114,36 @@ BatchProgram::BatchProgram(const std::vector<Program*>& programs) : impl_(std::m
   m_ = d.m = programs[0]->GetNumberOfVariables();
   const int m = m_;
   // ---- structure of program 0; every other program must match it ------------------------------
+  constexpr int kEquality = -1;
   struct Shape {
-    int type, n;
+    int type, n;                 // n: the order of a cone, the rows of an equality block
+    std::vector<int> variables;  // equality blocks: the columns of A
   };
   auto shape_of = [&](Container& c, Shape* sh) {
+    sh->variables.clear();
     if (auto* lp = std::any_cast<LinearConstraint>(&c.obj)) {
-      *sh = {CXB_CONE_LP, lp->order()};
+      sh->type = CXB_CONE_LP;
+      sh->n = lp->order();
     } else if (auto* soc = std::any_cast<SOCConstraint>(&c.obj)) {
-      *sh = {CXB_CONE_SOC, soc->order()};
+      sh->type = CXB_CONE_SOC;
+      sh->n = soc->order();
     } else if (auto* lmi = std::any_cast<DenseLMIConstraint>(&c.obj)) {
-      *sh = {CXB_CONE_PSD, lmi->order()};
+      sh->type = CXB_CONE_PSD;
+      sh->n = lmi->order();
+    } else if (auto* eq = std::any_cast<EqualityConstraints>(&c.obj)) {
+      // any subset of the variables, followed by the block's multipliers (Program::AddConstraint)
+      sh->type = kEquality;
+      sh->n = eq->rows();
+      const int nv = static_cast<int>(c.variables.size()) - eq->rows();
+      if (nv != eq->number_of_columns()) throw std::runtime_error("conex-b200: malformed equality block");
+      sh->variables.assign(c.variables.begin(), c.variables.begin() + nv);
+      for (int v : sh->variables) {
+        if (v < 0 || v >= m) throw std::runtime_error("conex-b200: malformed equality block");
+      }
+      return;
     } else {
-      throw std::runtime_error("conex-b200: batched solves support LP, second-order and dense LMI cones");
+      throw std::runtime_error(
+          "conex-b200: batched solves support LP, second-order and dense LMI cones and equality constraints");
     }
     if (static_cast<int>(c.variables.size()) != m) {
       throw std::runtime_error("conex-b200: batched solves need every cone on all variables");
@@ -106,14 +158,32 @@ BatchProgram::BatchProgram(const std::vector<Program*>& programs) : impl_(std::m
     shape_of(c, &sh);
     shapes.push_back(sh);
   }
-  if (shapes.empty()) throw std::runtime_error("conex-b200: batched programs have no constraints");
-  const size_t nc = shapes.size();
-  d.cones.resize(nc);
+  const size_t nconstraints = shapes.size();
+  for (const Shape& sh : shapes) {
+    if (sh.type == kEquality) {
+      EqualitySlot e;
+      e.rows = sh.n;
+      e.offset = d.multipliers;
+      e.variables = sh.variables;
+      d.multipliers += sh.n;
+      d.slot_of.push_back(-1);
+      d.equalities.push_back(std::move(e));
+    } else {
+      d.slot_of.push_back(static_cast<int>(d.cones.size()));
+      d.cones.emplace_back();
+      d.cones.back().type = sh.type;
+      d.cones.back().n = sh.n;
+    }
+  }
+  if (d.cones.empty()) throw std::runtime_error("conex-b200: batched programs have no cones");
+  if (programs[0]->NumberOfMultipliers() != d.multipliers) {
+    throw std::runtime_error("conex-b200: malformed equality blocks");
+  }
+  const int N = d.N = m + d.multipliers;
+  const size_t nc = d.cones.size();
   d.rank = 0;
   for (size_t k = 0; k < nc; k++) {
     ConeSlot& c = d.cones[k];
-    c.type = shapes[k].type;
-    c.n = shapes[k].n;
     c.m = m;
     c.rows = c.type == CXB_CONE_LP ? c.n : (c.type == CXB_CONE_SOC ? c.n + 1 : c.n * c.n);
     c.rank = c.type == CXB_CONE_LP ? c.n : (c.type == CXB_CONE_SOC ? 2 : c.n);
@@ -136,20 +206,41 @@ BatchProgram::BatchProgram(const std::vector<Program*>& programs) : impl_(std::m
     c.desc.packed = nullptr;
     c.desc.packed_stride = 0;
   }
-  // ---- pack the cone data -----------------------------------------------------------------------
+  // ---- pack the cone data; gather the equality data on the host --------------------------------------
+  const size_t nm = static_cast<size_t>(d.multipliers);
+  std::vector<double> eq_rows(nm * N * B, 0.0);  // rows m..N-1 of every H, column by column
+  std::vector<double> eq_b(nm * B, 0.0);         // AQc[m..N) of every program
+  std::vector<double> host_A;
   for (int p = 0; p < B; p++) {
     Program& prog = *programs[p];
-    if (prog.GetNumberOfVariables() != m || prog.NumberOfMultipliers() != 0 || prog.eqs.size() != nc) {
+    if (prog.GetNumberOfVariables() != m || prog.NumberOfMultipliers() != d.multipliers ||
+        prog.eqs.size() != nconstraints) {
       throw std::runtime_error("conex-b200: programs of a batch must have identical structure");
     }
-    size_t k = 0;
+    size_t k = 0, q = 0;
     for (auto& c : prog.eqs) {
       Shape sh;
       shape_of(c, &sh);
-      if (sh.type != shapes[k].type || sh.n != shapes[k].n) {
+      if (sh.type != shapes[k].type || sh.n != shapes[k].n || sh.variables != shapes[k].variables) {
         throw std::runtime_error("conex-b200: programs of a batch must have identical structure");
       }
-      ConeSlot& slot = d.cones[k];
+      if (sh.type == kEquality) {
+        // ConstructSchurComplementSystem(EqualityConstraints*) (equality_constraint.cc:13-30): A on (multipliers,
+        // variables), zeros elsewhere in these rows of H, including the multiplier block; b in AQc, zeros in AW
+        const EqualitySlot& e = d.equalities[q++];
+        auto* eq = std::any_cast<EqualityConstraints>(&c.obj);
+        const size_t nv = e.variables.size();
+        host_A.resize(static_cast<size_t>(e.rows) * nv);
+        d.ctx.Download(host_A.data(), eq->device_A(), host_A.size());
+        d.ctx.Download(eq_b.data() + nm * p + e.offset, eq->device_b(), e.rows);
+        for (size_t j = 0; j < nv; j++) {
+          double* col = eq_rows.data() + (static_cast<size_t>(p) * N + e.variables[j]) * nm + e.offset;
+          for (int r = 0; r < e.rows; r++) col[r] = host_A[j * e.rows + r];
+        }
+        k++;
+        continue;
+      }
+      ConeSlot& slot = d.cones[d.slot_of[k]];
       const size_t per = static_cast<size_t>(slot.rows) * (m + 1);
       double* dst = slot.data.get() + per * p;
       if (sh.type == CXB_CONE_PSD) {
@@ -197,9 +288,14 @@ BatchProgram::BatchProgram(const std::vector<Program*>& programs) : impl_(std::m
     for (auto& c : d.cones) d.descs.push_back(c.desc);
   }
   // ---- Newton-system storage ------------------------------------------------------------------------
-  d.ldh = static_cast<long>(Align4(m));
-  d.vstride = Align4(m);
-  d.H.Resize(static_cast<size_t>(d.ldh) * m * B);
+  d.ldh = static_cast<long>(Align4(N));
+  d.vstride = Align4(N);
+  d.H.Resize(static_cast<size_t>(d.ldh) * N * B);
+  if (d.multipliers) {
+    d.L.Resize(static_cast<size_t>(d.ldh) * N * B);
+    d.perm.Resize(static_cast<size_t>(N) * B);
+    d.signs.Resize(static_cast<size_t>(N) * B);
+  }
   d.AW.Resize(d.vstride * B);
   d.AQc.Resize(d.vstride * B);
   d.scal.Resize(2 * static_cast<size_t>(B));
@@ -208,25 +304,43 @@ BatchProgram::BatchProgram(const std::vector<Program*>& programs) : impl_(std::m
   d.y2.Resize(d.vstride * B);
   d.coef.Resize(5 * static_cast<size_t>(B));
   d.out.Resize(static_cast<size_t>(B) * (4 * nc + 4));
-  d.info.Resize(2 * static_cast<size_t>(B));
+  d.info.Resize((d.multipliers ? 3 : 2) * static_cast<size_t>(B));
   d.mask.Resize(2 * static_cast<size_t>(B));
   d.hcoef.Reserve(std::max<size_t>(5 * static_cast<size_t>(B), d.vstride * B));
   d.hout.Reserve(std::max<size_t>(static_cast<size_t>(B) * (4 * nc + 4), d.vstride * B));
   d.hinfo.Reserve(2 * static_cast<size_t>(B));
   d.hmask.Reserve(2 * static_cast<size_t>(B));
   results_.assign(B, BatchResult());
+  if (d.multipliers) {
+    // The constant rows m..N-1 of every H (H[p] is ldh x N, so column c of program p is column p N + c of one
+    // B N-column matrix), AQc[m..N) and AW[m..N). The cones' Schur kernels assign only the leading m x m block of H
+    // and the first m entries of AW / AQc, and the LDL^T leaves H as it is: these survive every Newton step.
+    cudaStream_t cs = d.ctx.cuda_stream();
+    CudaCheck(cudaMemcpy2DAsync(d.H.get() + m, sizeof(double) * d.ldh, eq_rows.data(), sizeof(double) * nm,
+                                sizeof(double) * nm, static_cast<size_t>(N) * B, cudaMemcpyHostToDevice, cs),
+              "upload of the equality rows");
+    CudaCheck(cudaMemcpy2DAsync(d.AQc.get() + m, sizeof(double) * d.vstride, eq_b.data(), sizeof(double) * nm,
+                                sizeof(double) * nm, B, cudaMemcpyHostToDevice, cs),
+              "upload of the equality right-hand sides");
+    CudaCheck(cudaMemset2DAsync(d.AW.get() + m, sizeof(double) * d.vstride, 0, sizeof(double) * nm, B, cs), "memset");
+    d.ctx.Synchronize();  // eq_rows / eq_b are pageable
+  }
 }
 
 BatchProgram::~BatchProgram() = default;
 
 int BatchProgram::DualVariableSize(int cone) const {
-  const ConeSlot& c = impl_->cones.at(cone);
+  const int k = impl_->slot_of.at(cone);
+  if (k < 0) return 0;  // an equality block has no dual variable (equality_constraint.h:9-18)
+  const ConeSlot& c = impl_->cones.at(k);
   return c.type == CXB_CONE_PSD ? c.n * c.n : c.rows;
 }
 
 void BatchProgram::GetDualVariable(int p, int cone, double* host_out) {
   Impl& d = *impl_;
-  const ConeSlot& c = d.cones.at(cone);
+  const int k = d.slot_of.at(cone);
+  if (k < 0) return;
+  const ConeSlot& c = d.cones.at(k);
   const int sz = DualVariableSize(cone);
   d.ctx.Download(host_out, c.state.get() + c.state_size * p, sz);
   const BatchResult& r = results_.at(p);
@@ -252,7 +366,7 @@ struct ProgramState {
 
 int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, double* y_out) {
   Impl& d = *impl_;
-  const int B = batch_, m = m_;
+  const int B = batch_, m = m_, N = d.N;
   const size_t nc = d.cones.size();
   const size_t vs = d.vstride;
   if (cfg.initialization_mode != CONEX_INITIALIZATION_MODE_COLDSTART) {
@@ -261,10 +375,19 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
   if (cfg.kkt_solver == CONEX_QR_FACTORIZATION) {
     throw std::runtime_error("conex-b200: the QR KKT mode is not implemented on the device");
   }
+  if (d.multipliers > 0 && cfg.iterative_refinement_iterations > 0) {
+    throw std::runtime_error(
+        "conex-b200: iterative refinement is not implemented for batched programs with equality constraints");
+  }
   if (cfg.enable_line_search) {
+    // the reference runs a line search when every constraint is an LP cone or an equality block
+    // (cone_program.h:211-216); `cones` holds no equality blocks
     bool lp_only = true;
     for (const auto& c : d.cones) lp_only = lp_only && (c.type == CXB_CONE_LP);
-    if (lp_only) throw std::runtime_error("conex-b200: enable_line_search on LP-only programs is not implemented");
+    if (lp_only) {
+      throw std::runtime_error(
+          "conex-b200: enable_line_search on programs of LP cones and equality constraints only is not implemented");
+    }
   }
   void* s = d.s();
   cudaStream_t cs = d.ctx.cuda_stream();
@@ -336,10 +459,13 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
     d.Assemble(active);
     const bool rescale = (i == 0) && cfg.enable_rescaling;
     if (rescale) {
-      DeviceCheck(cxb_batched_dot(s, B, m, d.AQc.get(), vs, d.AQc.get(), vs, dots, 4), "cxb_batched_dot");
+      DeviceCheck(cxb_batched_dot(s, B, N, d.AQc.get(), vs, d.AQc.get(), vs, dots, 4), "cxb_batched_dot");
     }
-    DeviceCheck(cxb_small_potrf(s, B, m, d.H.get(), d.ldh, d.ldh * m, d.info.get(), active), "cxb_small_potrf");
-    CudaCheck(cudaMemcpyAsync(d.hinfo.get(), d.info.get(), sizeof(int) * B, cudaMemcpyDeviceToHost, cs), "D2H info");
+    d.Factor(active);
+    if (!d.multipliers) {
+      CudaCheck(cudaMemcpyAsync(d.hinfo.get(), d.info.get(), sizeof(int) * B, cudaMemcpyDeviceToHost, cs),
+                "D2H info");
+    }
     if (rescale) {
       CudaCheck(cudaMemcpyAsync(d.hout.get(), dots, sizeof(double) * 4 * B, cudaMemcpyDeviceToHost, cs), "D2H norms");
     }
@@ -357,7 +483,7 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
         const double mu_target = (1.0 / (q.kmax * q.kmax)) * (q.b_scaling * q.c_scaling);
         q.kmax = 1.0 / std::sqrt(mu_target);
       }
-      if (d.hinfo[p] != 0) {  // Factor() failed: the solve returns unsolved (cone_program.cc:360-371)
+      if (!d.multipliers && d.hinfo[p] != 0) {  // Factor() failed: the solve returns unsolved (cone_program.cc:360-371)
         q.active = false;
         q.failed = true;
         d.hmask[p] = 0;
@@ -381,10 +507,10 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
       }
       d.UploadCoef(0, 2 * static_cast<size_t>(B));
       d.UploadCoef(3 * static_cast<size_t>(B), B);
-      DeviceCheck(cxb_batched_lincomb(s, B, m, coef_a, d.AQc.get(), vs, coef_b, d.b.get(), vs, nullptr, nullptr, 0,
+      DeviceCheck(cxb_batched_lincomb(s, B, N, coef_a, d.AQc.get(), vs, coef_b, d.b.get(), vs, nullptr, nullptr, 0,
                                       d.y.get(), vs, mu_mask),
                   "cxb_batched_lincomb");
-      DeviceCheck(cxb_small_potrs(s, B, m, d.H.get(), d.ldh, d.ldh * m, d.y.get(), vs, mu_mask), "cxb_small_potrs");
+      d.Solve(d.y.get(), mu_mask);
       DeviceCheck(cxb_small_eigen_multi(s, B, ncones, d.descs.data(), d.y.get(), vs, 0.0, coef_cw, cone_out, ostride,
                                         mu_mask),
                   "cxb_small_eigen_multi");
@@ -435,10 +561,10 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
 
     // ---- Newton direction: y = H^{-1} (k (b b_s + AQc c_s) - 2 AW) (cone_program.cc:409-414) ------
     d.UploadCoef(0, 4 * static_cast<size_t>(B));
-    DeviceCheck(cxb_batched_lincomb(s, B, m, coef_a, d.b.get(), vs, coef_b, d.AQc.get(), vs, coef_c, d.AW.get(), vs,
+    DeviceCheck(cxb_batched_lincomb(s, B, N, coef_a, d.b.get(), vs, coef_b, d.AQc.get(), vs, coef_c, d.AW.get(), vs,
                                     d.y.get(), vs, active),
                 "cxb_batched_lincomb");
-    DeviceCheck(cxb_small_potrs(s, B, m, d.H.get(), d.ldh, d.ldh * m, d.y.get(), vs, active), "cxb_small_potrs");
+    d.Solve(d.y.get(), active);
     DeviceCheck(cxb_small_prepare_multi(s, B, ncones, d.descs.data(), d.y.get(), vs, 0, 0.0, coef_cw, 1.0, cone_out,
                                         ostride, active),
                 "cxb_small_prepare_multi");
@@ -462,8 +588,8 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
     DeviceCheck(cxb_small_take_step_multi(s, B, ncones, d.descs.data(), 1.0, coef_step, 1.0, d.info.get() + B, active),
                 "cxb_small_take_step_multi");
     // ---- objectives (cone_program.cc:441-467) -------------------------------------------------------
-    DeviceCheck(cxb_batched_dot(s, B, m, d.b.get(), vs, d.y.get(), vs, dots + 0, 4), "cxb_batched_dot");
-    DeviceCheck(cxb_batched_dot(s, B, m, d.AQc.get(), vs, d.y.get(), vs, dots + 1, 4), "cxb_batched_dot");
+    DeviceCheck(cxb_batched_dot(s, B, N, d.b.get(), vs, d.y.get(), vs, dots + 0, 4), "cxb_batched_dot");
+    DeviceCheck(cxb_batched_dot(s, B, N, d.AQc.get(), vs, d.y.get(), vs, dots + 1, 4), "cxb_batched_dot");
     CudaCheck(cudaEventRecord(ev_b, cs), "cudaEventRecord");
     CudaCheck(cudaMemcpyAsync(d.hout.get(), dots, sizeof(double) * 4 * B, cudaMemcpyDeviceToHost, cs), "D2H dots");
     CudaCheck(cudaMemcpyAsync(d.hout.get() + 4 * static_cast<size_t>(B), d.scal.get(), sizeof(double) * 2 * B,
@@ -535,16 +661,16 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
     // reference cone_program.cc:500-516
     d.UploadMask(0);
     d.Assemble(active);
-    DeviceCheck(cxb_small_potrf(s, B, m, d.H.get(), d.ldh, d.ldh * m, d.info.get(), active), "cxb_small_potrf");
+    d.Factor(active);
     for (int p = 0; p < B; p++) {
       d.hcoef[p] = st[p].k * st[p].b_scaling;
       d.hcoef[B + p] = -1.0;
     }
     d.UploadCoef(0, 2 * static_cast<size_t>(B));
-    DeviceCheck(cxb_batched_lincomb(s, B, m, coef_a, d.b.get(), vs, coef_b, d.AW.get(), vs, nullptr, nullptr, 0,
+    DeviceCheck(cxb_batched_lincomb(s, B, N, coef_a, d.b.get(), vs, coef_b, d.AW.get(), vs, nullptr, nullptr, 0,
                                     d.y2.get(), vs, active),
                 "cxb_batched_lincomb");
-    DeviceCheck(cxb_small_potrs(s, B, m, d.H.get(), d.ldh, d.ldh * m, d.y2.get(), vs, active), "cxb_small_potrs");
+    d.Solve(d.y2.get(), active);
     DeviceCheck(cxb_small_prepare_multi(s, B, ncones, d.descs.data(), d.y2.get(), vs, 1, 0.0, nullptr, 0.0, cone_out,
                                         ostride, active),
                 "cxb_small_prepare_multi");

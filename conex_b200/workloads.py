@@ -73,12 +73,50 @@ def small_multicone_problem(seed, m=40, psd_blocks=3, psd_order=20, soc_cones=2,
     return cones, b
 
 
+def small_multicone_equality_problem(seed, equalities=((8, None, None),), y0_scale=0.02, **shape):
+    """small_multicone_problem with equality blocks A_eq y[variables] = b_eq added. `equalities`: one
+    (rows, variables, position) per block; variables None = all m variables in order, position None = after the
+    cones, else the block's index in the constraint list. Both sides stay strictly feasible: b_eq = A_eq y0[variables]
+    for a small y0 at which every cone slack is interior, and A_eq^T lambda0 is added to b (the cone part of the
+    primal point is unchanged, the multipliers are free). Equality entries of the returned list are
+    ("eq", A_eq, (b_eq, variables))."""
+    cones, b = small_multicone_problem(seed, **shape)
+    m = b.size
+    rng = np.random.Generator(np.random.PCG64(10 ** 6 + seed))
+    y0 = y0_scale * rng.uniform(-1.0, 1.0, size=m)
+    for kind, A, c in cones:  # the slacks at y0 are interior
+        if kind == "psd":
+            assert np.linalg.eigvalsh(c - sum(yi * Ai for yi, Ai in zip(y0, A))).min() > 0.1
+        elif kind == "soc":
+            s = c - A @ y0
+            assert s[0] - np.linalg.norm(s[1:]) > 0.1
+        else:
+            assert (c - A @ y0).min() > 0.1
+    out = list(cones)
+    blocks = []
+    for rows, variables, position in equalities:
+        v = list(range(m)) if variables is None else list(variables)
+        A_eq = rng.uniform(-1.0, 1.0, size=(rows, len(v)))
+        b_eq = A_eq @ y0[v]
+        lam0 = rng.uniform(-1.0, 1.0, size=rows)
+        np.add.at(b, v, A_eq.T @ lam0)
+        blocks.append((position, ("eq", A_eq, (b_eq, None if variables is None else v))))
+    for position, entry in blocks:
+        if position is None:
+            out.append(entry)
+        else:
+            out.insert(position, entry)
+    return out, b
+
+
 def add_cones(P, cones):
     for kind, A, c in cones:
         if kind == "psd":
             P.add_dense_lmi(A, c)
         elif kind == "soc":
             P.add_soc(A, c)
+        elif kind == "eq":
+            P.add_equality(A, c[0], c[1])
         else:
             P.add_linear(A, c)
 

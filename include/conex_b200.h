@@ -188,12 +188,16 @@ void CONEXB200_RldltPivotOrder(int n, const double* diag, int* perm);
 
 /* ---- many small programs in lock step (BASELINE config 3) ------------------------------------
  * `programs`: `count` handles built through the CONEX_* calls with identical structure (same number
- * of variables, same list of LP / second-order / dense-LMI cones, every cone on all variables, no
- * equalities). CONEXB200_CreateBatch packs their data into batched device arrays (the handles may be
- * deleted afterwards); CONEXB200_BatchMaximize solves all of them from a cold start: b and y are
- * m x count column-major HOST arrays, solved[p] / the return value follow CONEX_Maximize (1 = solved;
- * the return value is the number of solved programs, -1 on an error). Every program follows the same
- * iteration sequence it would follow through CONEX_Maximize alone. */
+ * of variables, same list of LP / second-order / dense-LMI cones, every cone on all variables, and
+ * the same equality blocks — rows, variable subset, position among the cones — e.g. the lb == ub rows
+ * of CONEX_AddLinearInequalities; at least one cone). CONEXB200_CreateBatch packs their data into
+ * batched device arrays (the handles may be deleted afterwards); it returns NULL for mismatched
+ * structures. CONEXB200_BatchMaximize solves all of them from a cold start: b and y are m x count
+ * column-major HOST arrays, solved[p] / the return value follow CONEX_Maximize (1 = solved; the
+ * return value is the number of solved programs, -1 on an error). Every program follows the same
+ * iteration sequence it would follow through CONEX_Maximize alone. With equality blocks the KKT
+ * systems are factored by a batched regularised LDL^T; iterative_refinement_iterations > 0 is then
+ * refused (-1), as is enable_line_search when every constraint is an LP cone or an equality block. */
 void* CONEXB200_CreateBatch(void* const* programs, int count);
 void CONEXB200_DeleteBatch(void* batch);
 int CONEXB200_BatchMaximize(void* batch, const double* b, const CONEX_SolverConfiguration* config, double* y,
@@ -203,7 +207,8 @@ void CONEXB200_BatchGetResults(void* batch, int* iterations, double* by, double*
 /* Device time of the last batched solve and of its Newton steps (CUDA events). */
 double CONEXB200_BatchMilliseconds(void* batch);
 int CONEXB200_BatchStepMilliseconds(void* batch, double* out, int capacity);
-/* Scaled dual variable of cone `cone` of program `program` (like CONEX_GetDualVariable); returns its size. */
+/* Scaled dual variable of constraint `cone` of program `program` (like CONEX_GetDualVariable, same
+ * numbering); returns its size. Equality blocks have none: nothing is written, the return value is 0. */
 int CONEXB200_BatchGetDualVariable(void* batch, int program, int cone, double* x);
 
 #ifdef __cplusplus

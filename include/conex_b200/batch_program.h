@@ -11,6 +11,13 @@
 // the host over arrays of B scalars fetched once per phase. Programs that have terminated are masked
 // out of later launches, so every program follows exactly the iteration sequence it would follow
 // alone.
+//
+// Equality constraints (EqualityConstraints blocks, on any subset of the variables) add their
+// multipliers as KKT unknowns m..N-1, in the order the blocks were added (Program::AddConstraint).
+// Their rows of the KKT matrices and of AQc / AW are constant and written once per batch; the cones'
+// Schur kernels assign only the leading m x m block. A batch with multipliers factors its KKT systems
+// with the batched regularised LDL^T (cxb_small_ldlt, never fails), one without keeps the batched
+// Cholesky — the input decides, as in kkt_solver.cc:172-199.
 #pragma once
 #include <memory>
 #include <vector>
@@ -30,8 +37,9 @@ struct BatchResult {
 
 class BatchProgram {
  public:
-  // All programs must have the same number of variables and the same list of cones (type, order),
-  // every cone on all variables in order, no equality constraints. Throws otherwise.
+  // All programs must have the same number of variables and the same list of constraints: cones
+  // (LP, second-order, dense LMI; type, order) on all variables in order, and equality blocks (rows,
+  // variable subset) at the same positions among them; at least one cone. Throws otherwise.
   explicit BatchProgram(const std::vector<Program*>& programs);
   ~BatchProgram();
 
@@ -44,7 +52,8 @@ class BatchProgram {
   // individual Newton steps.
   double milliseconds() const { return total_ms_; }
   const std::vector<float>& step_milliseconds() const { return step_ms_; }
-  // Scaling point of cone `cone` of program `p`, rescaled like Program::GetDualVariable.
+  // Scaling point of constraint `cone` of program `p`, rescaled like Program::GetDualVariable; the
+  // numbering counts equality blocks, which have no dual variable (size 0, nothing written).
   int DualVariableSize(int cone) const;
   void GetDualVariable(int p, int cone, double* host_out);
 

@@ -24,6 +24,12 @@ class EqualityConstraints {
   WorkspaceEqualityConstraints* workspace() { return &workspace_; }
   int number_of_variables() const { return 0; }  // equality_constraint.h:46
   void bind(DeviceContext* ctx) { ctx_ = ctx; }
+  // Read-only views of the data (the batched solver writes it into its KKT matrices): A is rows x
+  // number_of_columns() column-major, b has rows entries; both in device memory.
+  int rows() const { return rows_; }
+  int number_of_columns() const { return nv_; }
+  const double* device_A() const { return dev_->A.get(); }
+  const double* device_b() const { return dev_->b.get(); }
 
   friend int Rank(const EqualityConstraints&) { return 0; }
   friend void SetIdentity(EqualityConstraints*) {}

@@ -347,6 +347,21 @@ int cxb_small_potrf(void* stream, int batch, int N, double* dH, long ldh, long h
                     const int* d_active);
 int cxb_small_potrs(void* stream, int batch, int N, const double* dL, long ldl, long lstride, double* dX,
                     long xstride, const int* d_active);
+/* Regularised LDL^T of `batch` symmetric indefinite N x N matrices (KKT systems with equality multipliers; the
+ * batched counterpart of cxb_sym_permute_lower + cxb_ldlt_lower, one program per CTA like cxb_small_potrf): per
+ * program the pivot order of Eigen::RLDLT from diag(K) (RLDLT.h:328-356, as CONEXB200_RldltPivotOrder), the
+ * permuted copy P K P^T gathered from the lower triangle of K, and its factorisation L S L^T, S = diag(+-1), with
+ * |D|^{1/2} folded into L. Pivots with |d| <= 1e-9 become -1e-9 when d < 0, +1e-9 otherwise; d_info[p] = 1 then,
+ * else 0 — it never fails. K is not modified; the lower triangle of L (ldl, lstride), d_perm (ints, perm[i] =
+ * original index at pivot position i) and d_signs (S) are written. Shared memory: N^2 + O(N) doubles per program;
+ * returns an error code when that does not fit. */
+int cxb_small_ldlt(void* stream, int batch, int N, const double* dK, long ldk, long kstride, double* dL, long ldl,
+                   long lstride, int* d_perm, long pstride, double* d_signs, long sstride, int* d_info,
+                   const int* d_active);
+/* x <- P^T L^{-T} S L^{-1} P x with the factors of cxb_small_ldlt, nrhs = 1. */
+int cxb_small_ldlt_solve(void* stream, int batch, int N, const double* dL, long ldl, long lstride, const int* d_perm,
+                         long pstride, const double* d_signs, long sstride, double* dX, long xstride,
+                         const int* d_active);
 /* out[p] = a[p] x[p] + b[p] y[p] + c[p] z[p] (n entries each; coefficient arrays on the device,
  * NULL coefficient array / vector = term absent). */
 int cxb_batched_lincomb(void* stream, int batch, int n, const double* d_a, const double* dx, long xs,
