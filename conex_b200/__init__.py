@@ -79,6 +79,8 @@ _lib.CONEXB200_CreateBatch.argtypes = [_C.POINTER(_C.c_void_p), _C.c_int]
 _lib.CONEXB200_DeleteBatch.argtypes = [_C.c_void_p]
 _lib.CONEXB200_BatchMaximize.argtypes = [_C.c_void_p, _dp, _C.POINTER(CONEX_SolverConfiguration), _dp, _ip]
 _lib.CONEXB200_BatchGetResults.argtypes = [_C.c_void_p, _ip, _dp, _dp, _dp]
+_lib.CONEXB200_BatchUpdateConstraintData.argtypes = [_C.c_void_p, _C.c_int, _C.c_int, _C.c_int, _dp]
+_lib.CONEXB200_BatchConstraintDataShape.argtypes = [_C.c_void_p, _C.c_int, _ip, _ip]
 
 
 _lib.CONEXB200_SetKKTSolverKind.argtypes = [_C.c_void_p, _C.c_int]
@@ -329,7 +331,11 @@ class ConexBatch:
     constraints (e.g. the lb == ub rows of AddLinearInequalities, on any subset of the variables);
     every program must have the same constraints in the same order. With equality constraints the
     KKT systems are factored by a batched regularised LDL^T, and iterative refinement, or a line
-    search on programs of LP cones and equalities only, is refused."""
+    search on programs of LP cones and equalities only, is refused.
+
+    A batch lives across solves: `config.initialization_mode = 1` warm-starts every program from the
+    iterate of the previous Maximize (an error before the first one), and UpdateConstraintData
+    changes the programs' data in place between solves."""
 
     def __init__(self, programs):
         self.count = len(programs)
@@ -360,6 +366,23 @@ class ConexBatch:
             s.y, s.status = y[p], status[p]
             out.append(s)
         return out
+
+    def UpdateConstraintData(self, constraint, first, data):
+        """Replaces columns [first, first + ncols) of the data of constraint `constraint` (numbered like
+        GetDualVariables) in every program; data has shape (count, rows, ncols), data[p] for program p.
+        Cones: column j < m holds the coefficients of y_j (LP / second-order: column j of A; LMI: the
+        column-major vec of A_j, rows = n * n), column m the affine term. Equality constraints: column
+        j < nvars is column j of A, column nvars is b."""
+        data = _np.asarray(data, dtype=_np.float64)
+        rows, columns = _C.c_int(), _C.c_int()
+        if _lib.CONEXB200_BatchConstraintDataShape(self.h, int(constraint), _C.byref(rows), _C.byref(columns)) != 0:
+            raise NameError("The batch has no constraint %d." % constraint)
+        if data.ndim != 3 or data.shape[0] != self.count or data.shape[1] != rows.value:
+            raise NameError("Constraint data must have shape (%d, %d, columns)." % (self.count, rows.value))
+        blocks = _np.ascontiguousarray(data.transpose(0, 2, 1))
+        if _lib.CONEXB200_BatchUpdateConstraintData(self.h, int(constraint), int(first), data.shape[2],
+                                                    _ptr(blocks)) != 0:
+            raise NameError("Failed to update the constraint data (constraint or column range out of range).")
 
 
 def programs_default_configuration():

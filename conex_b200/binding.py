@@ -385,6 +385,8 @@ class Batch:
         L.CONEXB200_BatchMilliseconds.argtypes = [C.c_void_p]
         L.CONEXB200_BatchStepMilliseconds.argtypes = [C.c_void_p, c_double_p, C.c_int]
         L.CONEXB200_BatchGetDualVariable.argtypes = [C.c_void_p, C.c_int, C.c_int, c_double_p]
+        L.CONEXB200_BatchUpdateConstraintData.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, c_double_p]
+        L.CONEXB200_BatchConstraintDataShape.argtypes = [C.c_void_p, C.c_int, c_int_p, c_int_p]
         self.count = len(programs)
         self.m = programs[0].m
         handles = (C.c_void_p * self.count)(*[p.h for p in programs])
@@ -407,6 +409,17 @@ class Batch:
         rc = self.L.lib.CONEXB200_BatchMaximize(self.h, dptr(b), C.byref(cfg), dptr(y), solved)
         assert rc >= 0, "CONEXB200_BatchMaximize failed"
         return np.array(list(solved)), y
+
+    def update(self, constraint, first, data):
+        """CONEXB200_BatchUpdateConstraintData: data (count, rows, ncols) replaces columns [first, first + ncols) of
+        constraint `constraint` in every program."""
+        data = np.asarray(data, dtype=np.float64)
+        rows, columns = C.c_int(), C.c_int()
+        assert self.L.lib.CONEXB200_BatchConstraintDataShape(self.h, constraint, C.byref(rows), C.byref(columns)) == 0
+        assert data.ndim == 3 and data.shape[:2] == (self.count, rows.value), (data.shape, rows.value)
+        blocks = np.ascontiguousarray(data.transpose(0, 2, 1))  # program p: rows x ncols column-major
+        rc = self.L.lib.CONEXB200_BatchUpdateConstraintData(self.h, constraint, first, data.shape[2], dptr(blocks))
+        assert rc == 0, "CONEXB200_BatchUpdateConstraintData failed"
 
     def results(self):
         it = (C.c_int * self.count)()

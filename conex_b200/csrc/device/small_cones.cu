@@ -313,15 +313,16 @@ __global__ void __launch_bounds__(kThreads) TakeStepMultiKernel(int batch, long 
   TakeStepBody<false>(batch, per, l.c[blockIdx.y], step, step_p, ew, info, active);
 }
 
-// Lower triangles of the m + 1 matrices of a PSD cone, one CTA per program; flags matrices that are not symmetric.
-__global__ void __launch_bounds__(kThreads) PackSymmetricKernel(ConeArgs c, double* packed, long packed_stride,
-                                                               int* asymmetric) {
+// Lower triangles of the matrices [first, first + count) of a PSD cone, one CTA per program; flags matrices that are
+// not symmetric.
+__global__ void __launch_bounds__(kThreads) PackSymmetricKernel(ConeArgs c, int first, int count, double* packed,
+                                                               long packed_stride, int* asymmetric) {
   const int p = blockIdx.x;
   const int n = c.n, kp = n * (n + 1) / 2;
-  const double* data = c.data + p * c.data_stride;
-  double* out = packed + p * packed_stride;
+  const double* data = c.data + p * c.data_stride + (long)first * n * n;
+  double* out = packed + p * packed_stride + (long)first * kp;
   bool bad = false;
-  for (int e = threadIdx.x; e < (c.m + 1) * n * n; e += blockDim.x) {
+  for (int e = threadIdx.x; e < count * n * n; e += blockDim.x) {
     const int j = e / (n * n), q = e - j * n * n;
     const int col = q / n, row = q - col * n;
     if (row < col) continue;
@@ -522,15 +523,24 @@ int cxb_small_set_identity(void* stream, int batch, const cxb_small_cone* cone, 
   return LaunchStatus();
 }
 
-int cxb_small_pack_symmetric(void* stream, int batch, const cxb_small_cone* cone, double* d_packed, long packed_stride,
-                             int* d_asymmetric) {
+int cxb_small_pack_symmetric_columns(void* stream, int batch, const cxb_small_cone* cone, int first, int count,
+                                     double* d_packed, long packed_stride, int* d_asymmetric) {
   if (batch <= 0) return 0;
   if (!ValidCone(cone) || cone->type != CXB_CONE_PSD || !d_packed || !d_asymmetric) return -1;
+  if (first < 0 || count < 1 || first + count > cone->m + 1) return -1;
   if (packed_stride < (long)(cone->m + 1) * (cone->n * (cone->n + 1) / 2)) return -1;
   ConeArgs c = Convert(cone);
   CountLaunch();
-  PackSymmetricKernel<<<batch, kThreads, 0, AsStream(stream)>>>(c, d_packed, packed_stride, d_asymmetric);
+  PackSymmetricKernel<<<batch, kThreads, 0, AsStream(stream)>>>(c, first, count, d_packed, packed_stride,
+                                                                d_asymmetric);
   return LaunchStatus();
+}
+
+int cxb_small_pack_symmetric(void* stream, int batch, const cxb_small_cone* cone, double* d_packed, long packed_stride,
+                             int* d_asymmetric) {
+  if (batch <= 0) return 0;
+  if (!cone) return -1;
+  return cxb_small_pack_symmetric_columns(stream, batch, cone, 0, cone->m + 1, d_packed, packed_stride, d_asymmetric);
 }
 
 int cxb_small_schur(void* stream, int batch, const cxb_small_cone* cone, double* dG, long ldg,

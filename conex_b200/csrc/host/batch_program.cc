@@ -39,7 +39,8 @@ struct BatchProgram::Impl {
   std::vector<ConeSlot> cones;
   std::vector<cxb_small_cone> descs;  // the descriptors of `cones`, contiguous, for the fused launches
   std::vector<EqualitySlot> equalities;
-  std::vector<int> slot_of;  // constraint number -> index into `cones`, or -1 for an equality block
+  // constraint number -> index k into `cones`, or -1 - q for equalities[q]
+  std::vector<int> slot_of;
   // N = m + multipliers: the order of the KKT systems (reference constraint_manager.h:42-48)
   int B = 0, m = 0, N = 0, multipliers = 0;
   long ldh = 0;
@@ -53,16 +54,38 @@ struct BatchProgram::Impl {
   DeviceBuffer<double> coef;   // 3 x B coefficient arrays | B c_weights | B step sizes
   DeviceBuffer<double> out;    // cone outputs: B x ncones x 4, then B x 4 dots/scalars
   DeviceBuffer<int> info;      // B Cholesky flags | B Padé flags (| B regularisation flags of the LDL^T)
-  DeviceBuffer<int> mask;      // B active | B mu-update
+  DeviceBuffer<int> mask;      // B active | B mu-update | B aborted warm start
+  DeviceBuffer<int> asymmetric;  // UpdateConstraintData: set when new LMI data is not symmetric
   PinnedBuffer<double> hcoef, hout;
   PinnedBuffer<int> hinfo, hmask;
   int rank = 0;
+  // what a warm start continues from besides the cones' states: the scalings of the last solve (the reference
+  // keeps them in the program's memory, WorkspaceStats) and whether the states were ever initialised
+  std::vector<double> b_scaling, c_scaling;
+  bool initialised = false;
 
   void* s() const { return ctx.stream(); }
   void UploadCoef(size_t offset, size_t count) {
     CudaCheck(cudaMemcpyAsync(coef.get() + offset, hcoef.get() + offset, sizeof(double) * count,
                               cudaMemcpyHostToDevice, ctx.cuda_stream()),
               "H2D coefficients");
+  }
+  // Columns [first, first + count) of equality block `e` (column j < nvars: column j of A, column nvars: b) from
+  // `data`, B host blocks of rows x count column-major, into the constant rows m + offset .. of every program's H
+  // (column variables[j]; H[p] is ldh x N) and AQc (b). The cones' Schur kernels assign only the leading m x m block
+  // of H and the first m entries of AW / AQc, and the LDL^T leaves H as it is: these survive every Newton step.
+  void WriteEqualityColumns(const EqualitySlot& e, int first, int count, const double* data) {
+    const int nv = static_cast<int>(e.variables.size());
+    for (int j = first; j < first + count; j++) {
+      const double* src = data + static_cast<size_t>(j - first) * e.rows;
+      double* dst = (j < nv) ? H.get() + static_cast<size_t>(e.variables[j]) * ldh + m + e.offset
+                             : AQc.get() + m + e.offset;
+      const size_t dpitch = sizeof(double) * ((j < nv) ? static_cast<size_t>(ldh) * N : vstride);
+      CudaCheck(cudaMemcpy2DAsync(dst, dpitch, src, sizeof(double) * e.rows * count, sizeof(double) * e.rows, B,
+                                  cudaMemcpyHostToDevice, ctx.cuda_stream()),
+                "upload of equality data");
+    }
+    ctx.Synchronize();  // data is pageable
   }
   void UploadMask(size_t offset) {
     CudaCheck(cudaMemcpyAsync(mask.get() + offset, hmask.get() + offset, sizeof(int) * B,
@@ -166,7 +189,7 @@ BatchProgram::BatchProgram(const std::vector<Program*>& programs) : impl_(std::m
       e.offset = d.multipliers;
       e.variables = sh.variables;
       d.multipliers += sh.n;
-      d.slot_of.push_back(-1);
+      d.slot_of.push_back(-1 - static_cast<int>(d.equalities.size()));
       d.equalities.push_back(std::move(e));
     } else {
       d.slot_of.push_back(static_cast<int>(d.cones.size()));
@@ -208,9 +231,12 @@ BatchProgram::BatchProgram(const std::vector<Program*>& programs) : impl_(std::m
   }
   // ---- pack the cone data; gather the equality data on the host --------------------------------------
   const size_t nm = static_cast<size_t>(d.multipliers);
-  std::vector<double> eq_rows(nm * N * B, 0.0);  // rows m..N-1 of every H, column by column
-  std::vector<double> eq_b(nm * B, 0.0);         // AQc[m..N) of every program
-  std::vector<double> host_A;
+  // per equality block, [A | b] of every program: B blocks of rows x (nvars + 1), as WriteEqualityColumns takes them
+  std::vector<std::vector<double>> eq_data(d.equalities.size());
+  for (size_t q = 0; q < d.equalities.size(); q++) {
+    const EqualitySlot& e = d.equalities[q];
+    eq_data[q].resize(static_cast<size_t>(e.rows) * (e.variables.size() + 1) * B);
+  }
   for (int p = 0; p < B; p++) {
     Program& prog = *programs[p];
     if (prog.GetNumberOfVariables() != m || prog.NumberOfMultipliers() != d.multipliers ||
@@ -227,16 +253,12 @@ BatchProgram::BatchProgram(const std::vector<Program*>& programs) : impl_(std::m
       if (sh.type == kEquality) {
         // ConstructSchurComplementSystem(EqualityConstraints*) (equality_constraint.cc:13-30): A on (multipliers,
         // variables), zeros elsewhere in these rows of H, including the multiplier block; b in AQc, zeros in AW
-        const EqualitySlot& e = d.equalities[q++];
+        const EqualitySlot& e = d.equalities[q];
         auto* eq = std::any_cast<EqualityConstraints>(&c.obj);
         const size_t nv = e.variables.size();
-        host_A.resize(static_cast<size_t>(e.rows) * nv);
-        d.ctx.Download(host_A.data(), eq->device_A(), host_A.size());
-        d.ctx.Download(eq_b.data() + nm * p + e.offset, eq->device_b(), e.rows);
-        for (size_t j = 0; j < nv; j++) {
-          double* col = eq_rows.data() + (static_cast<size_t>(p) * N + e.variables[j]) * nm + e.offset;
-          for (int r = 0; r < e.rows; r++) col[r] = host_A[j * e.rows + r];
-        }
+        double* block = eq_data[q++].data() + static_cast<size_t>(p) * e.rows * (nv + 1);
+        d.ctx.Download(block, eq->device_A(), static_cast<size_t>(e.rows) * nv);
+        d.ctx.Download(block + static_cast<size_t>(e.rows) * nv, eq->device_b(), e.rows);
         k++;
         continue;
       }
@@ -305,25 +327,27 @@ BatchProgram::BatchProgram(const std::vector<Program*>& programs) : impl_(std::m
   d.coef.Resize(5 * static_cast<size_t>(B));
   d.out.Resize(static_cast<size_t>(B) * (4 * nc + 4));
   d.info.Resize((d.multipliers ? 3 : 2) * static_cast<size_t>(B));
-  d.mask.Resize(2 * static_cast<size_t>(B));
+  d.mask.Resize(3 * static_cast<size_t>(B));
+  d.asymmetric.Resize(1);
   d.hcoef.Reserve(std::max<size_t>(5 * static_cast<size_t>(B), d.vstride * B));
   d.hout.Reserve(std::max<size_t>(static_cast<size_t>(B) * (4 * nc + 4), d.vstride * B));
   d.hinfo.Reserve(2 * static_cast<size_t>(B));
-  d.hmask.Reserve(2 * static_cast<size_t>(B));
+  d.hmask.Reserve(3 * static_cast<size_t>(B));
+  d.b_scaling.assign(B, 1.0);
+  d.c_scaling.assign(B, 1.0);
   results_.assign(B, BatchResult());
   if (d.multipliers) {
-    // The constant rows m..N-1 of every H (H[p] is ldh x N, so column c of program p is column p N + c of one
-    // B N-column matrix), AQc[m..N) and AW[m..N). The cones' Schur kernels assign only the leading m x m block of H
-    // and the first m entries of AW / AQc, and the LDL^T leaves H as it is: these survive every Newton step.
+    // rows m..N-1 of every H (H[p] is ldh x N, so column c of program p is column p N + c of one B N-column matrix)
+    // and AW[m..N) are zero outside the blocks' A (equality_constraint.cc:13-30, including the multiplier block)
     cudaStream_t cs = d.ctx.cuda_stream();
-    CudaCheck(cudaMemcpy2DAsync(d.H.get() + m, sizeof(double) * d.ldh, eq_rows.data(), sizeof(double) * nm,
-                                sizeof(double) * nm, static_cast<size_t>(N) * B, cudaMemcpyHostToDevice, cs),
-              "upload of the equality rows");
-    CudaCheck(cudaMemcpy2DAsync(d.AQc.get() + m, sizeof(double) * d.vstride, eq_b.data(), sizeof(double) * nm,
-                                sizeof(double) * nm, B, cudaMemcpyHostToDevice, cs),
-              "upload of the equality right-hand sides");
+    CudaCheck(cudaMemset2DAsync(d.H.get() + m, sizeof(double) * d.ldh, 0, sizeof(double) * nm,
+                                static_cast<size_t>(N) * B, cs),
+              "memset");
     CudaCheck(cudaMemset2DAsync(d.AW.get() + m, sizeof(double) * d.vstride, 0, sizeof(double) * nm, B, cs), "memset");
-    d.ctx.Synchronize();  // eq_rows / eq_b are pageable
+    for (size_t q = 0; q < d.equalities.size(); q++) {
+      const EqualitySlot& e = d.equalities[q];
+      d.WriteEqualityColumns(e, 0, static_cast<int>(e.variables.size()) + 1, eq_data[q].data());
+    }
   }
 }
 
@@ -351,6 +375,53 @@ void BatchProgram::GetDualVariable(int p, int cone, double* host_out) {
   }
 }
 
+bool BatchProgram::ConstraintDataShape(int constraint, int* rows, int* columns) const {
+  const Impl& d = *impl_;
+  if (constraint < 0 || constraint >= static_cast<int>(d.slot_of.size())) return false;
+  const int k = d.slot_of[constraint];
+  *rows = k < 0 ? d.equalities[-1 - k].rows : d.cones[k].rows;
+  *columns = k < 0 ? static_cast<int>(d.equalities[-1 - k].variables.size()) + 1 : d.m + 1;
+  return true;
+}
+
+void BatchProgram::UpdateConstraintData(int constraint, int first, int count, const double* data) {
+  Impl& d = *impl_;
+  int rows = 0, columns = 0;
+  if (!ConstraintDataShape(constraint, &rows, &columns)) {
+    throw std::runtime_error("conex-b200: no such constraint in the batch");
+  }
+  const int k = d.slot_of[constraint];
+  if (first < 0 || count < 1 || count > columns - first || !data) {
+    throw std::runtime_error("conex-b200: bad column range or data for a constraint update");
+  }
+  if (k < 0) {
+    d.WriteEqualityColumns(d.equalities[-1 - k], first, count, data);
+    return;
+  }
+  ConeSlot& c = d.cones[k];
+  const size_t width = sizeof(double) * rows * count;
+  CudaCheck(cudaMemcpy2DAsync(c.data.get() + static_cast<size_t>(first) * rows, sizeof(double) * c.desc.data_stride,
+                              data, width, width, d.B, cudaMemcpyHostToDevice, d.ctx.cuda_stream()),
+            "upload of constraint data");
+  if (c.desc.packed) {
+    // refresh the packed lower triangles of the changed matrices; data that is not symmetric drops the packed copy
+    // for good, as at construction
+    CudaCheck(cudaMemsetAsync(d.asymmetric.get(), 0, sizeof(int), d.ctx.cuda_stream()), "memset");
+    DeviceCheck(cxb_small_pack_symmetric_columns(d.s(), d.B, &c.desc, first, count, c.packed.get(),
+                                                 c.desc.packed_stride, d.asymmetric.get()),
+                "cxb_small_pack_symmetric_columns");
+    int asymmetric = 0;
+    d.ctx.DownloadInts(&asymmetric, d.asymmetric.get(), 1);
+    if (asymmetric) {
+      c.desc.packed = nullptr;
+      c.desc.packed_stride = 0;
+      c.packed.Resize(0);
+      d.descs[k] = c.desc;
+    }
+  }
+  d.ctx.Synchronize();  // data is pageable
+}
+
 namespace {
 
 // Host state of one program of the batch: the locals of Solve() (reference cone_program.cc:276-309).
@@ -360,6 +431,8 @@ struct ProgramState {
   int centering_steps = 0, num_iter = 0;
   bool active = true, failed = false, max_iters_reached = true;
   bool initial_centering = false, final_centering = false, update_mu = false;
+  bool warmstart_aborted = false;
+  bool restarted = false;  // this iteration: the warm start failed to factor, the cones were reset, nothing else runs
 };
 
 }  // namespace
@@ -369,8 +442,9 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
   const int B = batch_, m = m_, N = d.N;
   const size_t nc = d.cones.size();
   const size_t vs = d.vstride;
-  if (cfg.initialization_mode != CONEX_INITIALIZATION_MODE_COLDSTART) {
-    throw std::runtime_error("conex-b200: batched solves are cold starts");
+  const bool warm = cfg.initialization_mode != CONEX_INITIALIZATION_MODE_COLDSTART;
+  if (warm && !d.initialised) {
+    throw std::runtime_error("conex-b200: a warm start needs a previous solve of the batch");
   }
   if (cfg.kkt_solver == CONEX_QR_FACTORIZATION) {
     throw std::runtime_error("conex-b200: the QR KKT mode is not implemented on the device");
@@ -395,7 +469,7 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
   results_.assign(B, BatchResult());
   step_ms_.clear();
 
-  // ---- cost vectors, cold start -------------------------------------------------------------------
+  // ---- cost vectors; a cold start resets the scalings and the cones (cone_program.cc:350-354) ------------
   for (int p = 0; p < B; p++) {
     double nrm = 0;
     for (int i = 0; i < m; i++) {
@@ -406,13 +480,22 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
     for (size_t i = m; i < vs; i++) d.hcoef[p * vs + i] = 0;
     st[p].b_norm = std::sqrt(nrm);
     st[p].kmax = cfg.inv_sqrt_mu_max;
+    if (warm) {
+      st[p].b_scaling = d.b_scaling[p];
+      st[p].c_scaling = d.c_scaling[p];
+    }
   }
   CudaCheck(cudaMemcpyAsync(d.b.get(), d.hcoef.get(), sizeof(double) * vs * B, cudaMemcpyHostToDevice, cs),
             "H2D cost vectors");
   d.ctx.Synchronize();  // hcoef is reused below
   d.ctx.Zero(d.y.get(), vs * B);
   const int ncones = static_cast<int>(nc);
-  DeviceCheck(cxb_small_set_identity_multi(s, B, ncones, d.descs.data(), nullptr), "cxb_small_set_identity_multi");
+  if (!warm) {
+    DeviceCheck(cxb_small_set_identity_multi(s, B, ncones, d.descs.data(), nullptr), "cxb_small_set_identity_multi");
+    d.initialised = true;
+  }
+  const int initial_centering_steps =
+      warm ? cfg.initial_centering_steps_warmstart : cfg.initial_centering_steps_coldstart;
   cudaEvent_t ev_begin, ev_end, ev_a, ev_b;
   CudaCheck(cudaEventCreate(&ev_begin), "cudaEventCreate");
   CudaCheck(cudaEventCreate(&ev_end), "cudaEventCreate");
@@ -422,6 +505,7 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
 
   int* active = d.mask.get();
   int* mu_mask = d.mask.get() + B;
+  int* abort_mask = d.mask.get() + 2 * static_cast<size_t>(B);
   double* coef_a = d.coef.get();
   double* coef_b = d.coef.get() + B;
   double* coef_c = d.coef.get() + 2 * static_cast<size_t>(B);
@@ -439,10 +523,12 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
       ProgramState& q = st[p];
       d.hmask[p] = 0;
       if (!q.active) continue;
-      q.initial_centering = i < cfg.initial_centering_steps_coldstart;
+      q.restarted = false;
+      q.initial_centering = i < initial_centering_steps;
       q.final_centering = (q.k >= q.kmax) || (q.kkt_error > cfg.kkt_error_tolerance) ||
                           (i >= cfg.max_iterations - cfg.final_centering_steps);
-      q.update_mu = (i == 0) || !(q.initial_centering || q.final_centering);
+      q.update_mu = (i == 0) || !(q.initial_centering || q.final_centering) || q.warmstart_aborted;
+      q.warmstart_aborted = false;
       if (q.final_centering && q.centering_steps >= cfg.final_centering_steps) {
         q.max_iters_reached = (i >= cfg.max_iterations - 1);
         q.active = false;
@@ -458,7 +544,9 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
     // ---- assemble, (rescale,) factor ---------------------------------------------------------------
     d.Assemble(active);
     const bool rescale = (i == 0) && cfg.enable_rescaling;
-    if (rescale) {
+    // a warm start keeps the scalings of the previous solve and only rescales kmax with them (NewtonDriver::Run)
+    const bool new_scalings = rescale && !warm;
+    if (new_scalings) {
       DeviceCheck(cxb_batched_dot(s, B, N, d.AQc.get(), vs, d.AQc.get(), vs, dots, 4), "cxb_batched_dot");
     }
     d.Factor(active);
@@ -466,28 +554,42 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
       CudaCheck(cudaMemcpyAsync(d.hinfo.get(), d.info.get(), sizeof(int) * B, cudaMemcpyDeviceToHost, cs),
                 "D2H info");
     }
-    if (rescale) {
+    if (new_scalings) {
       CudaCheck(cudaMemcpyAsync(d.hout.get(), dots, sizeof(double) * 4 * B, cudaMemcpyDeviceToHost, cs), "D2H norms");
     }
     d.ctx.Synchronize();
     bool mask_changed = false;
     bool any_mu = false;
+    bool any_restart = false;
     for (int p = 0; p < B; p++) {
       ProgramState& q = st[p];
       d.hmask[B + p] = 0;
+      d.hmask[2 * static_cast<size_t>(B) + p] = 0;
       if (!q.active) continue;
       if (rescale) {
-        // reference cone_program.cc:343-357 (cold start)
-        q.b_scaling = 1.0 / (1 + q.b_norm);
-        q.c_scaling = 1.0 / (1 + std::sqrt(d.hout[4 * p]));
+        // reference cone_program.cc:343-357
+        if (new_scalings) {
+          q.b_scaling = 1.0 / (1 + q.b_norm);
+          q.c_scaling = 1.0 / (1 + std::sqrt(d.hout[4 * p]));
+        }
         const double mu_target = (1.0 / (q.kmax * q.kmax)) * (q.b_scaling * q.c_scaling);
         q.kmax = 1.0 / std::sqrt(mu_target);
       }
-      if (!d.multipliers && d.hinfo[p] != 0) {  // Factor() failed: the solve returns unsolved (cone_program.cc:360-371)
-        q.active = false;
-        q.failed = true;
+      if (!d.multipliers && d.hinfo[p] != 0) {
         d.hmask[p] = 0;
         mask_changed = true;
+        if (i == 0 && warm) {
+          // the warm start is abandoned: restart from the identity and skip the rest of this iteration, as
+          // NewtonDriver::Run does for one program
+          q.restarted = true;
+          q.warmstart_aborted = true;
+          d.hmask[2 * static_cast<size_t>(B) + p] = 1;
+          any_restart = true;
+          continue;
+        }
+        // Factor() failed: the solve returns unsolved (cone_program.cc:360-371)
+        q.active = false;
+        q.failed = true;
         continue;
       }
       if (q.update_mu) {
@@ -496,6 +598,11 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
       }
     }
     if (mask_changed) d.UploadMask(0);
+    if (any_restart) {
+      d.UploadMask(2 * static_cast<size_t>(B));
+      DeviceCheck(cxb_small_set_identity_multi(s, B, ncones, d.descs.data(), abort_mask),
+                  "cxb_small_set_identity_multi");
+    }
 
     // ---- mu from the divergence bound (reference cone_program.cc:173-214) --------------------------
     if (any_mu) {
@@ -550,7 +657,7 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
     }
     for (int p = 0; p < B; p++) {
       ProgramState& q = st[p];
-      if (!q.active) continue;
+      if (!q.active || q.restarted) continue;
       if (!q.update_mu && !q.initial_centering) q.centering_steps++;
       q.k = std::max(std::min(q.k, q.kmax), std::sqrt(1.0 / (1e-15 + cfg.maximum_mu)));
       d.hcoef[p] = q.k * q.b_scaling;
@@ -570,10 +677,12 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
                 "cxb_small_prepare_multi");
     d.DownloadOut(static_cast<size_t>(B) * 4 * nc);
     std::vector<double> normsq(B, 0.0);
+    bool any_abort = false;
     for (int p = 0; p < B; p++) {
       ProgramState& q = st[p];
       d.hcoef[4 * static_cast<size_t>(B) + p] = 1.0;
-      if (!q.active) continue;
+      d.hmask[2 * static_cast<size_t>(B) + p] = 0;
+      if (!q.active || q.restarted) continue;
       double ninf = -1, nsq = 0;
       for (size_t k = 0; k < nc; k++) {
         const double* o = d.hout.get() + (static_cast<size_t>(p) * nc + k) * 4;
@@ -583,8 +692,22 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
       q.d_inf = std::fabs(ninf);
       normsq[p] = nsq;
       d.hcoef[4 * static_cast<size_t>(B) + p] = std::min(1.0, 2.0 / (ninf * ninf));
+      if (i == 0 && warm && ninf >= cfg.warmstart_abort_threshold) {
+        // too large a first step from the warm iterate: restart from the identity instead of taking it; the
+        // iteration is completed and logged (NewtonDriver::Run)
+        q.warmstart_aborted = true;
+        d.hmask[p] = 0;
+        d.hmask[2 * static_cast<size_t>(B) + p] = 1;
+        any_abort = true;
+      }
     }
     d.UploadCoef(4 * static_cast<size_t>(B), B);
+    if (any_abort) {
+      d.UploadMask(0);
+      d.UploadMask(2 * static_cast<size_t>(B));
+      DeviceCheck(cxb_small_set_identity_multi(s, B, ncones, d.descs.data(), abort_mask),
+                  "cxb_small_set_identity_multi");
+    }
     DeviceCheck(cxb_small_take_step_multi(s, B, ncones, d.descs.data(), 1.0, coef_step, 1.0, d.info.get() + B, active),
                 "cxb_small_take_step_multi");
     // ---- objectives (cone_program.cc:441-467) -------------------------------------------------------
@@ -601,7 +724,7 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
     step_ms_.push_back(ms);
     for (int p = 0; p < B; p++) {
       ProgramState& q = st[p];
-      if (!q.active) continue;
+      if (!q.active || q.restarted) continue;
       const double by_dot = d.hout[4 * p + 0], aqc_dot = d.hout[4 * p + 1];
       const double wc = d.hout[4 * static_cast<size_t>(B) + 2 * p], cqc = d.hout[4 * static_cast<size_t>(B) + 2 * p + 1];
       const double k = q.k;
@@ -631,8 +754,8 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
     r.by = q.by;
     r.cx = q.cx;
     r.inv_sqrt_mu = q.k;
-    r.b_scaling = q.b_scaling;
-    r.c_scaling = q.c_scaling;
+    r.b_scaling = d.b_scaling[p] = q.b_scaling;
+    r.c_scaling = d.c_scaling[p] = q.c_scaling;
     r.d_inf = q.d_inf;
     double* yp = y_out + static_cast<size_t>(p) * m;
     for (int j = 0; j < m; j++) yp[j] = d.hout[p * vs + j];

@@ -634,6 +634,23 @@ int CONEXB200_BatchGetDualVariable(void* batch, int program, int cone, double* x
       -1);
 }
 
+int CONEXB200_BatchUpdateConstraintData(void* batch, int constraint, int first, int count, const double* data) {
+  return Guard(
+      [&]() -> int {
+        static_cast<conex::BatchProgram*>(batch)->UpdateConstraintData(constraint, first, count, data);
+        return 0;
+      },
+      -1);
+}
+
+int CONEXB200_BatchConstraintDataShape(void* batch, int constraint, int* rows, int* columns) {
+  int r = 0, c = 0;
+  if (!static_cast<conex::BatchProgram*>(batch)->ConstraintDataShape(constraint, &r, &c)) return -1;
+  if (rows) *rows = r;
+  if (columns) *columns = c;
+  return 0;
+}
+
 // 1 when constraint `id` is an incremental LMI currently held in entry-sparse form (after the first
 // solve / assembly), 0 when dense, -1 for other constraint types.
 int CONEXB200_ConstraintIsEntrySparse(void* prog, int id) {

@@ -192,12 +192,14 @@ void CONEXB200_RldltPivotOrder(int n, const double* diag, int* perm);
  * the same equality blocks — rows, variable subset, position among the cones — e.g. the lb == ub rows
  * of CONEX_AddLinearInequalities; at least one cone). CONEXB200_CreateBatch packs their data into
  * batched device arrays (the handles may be deleted afterwards); it returns NULL for mismatched
- * structures. CONEXB200_BatchMaximize solves all of them from a cold start: b and y are m x count
- * column-major HOST arrays, solved[p] / the return value follow CONEX_Maximize (1 = solved; the
- * return value is the number of solved programs, -1 on an error). Every program follows the same
- * iteration sequence it would follow through CONEX_Maximize alone. With equality blocks the KKT
- * systems are factored by a batched regularised LDL^T; iterative_refinement_iterations > 0 is then
- * refused (-1), as is enable_line_search when every constraint is an LP cone or an equality block. */
+ * structures. CONEXB200_BatchMaximize solves all of them: b and y are m x count column-major HOST
+ * arrays, solved[p] / the return value follow CONEX_Maximize (1 = solved; the return value is the
+ * number of solved programs, -1 on an error). Every program follows the same iteration sequence it
+ * would follow through CONEX_Maximize alone, from a cold start or, with initialization_mode = 1, warm-
+ * started from the iterate of the batch's previous solve (-1 when there was none). With equality
+ * blocks the KKT systems are factored by a batched regularised LDL^T; iterative_refinement_iterations
+ * > 0 is then refused (-1), as is enable_line_search when every constraint is an LP cone or an
+ * equality block. */
 void* CONEXB200_CreateBatch(void* const* programs, int count);
 void CONEXB200_DeleteBatch(void* batch);
 int CONEXB200_BatchMaximize(void* batch, const double* b, const CONEX_SolverConfiguration* config, double* y,
@@ -210,6 +212,18 @@ int CONEXB200_BatchStepMilliseconds(void* batch, double* out, int capacity);
 /* Scaled dual variable of constraint `cone` of program `program` (like CONEX_GetDualVariable, same
  * numbering); returns its size. Equality blocks have none: nothing is written, the return value is 0. */
 int CONEXB200_BatchGetDualVariable(void* batch, int program, int cone, double* x);
+/* Replaces columns [first, first + count) of the data of constraint `constraint` (numbered like
+ * CONEX_GetDualVariable, equality blocks included) in every program of the batch. Cones: column j < m holds
+ * the coefficients of y_j (LP: column j of A; SOC: column j of the (n + 1) x m A; LMI: vec(A_j)), column m the
+ * affine term (c / C). Equality blocks: column j < nvars is column j of A, column nvars is b.
+ * data: host memory, B blocks of rows x count column-major (program p at data + p * rows * count).
+ * Returns 0, or -1 on bad arguments (the batch is then unchanged). The next BatchMaximize uses the new data;
+ * a warm start continues from the iterate of the previous solve. */
+int CONEXB200_BatchUpdateConstraintData(void* batch, int constraint, int first, int count, const double* data);
+/* The shape of that data for constraint `constraint`: *rows (cones: n for LP, n + 1 for SOC, n * n for LMI; equality
+ * blocks: their rows) and *columns (cones: m + 1; equality blocks: nvars + 1). Returns 0, or -1 when the batch has no
+ * such constraint. The caller of CONEXB200_BatchUpdateConstraintData must pass blocks of exactly these rows. */
+int CONEXB200_BatchConstraintDataShape(void* batch, int constraint, int* rows, int* columns);
 
 #ifdef __cplusplus
 }

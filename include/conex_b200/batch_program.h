@@ -18,6 +18,18 @@
 // Schur kernels assign only the leading m x m block. A batch with multipliers factors its KKT systems
 // with the batched regularised LDL^T (cxb_small_ldlt, never fails), one without keeps the batched
 // Cholesky — the input decides, as in kkt_solver.cc:172-199.
+//
+// A batch lives across many solves. Maximize with initialization_mode = warm start continues every
+// program from the iterate of the previous solve (cone states, including the dual-recovery update,
+// and the b / c scalings), exactly as Program's warm start does for one program: the warm centering
+// schedule, and a restart from the identity for a program whose first factorisation fails or whose
+// first step is too large (warmstart_abort_threshold). UpdateConstraintData replaces columns of a
+// constraint's data in every program on the device, so that the next instance of a parametric
+// problem is solved without building a new batch.
+//
+// Packed copies of the LMI operators: an update refreshes the lower triangles of the changed
+// matrices only; data that is not symmetric bit for bit drops the cone's packed copy for the life of
+// the batch (the slack passes then read the full matrices), as the constructor does.
 #pragma once
 #include <memory>
 #include <vector>
@@ -45,8 +57,16 @@ class BatchProgram {
 
   int size() const { return batch_; }
   int number_of_variables() const { return m_; }
-  // b, y: m x B column-major host arrays. Returns the number of solved programs.
+  // b, y: m x B column-major host arrays. Returns the number of solved programs. A warm start
+  // (config.initialization_mode != cold start) throws when the batch has never been solved.
   int Maximize(const double* b, const SolverConfiguration& config, double* y);
+  // Replaces columns [first, first + count) of the data of constraint `constraint` (numbered like
+  // GetDualVariable) in every program: cones [A | c] (rows x (m + 1); LMI: vec(A_j) and vec(C)),
+  // equality blocks [A | b] (rows x (nvars + 1)). data: B host blocks of rows x count, column-major,
+  // program p at data + p * rows * count. Throws on bad arguments before anything is written.
+  void UpdateConstraintData(int constraint, int first, int count, const double* data);
+  // The rows and columns of that data for `constraint`; false when there is no such constraint.
+  bool ConstraintDataShape(int constraint, int* rows, int* columns) const;
   const std::vector<BatchResult>& results() const { return results_; }
   // Device milliseconds of the last Maximize (CUDA events on the batch's stream) and of its
   // individual Newton steps.

@@ -296,6 +296,11 @@ int cxb_small_set_identity(void* stream, int batch, const cxb_small_cone* cone, 
  * full matrices, dense_lmi_constraint.cc:8-20). */
 int cxb_small_pack_symmetric(void* stream, int batch, const cxb_small_cone* cone, double* d_packed, long packed_stride,
                              int* d_asymmetric);
+/* The same for the matrices [first, first + count) of the m + 1 only (0 <= first, 1 <= count, first + count <= m + 1):
+ * refreshes the packed copy after an in-place update of those columns of `data`; the other matrices are neither read
+ * nor written. cxb_small_pack_symmetric is the full range. */
+int cxb_small_pack_symmetric_columns(void* stream, int batch, const cxb_small_cone* cone, int first, int count,
+                                     double* d_packed, long packed_stride, int* d_asymmetric);
 /* G (ldg, lower triangle), AW, AQc (m each, stride vstride), scal[2] = {<w,c>, <c,Qc>} (stride
  * sstride): assigned (accumulate == 0) or added to (ConstructSchurComplementSystem, initialize flag). */
 int cxb_small_schur(void* stream, int batch, const cxb_small_cone* cone, double* dG, long ldg,
