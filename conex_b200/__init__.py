@@ -327,9 +327,11 @@ class ConexBatch:
     (CONEXB200_CreateBatch / CONEXB200_BatchMaximize, include/conex_b200.h). No counterpart in the
     reference, which solves such programs one after the other.
 
-    The programs may combine LP, second-order and dense LMI cones on all variables with equality
-    constraints (e.g. the lb == ub rows of AddLinearInequalities, on any subset of the variables);
-    every program must have the same constraints in the same order. With equality constraints the
+    The programs may combine LP, second-order and dense LMI cones with equality constraints (e.g. the
+    lb == ub rows of AddLinearInequalities). Each cone or equality block acts on all variables or on a
+    list of distinct variables (a dense LMI added with a variable list, the LP and second-order cones of
+    CONEXB200_AddSparseLinearConstraint / CONEXB200_AddSparseSocConstraint); every program must have
+    the same constraints, on the same variable lists, in the same order. With equality constraints the
     KKT systems are factored by a batched regularised LDL^T, and iterative refinement, or a line
     search on programs of LP cones and equalities only, is refused.
 
@@ -371,8 +373,9 @@ class ConexBatch:
         """Replaces columns [first, first + ncols) of the data of constraint `constraint` (numbered like
         GetDualVariables) in every program; data has shape (count, rows, ncols), data[p] for program p.
         Cones: column j < m holds the coefficients of y_j (LP / second-order: column j of A; LMI: the
-        column-major vec of A_j, rows = n * n), column m the affine term. Equality constraints: column
-        j < nvars is column j of A, column nvars is b."""
+        column-major vec of A_j, rows = n * n), column m the affine term; a cone on a list of m_k
+        variables v has m_k + 1 columns, column j < m_k for y[v_j] and column m_k the affine term.
+        Equality constraints: column j < nvars is column j of A, column nvars is b."""
         data = _np.asarray(data, dtype=_np.float64)
         rows, columns = _C.c_int(), _C.c_int()
         if _lib.CONEXB200_BatchConstraintDataShape(self.h, int(constraint), _C.byref(rows), _C.byref(columns)) != 0:

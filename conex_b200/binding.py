@@ -115,6 +115,11 @@ class ConexLib:
             f = getattr(L, f"{self.ext}_{name}")
             f.argtypes = args
             f.restype = res
+        if kind != "oracle":  # cones on variable subsets: product library only
+            L.CONEXB200_AddSparseLinearConstraint.argtypes = [C.c_void_p, c_double_p, C.c_int, C.c_int, c_double_p,
+                                                              C.POINTER(C.c_long)]
+            L.CONEXB200_AddSparseSocConstraint.argtypes = [C.c_void_p, C.c_int, C.c_int, c_double_p, c_double_p,
+                                                           C.POINTER(C.c_long)]
 
     def fn(self, name):
         return getattr(self.lib, f"{self.ext}_{name}")
@@ -182,9 +187,18 @@ class Program:
         self.cone_shapes.append((n, n))
         return cid
 
-    def add_linear(self, A, c):
+    def add_linear(self, A, c, variables=None):
+        """c - A y >= 0. variables: the list of variables A's columns act on (CONEXB200_AddSparseLinearConstraint,
+        product library only; the program's number of variables must be set); None = all of them."""
         Af = fmat(A)
         cf = np.ascontiguousarray(np.array(c, dtype=np.float64).ravel())
+        if variables is not None:
+            v = (C.c_long * len(variables))(*variables)
+            cid = self.L.lib.CONEXB200_AddSparseLinearConstraint(self.h, dptr(Af), Af.shape[0], Af.shape[1],
+                                                                 dptr(cf), v)
+            if cid >= 0:
+                self.cone_shapes.append((Af.shape[0], 1))
+            return cid
         cid = self.L.lib.CONEX_AddDenseLinearConstraint(self.h, dptr(Af), Af.shape[0], Af.shape[1],
                                                         dptr(cf), Af.shape[0])
         if self.m == 0:
@@ -192,14 +206,23 @@ class Program:
         self.cone_shapes.append((Af.shape[0], 1))
         return cid
 
-    def add_soc(self, A, c, incremental=False):
+    def add_soc(self, A, c, incremental=False, variables=None):
         """c - A y in the Lorentz cone of order n+1 (A is (n+1) x m). incremental=True goes through
         CONEX_NewLorentzConeConstraint + CONEX_UpdateLinearOperator / CONEX_UpdateAffineTerm like
         interfaces/python/test/run_tests.py:23-34; otherwise through the SOCConstraint(A, c)
-        constructor the reference's C++ tests use (conex/test/test_socp.cc:41-46)."""
+        constructor the reference's C++ tests use (conex/test/test_socp.cc:41-46). variables: the list of
+        variables A's columns act on (CONEXB200_AddSparseSocConstraint, product library only; the program's
+        number of variables must be set); None = all of them."""
         Af = fmat(A)
         cf = np.ascontiguousarray(np.array(c, dtype=np.float64).ravel())
         order = Af.shape[0] - 1
+        if variables is not None:
+            assert not incremental
+            v = (C.c_long * len(variables))(*variables)
+            cid = self.L.lib.CONEXB200_AddSparseSocConstraint(self.h, order, Af.shape[1], dptr(Af), dptr(cf), v)
+            if cid >= 0:
+                self.cone_shapes.append((order + 1, 1))
+            return cid
         if self.m == 0:
             assert self.L.lib.CONEX_SetNumberOfVariables(self.h, Af.shape[1]) == 0
             self.m = Af.shape[1]

@@ -17,6 +17,7 @@ __host__ __device__ inline long Align4(long n) { return (n + 3) & ~3L; }
 
 struct ConeArgs {
   int type, n, m;
+  int y_offset;  // in the padding after m: the struct keeps its size
   const double* data;
   long data_stride;
   double* state;
@@ -27,8 +28,11 @@ struct ConeArgs {
   long packed_stride;
 };
 
+static_assert(offsetof(cxb_small_cone, data) == 16 && sizeof(cxb_small_cone) == 80,
+              "cxb_small_cone.y_offset must stay in the padding after m");
+
 ConeArgs Convert(const cxb_small_cone* c) {
-  return ConeArgs{c->type, c->n, c->m, c->data, c->data_stride, c->state, c->state_stride, c->work,
+  return ConeArgs{c->type, c->n, c->m, c->y_offset, c->data, c->data_stride, c->state, c->state_stride, c->work,
                   c->work_stride, c->type == CXB_CONE_PSD ? c->packed : nullptr, c->packed_stride};
 }
 
@@ -194,7 +198,7 @@ __device__ __forceinline__ void EigenBody(int batch, long per, const ConeArgs& c
   const double* data = c.data + p * c.data_stride;
   double* st = c.state + p * c.state_stride;
   double* work = c.work ? c.work + p * c.work_stride : nullptr;
-  const double* yp = y + p * ystride;
+  const double* yp = y + p * ystride + c.y_offset;
   const double k = cw_p ? cw_p[p] : cw;
   double* out = out4 + p * ostride;
   if (c.type == CXB_CONE_LP) {
@@ -221,7 +225,7 @@ __device__ __forceinline__ void PrepareBody(int batch, long per, const ConeArgs&
   const double* data = c.data + p * c.data_stride;
   double* st = c.state + p * c.state_stride;
   double* work = c.work ? c.work + p * c.work_stride : nullptr;
-  const double* yp = y + p * ystride;
+  const double* yp = y + p * ystride + c.y_offset;
   const double k = cw_p ? cw_p[p] : cw;
   double* out = out2 + p * ostride;
   if (c.type == CXB_CONE_LP) {
@@ -390,6 +394,65 @@ __global__ void __launch_bounds__(kThreads) LdltSolveKernel(int batch, long per,
                         base + 64);
 }
 
+// The y slices of the subset cones of a batch (cxb_small_gather): one CTA per program.
+__global__ void __launch_bounds__(kThreads) GatherKernel(int count, const int* __restrict__ idx, double* y,
+                                                         long ystride, long dst, const int* active) {
+  const int p = blockIdx.x;
+  if (active && !active[p]) return;
+  double* yp = y + p * ystride;
+  for (int i = threadIdx.x; i < count; i += blockDim.x) {
+    const int v = idx[i];
+    if (v >= 0) yp[dst + i] = yp[v];
+  }
+}
+
+// The Schur blocks of the subset cones into H / AW / AQc / scal (cxb_small_scatter_schur): one CTA per program, the
+// cones one after the other. Within a cone the targets are distinct (its variables are), so its entries are split
+// over the threads without atomics.
+__global__ void __launch_bounds__(kThreads) ScatterSchurKernel(int ncones, const int* __restrict__ cones,
+                                                               const int* __restrict__ idx, const double* S,
+                                                               long sstride, int m, double* H, long ldh, long hstride,
+                                                               double* AW, double* AQc, long vstride, double* scal,
+                                                               long scal_stride, int accumulate, const int* active) {
+  const int p = blockIdx.x;
+  if (active && !active[p]) return;
+  double* h = H + p * hstride;
+  double* aw = AW + p * vstride;
+  double* aq = AQc + p * vstride;
+  double* sc = scal + p * scal_stride;
+  const double* s = S + p * sstride;
+  if (!accumulate) {
+    for (int e = threadIdx.x; e < m * m; e += blockDim.x) {
+      const int j = e / m, i = e - j * m;
+      h[i + (long)j * ldh] = 0;
+    }
+    for (int i = threadIdx.x; i < m; i += blockDim.x) aw[i] = aq[i] = 0;
+    if (threadIdx.x == 0) sc[0] = sc[1] = 0;
+    __syncthreads();
+  }
+  for (int k = 0; k < ncones; k++) {
+    const int mk = cones[3 * k];
+    const int* v = idx + cones[3 * k + 1];
+    const double* g = s + cones[3 * k + 2];
+    const long ld = Align4(mk);
+    for (int e = threadIdx.x; e < mk * mk; e += blockDim.x) {
+      const int j = e / mk, i = e - j * mk;
+      if (i < j) continue;
+      const int vi = v[i], vj = v[j];
+      h[(vi > vj ? vi : vj) + (long)(vi > vj ? vj : vi) * ldh] += g[i + j * ld];
+    }
+    for (int i = threadIdx.x; i < mk; i += blockDim.x) {
+      aw[v[i]] += g[ld * mk + i];
+      aq[v[i]] += g[ld * (mk + 1) + i];
+    }
+    if (threadIdx.x == 0) {
+      sc[0] += g[ld * (mk + 2)];
+      sc[1] += g[ld * (mk + 2) + 1];
+    }
+    __syncthreads();  // the next cone may share targets with this one
+  }
+}
+
 __global__ void LincombKernel(int n, const double* a, const double* x, long xs, const double* b,
                               const double* y, long ys, const double* c, const double* z, long zs,
                               double* out, long os, const int* active) {
@@ -436,7 +499,7 @@ int g_small_psd_mma = 2;
 int g_small_team_mode = 2;
 
 bool ValidCone(const cxb_small_cone* c) {
-  if (!c || c->n < 1 || c->m < 1 || !c->data || !c->state) return false;
+  if (!c || c->n < 1 || c->m < 1 || c->y_offset < 0 || !c->data || !c->state) return false;
   if (c->type == CXB_CONE_LP) return true;
   if (c->type == CXB_CONE_SOC) return c->work != nullptr;
   if (c->type == CXB_CONE_PSD) return c->work != nullptr && c->n <= 64;
@@ -862,6 +925,27 @@ int cxb_small_ldlt_solve(void* stream, int batch, int N, const double* dL, long 
     CountLaunch(); LdltSolveKernel<false><<<g.grid, g.threads, g.smem, AsStream(stream)>>>(
         batch, g.per, N, dL, ldl, lstride, d_perm, pstride, d_signs, sstride, dX, xstride, d_active);
   }
+  return LaunchStatus();
+}
+
+int cxb_small_gather(void* stream, int batch, int count, const int* d_idx, double* dy, long ystride, long dst,
+                     const int* d_active) {
+  if (batch <= 0 || count <= 0) return 0;
+  if (!d_idx || !dy || dst < 0 || ystride < dst + count) return -1;
+  CountLaunch();
+  GatherKernel<<<batch, kThreads, 0, AsStream(stream)>>>(count, d_idx, dy, ystride, dst, d_active);
+  return LaunchStatus();
+}
+
+int cxb_small_scatter_schur(void* stream, int batch, int ncones, const int* d_cones, const int* d_idx, const double* dS,
+                            long sstride, int m, double* dH, long ldh, long hstride, double* dAW, double* dAQc,
+                            long vstride, double* d_scal, long scal_stride, int accumulate, const int* d_active) {
+  if (batch <= 0 || (ncones <= 0 && accumulate)) return 0;
+  if (m < 1 || ldh < m || !dH || !dAW || !dAQc || !d_scal || (ncones > 0 && (!d_cones || !d_idx || !dS))) return -1;
+  CountLaunch();
+  ScatterSchurKernel<<<batch, kThreads, 0, AsStream(stream)>>>(ncones, d_cones, d_idx, dS, sstride, m, dH, ldh, hstride,
+                                                               dAW, dAQc, vstride, d_scal, scal_stride, accumulate,
+                                                               d_active);
   return LaunchStatus();
 }
 

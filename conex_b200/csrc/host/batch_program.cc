@@ -15,7 +15,10 @@ namespace conex {
 namespace {
 
 struct ConeSlot {
-  int type = 0, n = 0, m = 0, rows = 0;
+  int type = 0, n = 0, m = 0, rows = 0;  // m: the number of the cone's variables
+  std::vector<int> variables;            // empty for a cone on all variables in order (a full cone)
+  size_t gather_offset = 0;              // subset cones: the slice of y (cxb_small_gather) ...
+  size_t scratch_offset = 0;             // ... and the Schur block (cxb_small_scatter_schur) of each program
   size_t state_size = 0, work_size = 0;
   DeviceBuffer<double> data, state, work;
   DeviceBuffer<double> packed;  // LMI blocks: lower triangles of the matrices, for the slack passes
@@ -45,6 +48,14 @@ struct BatchProgram::Impl {
   int B = 0, m = 0, N = 0, multipliers = 0;
   long ldh = 0;
   size_t vstride = 0;
+  // Cones on variable subsets (`subset`: their indices into `cones`, in constraint order). Each program's y and y2
+  // carry the subset cones' slices of y behind the first vstride entries: ystride = vstride + gather_count. Their
+  // Schur blocks are assigned into `sub_schur` (stride sub_stride per program) and scatter-added into H.
+  std::vector<int> subset;
+  int gather_count = 0;
+  size_t ystride = 0, sub_stride = 0;
+  DeviceBuffer<int> gather_idx, sub_table;
+  DeviceBuffer<double> sub_schur;
   // per-program Newton system and vectors
   DeviceBuffer<double> H, AW, AQc, scal, b, y, y2;
   // with multipliers: the factors of the regularised LDL^T (H itself is kept, its equality rows are constant)
@@ -98,14 +109,41 @@ struct BatchProgram::Impl {
               "D2H outputs");
     ctx.Synchronize();
   }
+  // The order of DenseKKTSolver::Assemble: the first full cone assigns the leading m x m block of H, AW[0..m),
+  // AQc[0..m) and scal, the other full cones add to them. Each subset cone assigns its own block into sub_schur, and
+  // one scatter-add adds those blocks in, zeroing the targets first when no cone is full. Rows m..N-1 (the
+  // equality blocks) are never touched.
   void Assemble(const int* active) {
     bool first = true;
     for (auto& c : cones) {
+      if (!c.variables.empty()) continue;
       DeviceCheck(cxb_small_schur(s(), B, &c.desc, H.get(), ldh, ldh * N, AW.get(), AQc.get(), vstride,
                                   scal.get(), 2, first ? 0 : 1, active),
                   "cxb_small_schur");
       first = false;
     }
+    if (subset.empty()) return;
+    for (int k : subset) {
+      ConeSlot& c = cones[k];
+      const long ld = static_cast<long>(Align4(c.m));
+      double* g = sub_schur.get() + c.scratch_offset;
+      const long ss = static_cast<long>(sub_stride);
+      DeviceCheck(cxb_small_schur(s(), B, &c.desc, g, ld, ss, g + ld * c.m, g + ld * (c.m + 1), ss, g + ld * (c.m + 2),
+                                  ss, 0, active),
+                  "cxb_small_schur");
+    }
+    DeviceCheck(cxb_small_scatter_schur(s(), B, static_cast<int>(subset.size()), sub_table.get(), gather_idx.get(),
+                                        sub_schur.get(), static_cast<long>(sub_stride), m, H.get(), ldh, ldh * N,
+                                        AW.get(), AQc.get(), static_cast<long>(vstride), scal.get(), 2, first ? 0 : 1,
+                                        active),
+                "cxb_small_scatter_schur");
+  }
+  // The subset cones' slices of x (y or y2) behind its first vstride entries, before a slack pass reads them.
+  void Gather(double* x, const int* active) {
+    if (gather_count == 0) return;
+    DeviceCheck(cxb_small_gather(s(), B, gather_count, gather_idx.get(), x, static_cast<long>(ystride),
+                                 static_cast<long>(vstride), active),
+                "cxb_small_gather");
   }
   // The KKT factor and solve: Cholesky without multipliers, the regularised LDL^T with them, which never fails
   // (kkt_solver.cc:172-199: the input decides).
@@ -118,12 +156,12 @@ struct BatchProgram::Impl {
                                N, info.get() + 2 * static_cast<size_t>(B), active),
                 "cxb_small_ldlt");
   }
-  void Solve(double* x, const int* active) {
+  void Solve(double* x, const int* active) {  // x: y or y2 (stride ystride)
     if (multipliers == 0) {
-      DeviceCheck(cxb_small_potrs(s(), B, N, H.get(), ldh, ldh * N, x, vstride, active), "cxb_small_potrs");
+      DeviceCheck(cxb_small_potrs(s(), B, N, H.get(), ldh, ldh * N, x, ystride, active), "cxb_small_potrs");
       return;
     }
-    DeviceCheck(cxb_small_ldlt_solve(s(), B, N, L.get(), ldh, ldh * N, perm.get(), N, signs.get(), N, x, vstride,
+    DeviceCheck(cxb_small_ldlt_solve(s(), B, N, L.get(), ldh, ldh * N, perm.get(), N, signs.get(), N, x, ystride,
                                      active),
                 "cxb_small_ldlt_solve");
   }
@@ -140,7 +178,7 @@ BatchProgram::BatchProgram(const std::vector<Program*>& programs) : impl_(std::m
   constexpr int kEquality = -1;
   struct Shape {
     int type, n;                 // n: the order of a cone, the rows of an equality block
-    std::vector<int> variables;  // equality blocks: the columns of A
+    std::vector<int> variables;  // equality blocks: the columns of A; cones: their variables, empty when all in order
   };
   auto shape_of = [&](Container& c, Shape* sh) {
     sh->variables.clear();
@@ -168,12 +206,17 @@ BatchProgram::BatchProgram(const std::vector<Program*>& programs) : impl_(std::m
       throw std::runtime_error(
           "conex-b200: batched solves support LP, second-order and dense LMI cones and equality constraints");
     }
-    if (static_cast<int>(c.variables.size()) != m) {
-      throw std::runtime_error("conex-b200: batched solves need every cone on all variables");
+    // any list of distinct variables (Program::AddConstraint); 0..m-1 in order is a full cone
+    bool full = static_cast<int>(c.variables.size()) == m;
+    std::vector<char> seen(m, 0);
+    for (size_t i = 0; i < c.variables.size(); i++) {
+      const int v = c.variables[i];
+      if (v < 0 || v >= m || seen[v]) throw std::runtime_error("conex-b200: malformed variable list of a cone");
+      seen[v] = 1;
+      full = full && v == static_cast<int>(i);
     }
-    for (int i = 0; i < m; i++) {
-      if (c.variables[i] != i) throw std::runtime_error("conex-b200: batched solves need ordered cliques");
-    }
+    if (c.variables.empty()) throw std::runtime_error("conex-b200: a cone without variables");
+    if (!full) sh->variables = c.variables;
   };
   std::vector<Shape> shapes;
   for (auto& c : programs[0]->eqs) {
@@ -196,6 +239,7 @@ BatchProgram::BatchProgram(const std::vector<Program*>& programs) : impl_(std::m
       d.cones.emplace_back();
       d.cones.back().type = sh.type;
       d.cones.back().n = sh.n;
+      d.cones.back().variables = sh.variables;
     }
   }
   if (d.cones.empty()) throw std::runtime_error("conex-b200: batched programs have no cones");
@@ -204,22 +248,54 @@ BatchProgram::BatchProgram(const std::vector<Program*>& programs) : impl_(std::m
   }
   const int N = d.N = m + d.multipliers;
   const size_t nc = d.cones.size();
+  d.vstride = Align4(N);
   d.rank = 0;
+  // subset cones: their slices of y at 4-aligned offsets behind y, their Schur blocks in one scratch area per program
+  std::vector<int> gather_idx, sub_table;
   for (size_t k = 0; k < nc; k++) {
     ConeSlot& c = d.cones[k];
-    c.m = m;
+    if (c.variables.empty()) {
+      c.m = m;
+      continue;
+    }
+    c.m = static_cast<int>(c.variables.size());
+    c.gather_offset = gather_idx.size();
+    c.scratch_offset = d.sub_stride;
+    sub_table.insert(sub_table.end(), {c.m, static_cast<int>(c.gather_offset), static_cast<int>(c.scratch_offset)});
+    gather_idx.insert(gather_idx.end(), c.variables.begin(), c.variables.end());
+    gather_idx.resize(Align4(gather_idx.size()), -1);
+    d.sub_stride += Align4(c.m) * (c.m + 2) + 4;  // G_k | AW_k | AQc_k | 2 scalars
+    d.subset.push_back(static_cast<int>(k));
+  }
+  d.gather_count = static_cast<int>(gather_idx.size());
+  d.ystride = d.vstride + gather_idx.size();
+  if (!d.subset.empty()) {
+    d.gather_idx.Resize(gather_idx.size());
+    d.sub_table.Resize(sub_table.size());
+    d.sub_schur.Resize(d.sub_stride * B);
+    // pageable sources: they stay alive until the synchronisation after the packing below
+    CudaCheck(cudaMemcpyAsync(d.gather_idx.get(), gather_idx.data(), sizeof(int) * gather_idx.size(),
+                              cudaMemcpyHostToDevice, d.ctx.cuda_stream()),
+              "upload of the subset cones' variables");
+    CudaCheck(cudaMemcpyAsync(d.sub_table.get(), sub_table.data(), sizeof(int) * sub_table.size(),
+                              cudaMemcpyHostToDevice, d.ctx.cuda_stream()),
+              "upload of the subset cones' layout");
+  }
+  for (size_t k = 0; k < nc; k++) {
+    ConeSlot& c = d.cones[k];
     c.rows = c.type == CXB_CONE_LP ? c.n : (c.type == CXB_CONE_SOC ? c.n + 1 : c.n * c.n);
     c.rank = c.type == CXB_CONE_LP ? c.n : (c.type == CXB_CONE_SOC ? 2 : c.n);
     d.rank += c.rank;
     c.state_size = cxb_small_state_size(c.type, c.n);
-    c.work_size = cxb_small_work_size(c.type, c.n, m);
-    const size_t per = static_cast<size_t>(c.rows) * (m + 1);
+    c.work_size = cxb_small_work_size(c.type, c.n, c.m);
+    const size_t per = static_cast<size_t>(c.rows) * (c.m + 1);
     c.data.Resize(per * B);
     c.state.Resize(c.state_size * B);
     if (c.work_size) c.work.Resize(c.work_size * B);
     c.desc.type = c.type;
     c.desc.n = c.n;
-    c.desc.m = m;
+    c.desc.m = c.m;
+    c.desc.y_offset = c.variables.empty() ? 0 : static_cast<int>(d.vstride + c.gather_offset);
     c.desc.data = c.data.get();
     c.desc.data_stride = static_cast<long>(per);
     c.desc.state = c.state.get();
@@ -263,7 +339,7 @@ BatchProgram::BatchProgram(const std::vector<Program*>& programs) : impl_(std::m
         continue;
       }
       ConeSlot& slot = d.cones[d.slot_of[k]];
-      const size_t per = static_cast<size_t>(slot.rows) * (m + 1);
+      const size_t per = static_cast<size_t>(slot.rows) * (slot.m + 1);
       double* dst = slot.data.get() + per * p;
       if (sh.type == CXB_CONE_PSD) {
         auto* lmi = std::any_cast<DenseLMIConstraint>(&c.obj);
@@ -289,7 +365,7 @@ BatchProgram::BatchProgram(const std::vector<Program*>& programs) : impl_(std::m
     for (size_t k = 0; k < nc; k++) {
       ConeSlot& c = d.cones[k];
       if (c.type != CXB_CONE_PSD) continue;
-      const size_t stride = Align4(static_cast<size_t>(m + 1) * (static_cast<size_t>(c.n) * (c.n + 1) / 2));
+      const size_t stride = Align4(static_cast<size_t>(c.m + 1) * (static_cast<size_t>(c.n) * (c.n + 1) / 2));
       c.packed.Resize(stride * B);
       DeviceCheck(cxb_small_pack_symmetric(d.s(), B, &c.desc, c.packed.get(), static_cast<long>(stride),
                                            flags.get() + k),
@@ -302,7 +378,7 @@ BatchProgram::BatchProgram(const std::vector<Program*>& programs) : impl_(std::m
       if (c.type == CXB_CONE_PSD && !asymmetric[k]) {
         c.desc.packed = c.packed.get();
         c.desc.packed_stride =
-            static_cast<long>(Align4(static_cast<size_t>(m + 1) * (static_cast<size_t>(c.n) * (c.n + 1) / 2)));
+            static_cast<long>(Align4(static_cast<size_t>(c.m + 1) * (static_cast<size_t>(c.n) * (c.n + 1) / 2)));
       } else {
         c.packed.Resize(0);
       }
@@ -311,7 +387,6 @@ BatchProgram::BatchProgram(const std::vector<Program*>& programs) : impl_(std::m
   }
   // ---- Newton-system storage ------------------------------------------------------------------------
   d.ldh = static_cast<long>(Align4(N));
-  d.vstride = Align4(N);
   d.H.Resize(static_cast<size_t>(d.ldh) * N * B);
   if (d.multipliers) {
     d.L.Resize(static_cast<size_t>(d.ldh) * N * B);
@@ -322,15 +397,15 @@ BatchProgram::BatchProgram(const std::vector<Program*>& programs) : impl_(std::m
   d.AQc.Resize(d.vstride * B);
   d.scal.Resize(2 * static_cast<size_t>(B));
   d.b.Resize(d.vstride * B);
-  d.y.Resize(d.vstride * B);
-  d.y2.Resize(d.vstride * B);
+  d.y.Resize(d.ystride * B);
+  d.y2.Resize(d.ystride * B);
   d.coef.Resize(5 * static_cast<size_t>(B));
   d.out.Resize(static_cast<size_t>(B) * (4 * nc + 4));
   d.info.Resize((d.multipliers ? 3 : 2) * static_cast<size_t>(B));
   d.mask.Resize(3 * static_cast<size_t>(B));
   d.asymmetric.Resize(1);
   d.hcoef.Reserve(std::max<size_t>(5 * static_cast<size_t>(B), d.vstride * B));
-  d.hout.Reserve(std::max<size_t>(static_cast<size_t>(B) * (4 * nc + 4), d.vstride * B));
+  d.hout.Reserve(std::max<size_t>(static_cast<size_t>(B) * (4 * nc + 4), d.ystride * B));
   d.hinfo.Reserve(2 * static_cast<size_t>(B));
   d.hmask.Reserve(3 * static_cast<size_t>(B));
   d.b_scaling.assign(B, 1.0);
@@ -380,7 +455,7 @@ bool BatchProgram::ConstraintDataShape(int constraint, int* rows, int* columns) 
   if (constraint < 0 || constraint >= static_cast<int>(d.slot_of.size())) return false;
   const int k = d.slot_of[constraint];
   *rows = k < 0 ? d.equalities[-1 - k].rows : d.cones[k].rows;
-  *columns = k < 0 ? static_cast<int>(d.equalities[-1 - k].variables.size()) + 1 : d.m + 1;
+  *columns = k < 0 ? static_cast<int>(d.equalities[-1 - k].variables.size()) + 1 : d.cones[k].m + 1;
   return true;
 }
 
@@ -442,6 +517,7 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
   const int B = batch_, m = m_, N = d.N;
   const size_t nc = d.cones.size();
   const size_t vs = d.vstride;
+  const size_t ys = d.ystride;  // y and y2
   const bool warm = cfg.initialization_mode != CONEX_INITIALIZATION_MODE_COLDSTART;
   if (warm && !d.initialised) {
     throw std::runtime_error("conex-b200: a warm start needs a previous solve of the batch");
@@ -488,7 +564,7 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
   CudaCheck(cudaMemcpyAsync(d.b.get(), d.hcoef.get(), sizeof(double) * vs * B, cudaMemcpyHostToDevice, cs),
             "H2D cost vectors");
   d.ctx.Synchronize();  // hcoef is reused below
-  d.ctx.Zero(d.y.get(), vs * B);
+  d.ctx.Zero(d.y.get(), ys * B);
   const int ncones = static_cast<int>(nc);
   if (!warm) {
     DeviceCheck(cxb_small_set_identity_multi(s, B, ncones, d.descs.data(), nullptr), "cxb_small_set_identity_multi");
@@ -615,10 +691,11 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
       d.UploadCoef(0, 2 * static_cast<size_t>(B));
       d.UploadCoef(3 * static_cast<size_t>(B), B);
       DeviceCheck(cxb_batched_lincomb(s, B, N, coef_a, d.AQc.get(), vs, coef_b, d.b.get(), vs, nullptr, nullptr, 0,
-                                      d.y.get(), vs, mu_mask),
+                                      d.y.get(), ys, mu_mask),
                   "cxb_batched_lincomb");
       d.Solve(d.y.get(), mu_mask);
-      DeviceCheck(cxb_small_eigen_multi(s, B, ncones, d.descs.data(), d.y.get(), vs, 0.0, coef_cw, cone_out, ostride,
+      d.Gather(d.y.get(), mu_mask);
+      DeviceCheck(cxb_small_eigen_multi(s, B, ncones, d.descs.data(), d.y.get(), ys, 0.0, coef_cw, cone_out, ostride,
                                         mu_mask),
                   "cxb_small_eigen_multi");
       d.DownloadOut(static_cast<size_t>(B) * 4 * nc);
@@ -669,10 +746,11 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
     // ---- Newton direction: y = H^{-1} (k (b b_s + AQc c_s) - 2 AW) (cone_program.cc:409-414) ------
     d.UploadCoef(0, 4 * static_cast<size_t>(B));
     DeviceCheck(cxb_batched_lincomb(s, B, N, coef_a, d.b.get(), vs, coef_b, d.AQc.get(), vs, coef_c, d.AW.get(), vs,
-                                    d.y.get(), vs, active),
+                                    d.y.get(), ys, active),
                 "cxb_batched_lincomb");
     d.Solve(d.y.get(), active);
-    DeviceCheck(cxb_small_prepare_multi(s, B, ncones, d.descs.data(), d.y.get(), vs, 0, 0.0, coef_cw, 1.0, cone_out,
+    d.Gather(d.y.get(), active);
+    DeviceCheck(cxb_small_prepare_multi(s, B, ncones, d.descs.data(), d.y.get(), ys, 0, 0.0, coef_cw, 1.0, cone_out,
                                         ostride, active),
                 "cxb_small_prepare_multi");
     d.DownloadOut(static_cast<size_t>(B) * 4 * nc);
@@ -711,8 +789,8 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
     DeviceCheck(cxb_small_take_step_multi(s, B, ncones, d.descs.data(), 1.0, coef_step, 1.0, d.info.get() + B, active),
                 "cxb_small_take_step_multi");
     // ---- objectives (cone_program.cc:441-467) -------------------------------------------------------
-    DeviceCheck(cxb_batched_dot(s, B, N, d.b.get(), vs, d.y.get(), vs, dots + 0, 4), "cxb_batched_dot");
-    DeviceCheck(cxb_batched_dot(s, B, N, d.AQc.get(), vs, d.y.get(), vs, dots + 1, 4), "cxb_batched_dot");
+    DeviceCheck(cxb_batched_dot(s, B, N, d.b.get(), vs, d.y.get(), ys, dots + 0, 4), "cxb_batched_dot");
+    DeviceCheck(cxb_batched_dot(s, B, N, d.AQc.get(), vs, d.y.get(), ys, dots + 1, 4), "cxb_batched_dot");
     CudaCheck(cudaEventRecord(ev_b, cs), "cudaEventRecord");
     CudaCheck(cudaMemcpyAsync(d.hout.get(), dots, sizeof(double) * 4 * B, cudaMemcpyDeviceToHost, cs), "D2H dots");
     CudaCheck(cudaMemcpyAsync(d.hout.get() + 4 * static_cast<size_t>(B), d.scal.get(), sizeof(double) * 2 * B,
@@ -743,7 +821,7 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
   }
 
   // ---- results (cone_program.cc:486-530) -------------------------------------------------------------
-  CudaCheck(cudaMemcpyAsync(d.hout.get(), d.y.get(), sizeof(double) * vs * B, cudaMemcpyDeviceToHost, cs), "D2H y");
+  CudaCheck(cudaMemcpyAsync(d.hout.get(), d.y.get(), sizeof(double) * ys * B, cudaMemcpyDeviceToHost, cs), "D2H y");
   d.ctx.Synchronize();
   int solved_count = 0;
   bool any_recover = false;
@@ -758,7 +836,7 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
     r.c_scaling = d.c_scaling[p] = q.c_scaling;
     r.d_inf = q.d_inf;
     double* yp = y_out + static_cast<size_t>(p) * m;
-    for (int j = 0; j < m; j++) yp[j] = d.hout[p * vs + j];
+    for (int j = 0; j < m; j++) yp[j] = d.hout[p * ys + j];
     d.hmask[p] = 0;
     if (q.failed) {
       r.solved = 0;
@@ -791,10 +869,11 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
     }
     d.UploadCoef(0, 2 * static_cast<size_t>(B));
     DeviceCheck(cxb_batched_lincomb(s, B, N, coef_a, d.b.get(), vs, coef_b, d.AW.get(), vs, nullptr, nullptr, 0,
-                                    d.y2.get(), vs, active),
+                                    d.y2.get(), ys, active),
                 "cxb_batched_lincomb");
     d.Solve(d.y2.get(), active);
-    DeviceCheck(cxb_small_prepare_multi(s, B, ncones, d.descs.data(), d.y2.get(), vs, 1, 0.0, nullptr, 0.0, cone_out,
+    d.Gather(d.y2.get(), active);
+    DeviceCheck(cxb_small_prepare_multi(s, B, ncones, d.descs.data(), d.y2.get(), ys, 1, 0.0, nullptr, 0.0, cone_out,
                                         ostride, active),
                 "cxb_small_prepare_multi");
   }

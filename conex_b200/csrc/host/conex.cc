@@ -557,6 +557,39 @@ int CONEXB200_AddSocConstraint(void* prog, int n, int m, const double* A, const 
       -1);
 }
 
+// The LP cone and the second-order cone on a list of variables, like CONEX_AddSparseLMIConstraint for LMIs:
+// c - A y[vars] >= 0 (A is rows x nvars) and c - A y[vars] in the Lorentz cone of order n + 1 (A is (n + 1) x nvars),
+// column-major. Duplicate or out-of-range variables add nothing and return -1; otherwise the constraint id.
+int CONEXB200_AddSparseLinearConstraint(void* prog, const double* A, int rows, int nvars, const double* c,
+                                        const long* vars) {
+  return Guard(
+      [&]() -> int {
+        Program& program = *static_cast<Program*>(prog);
+        if (rows < 1 || nvars < 1 || !vars) return -1;
+        std::vector<int> variables(nvars);
+        for (int i = 0; i < nvars; i++) variables[i] = static_cast<int>(vars[i]);
+        const int id = program.NumberOfConstraints();
+        if (program.AddConstraint(LinearConstraint(rows, nvars, A, c), variables)) return -1;
+        return id;
+      },
+      -1);
+}
+
+int CONEXB200_AddSparseSocConstraint(void* prog, int n, int nvars, const double* A, const double* c,
+                                     const long* vars) {
+  return Guard(
+      [&]() -> int {
+        Program& program = *static_cast<Program*>(prog);
+        if (n < 1 || nvars < 1 || !vars) return -1;
+        std::vector<int> variables(nvars);
+        for (int i = 0; i < nvars; i++) variables[i] = static_cast<int>(vars[i]);
+        const int id = program.NumberOfConstraints();
+        if (program.AddConstraint(SOCConstraint(n, nvars, A, c), variables)) return -1;
+        return id;
+      },
+      -1);
+}
+
 // Program::AddConstraint(EqualityConstraints{A, b}[, vars]) (cone_program.h:193-217); A is
 // rows x nvars column-major, vars == NULL: all variables. Returns the constraint id or -1.
 int CONEXB200_AddEqualityConstraint(void* prog, int rows, int nvars, const double* A, const double* b,

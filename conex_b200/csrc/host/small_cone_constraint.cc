@@ -34,6 +34,7 @@ cxb_small_cone SmallConeConstraint::Descriptor() {
   c.type = type_;
   c.n = n_;
   c.m = m_;
+  c.y_offset = 0;
   c.data = d.data.get();
   c.data_stride = 0;
   c.state = workspace_.state;

@@ -110,15 +110,104 @@ def small_multicone_equality_problem(seed, equalities=((8, None, None),), y0_sca
 
 
 def add_cones(P, cones):
-    for kind, A, c in cones:
-        if kind == "psd":
+    """Adds the constraints of a generator's list to P. A cone entry may carry a fourth element, the list of
+    variables its columns act on (dense LMIs through CONEX_AddSparseLMIConstraint, LP and second-order cones through
+    CONEXB200_AddSparseLinearConstraint / CONEXB200_AddSparseSocConstraint); without one it acts on all variables."""
+    for entry in cones:
+        kind, A, c = entry[:3]
+        variables = entry[3] if len(entry) > 3 else None
+        if kind == "eq":
+            P.add_equality(A, c[0], c[1])
+        elif variables is not None:
+            if kind == "psd":
+                P.add_dense_lmi(A, c, variables)
+            elif kind == "soc":
+                P.add_soc(A, c, variables=variables)
+            else:
+                P.add_linear(A, c, variables=variables)
+        elif kind == "psd":
             P.add_dense_lmi(A, c)
         elif kind == "soc":
             P.add_soc(A, c)
-        elif kind == "eq":
-            P.add_equality(A, c[0], c[1])
         else:
             P.add_linear(A, c)
+
+
+def pad_cones(cones, m):
+    """The same constraints with every cone on all m variables in order: zero columns (LMIs: zero matrices) for the
+    variables a cone does not act on. Equality blocks are kept as they are."""
+    out = []
+    for entry in cones:
+        kind, A, c = entry[:3]
+        variables = entry[3] if len(entry) > 3 else None
+        if kind == "eq" or variables is None:
+            out.append((kind, A, c))
+        elif kind == "psd":
+            mats = [np.zeros_like(c, dtype=np.float64) for _ in range(m)]
+            for j, v in enumerate(variables):
+                mats[v] = A[j]
+            out.append((kind, mats, c))
+        else:
+            Ap = np.zeros((A.shape[0], m))
+            Ap[:, list(variables)] = A
+            out.append((kind, Ap, c))
+    return out
+
+
+def mpc_problem(seed, stages=8, stage_vars=6, lp_rows=12, soc_order=6, lmi_order=8, eq_rows=4, y0_scale=0.02):
+    """A program shaped like a model-predictive-control horizon: `stages` stages of `stage_vars` variables
+    (m = stages * stage_vars). Per stage, an LP block of `lp_rows` rows (A uniform, c = 1) and a Lorentz cone of
+    order `soc_order` (A uniform, c = e_0) on the stage's variables; per pair of adjacent stages, a dense LMI of order
+    `lmi_order` (A_i = sym(U[-1,1]), C = I) and an equality block of `eq_rows` rows on the two stages' variables.
+    Constraint order: stage s's LP and SOC, then (s > 0) the LMI and the equality block coupling s - 1 and s.
+    Strictly feasible by construction, like small_multicone_equality_problem: b = sum over cones of AW/2 at W = I plus
+    A_eq^T lambda0, and b_eq = A_eq y0[variables] for a y0 at which every cone slack is interior.
+    Returns (cones, padded, b): the list in the add_cones format with a variable list per cone, the same program
+    with every cone on all m variables (pad_cones), and b."""
+    rng = np.random.Generator(np.random.PCG64(seed))
+    m = stages * stage_vars
+    b = np.zeros(m)
+    cones = []
+    couplings = []
+    for s in range(stages):
+        v = list(range(s * stage_vars, (s + 1) * stage_vars))
+        A = rng.uniform(-1.0, 1.0, size=(lp_rows, stage_vars))
+        cones.append(("lp", A, np.ones(lp_rows), v))
+        np.add.at(b, v, 0.5 * A.sum(axis=0))
+        A = rng.uniform(-1.0, 1.0, size=(soc_order + 1, stage_vars))
+        c = np.zeros(soc_order + 1)
+        c[0] = 1.0
+        cones.append(("soc", A, c, v))
+        np.add.at(b, v, A[0, :])
+        if s > 0:
+            w = list(range((s - 1) * stage_vars, (s + 1) * stage_vars))
+            mats = [random_sym(rng, lmi_order) for _ in w]
+            cones.append(("psd", mats, np.eye(lmi_order), w))
+            np.add.at(b, w, 0.5 * np.array([np.trace(M) for M in mats]))
+            couplings.append((len(cones), w))
+    # an interior y0: halved until every cone slack is interior with a margin
+    y0 = y0_scale * rng.uniform(-1.0, 1.0, size=m)
+
+    def margin(y):
+        out = np.inf
+        for kind, A, c, v in cones:
+            if kind == "psd":
+                out = min(out, np.linalg.eigvalsh(c - sum(yi * Ai for yi, Ai in zip(y[v], A))).min())
+            elif kind == "soc":
+                sl = c - A @ y[v]
+                out = min(out, sl[0] - np.linalg.norm(sl[1:]))
+            else:
+                out = min(out, (c - A @ y[v]).min())
+        return out
+
+    while margin(y0) <= 0.1:
+        y0 *= 0.5
+    for position, w in reversed(couplings):  # after each LMI; reversed: earlier positions stay valid
+        A_eq = rng.uniform(-1.0, 1.0, size=(eq_rows, len(w)))
+        lam0 = rng.uniform(-1.0, 1.0, size=eq_rows)
+        np.add.at(b, w, A_eq.T @ lam0)
+        cones.insert(position, ("eq", A_eq, (A_eq @ y0[w], w)))
+    return cones, pad_cones(cones, m), b
 
 
 def block_arrow_program(blocks, private, shared, order, seed):

@@ -143,6 +143,16 @@ int CONEXB200_DeviceAvailable();
 /* SOCConstraint(A, c) (conex/soc_constraint.h:9-15): c - A y in the Lorentz cone of R^{n+1};
  * A is (n + 1) x m column-major. Returns the constraint id. */
 int CONEXB200_AddSocConstraint(void* prog, int n, int m, const double* A, const double* c);
+/* The LP cone and the second-order cone on a list of `nvars` distinct variables `vars`, like
+ * CONEX_AddSparseLMIConstraint for LMIs (Program::AddConstraint(cone, variables)):
+ *   CONEXB200_AddSparseLinearConstraint: c - A y[vars] >= 0, A rows x nvars column-major, c `rows` entries;
+ *   CONEXB200_AddSparseSocConstraint:    c - A y[vars] in the Lorentz cone of R^{n+1}, A (n + 1) x nvars.
+ * The program's number of variables must be set. Duplicate or out-of-range variables add nothing and return -1;
+ * otherwise the constraint id. */
+int CONEXB200_AddSparseLinearConstraint(void* prog, const double* A, int rows, int nvars, const double* c,
+                                        const long* vars);
+int CONEXB200_AddSparseSocConstraint(void* prog, int n, int nvars, const double* A, const double* c,
+                                     const long* vars);
 /* Program::AddConstraint(EqualityConstraints{A, b}[, vars]) (conex/cone_program.h:193-217):
  * A y[vars] = b, A rows x nvars column-major, vars == NULL means all variables. The multipliers
  * become extra unknowns of the KKT system, which is then factored by the regularised LDL^T. */
@@ -188,9 +198,12 @@ void CONEXB200_RldltPivotOrder(int n, const double* diag, int* perm);
 
 /* ---- many small programs in lock step (BASELINE config 3) ------------------------------------
  * `programs`: `count` handles built through the CONEX_* calls with identical structure (same number
- * of variables, same list of LP / second-order / dense-LMI cones, every cone on all variables, and
- * the same equality blocks — rows, variable subset, position among the cones — e.g. the lb == ub rows
- * of CONEX_AddLinearInequalities; at least one cone). CONEXB200_CreateBatch packs their data into
+ * of variables, same list of LP / second-order / dense-LMI cones, each on the same list of distinct
+ * variables in every program — all of them, or any subset in any order, as CONEX_AddSparseLMIConstraint,
+ * CONEXB200_AddSparseLinearConstraint and CONEXB200_AddSparseSocConstraint build them — and the same
+ * equality blocks — rows, variable subset, position among the cones — e.g. the lb == ub rows of
+ * CONEX_AddLinearInequalities; at least one cone). A variable that no cone covers leaves the KKT
+ * system singular, as in CONEX_Maximize. CONEXB200_CreateBatch packs their data into
  * batched device arrays (the handles may be deleted afterwards); it returns NULL for mismatched
  * structures. CONEXB200_BatchMaximize solves all of them: b and y are m x count column-major HOST
  * arrays, solved[p] / the return value follow CONEX_Maximize (1 = solved; the return value is the
@@ -213,15 +226,18 @@ int CONEXB200_BatchStepMilliseconds(void* batch, double* out, int capacity);
  * numbering); returns its size. Equality blocks have none: nothing is written, the return value is 0. */
 int CONEXB200_BatchGetDualVariable(void* batch, int program, int cone, double* x);
 /* Replaces columns [first, first + count) of the data of constraint `constraint` (numbered like
- * CONEX_GetDualVariable, equality blocks included) in every program of the batch. Cones: column j < m holds
- * the coefficients of y_j (LP: column j of A; SOC: column j of the (n + 1) x m A; LMI: vec(A_j)), column m the
- * affine term (c / C). Equality blocks: column j < nvars is column j of A, column nvars is b.
+ * CONEX_GetDualVariable, equality blocks included) in every program of the batch. Cones on all m variables:
+ * column j < m holds the coefficients of y_j (LP: column j of A; SOC: column j of the (n + 1) x m A; LMI:
+ * vec(A_j)), column m the affine term (c / C). Cones on a list of m_k variables v: column j < m_k holds the
+ * coefficients of y[v_j], column m_k the affine term. Equality blocks: column j < nvars is column j of A,
+ * column nvars is b.
  * data: host memory, B blocks of rows x count column-major (program p at data + p * rows * count).
  * Returns 0, or -1 on bad arguments (the batch is then unchanged). The next BatchMaximize uses the new data;
  * a warm start continues from the iterate of the previous solve. */
 int CONEXB200_BatchUpdateConstraintData(void* batch, int constraint, int first, int count, const double* data);
 /* The shape of that data for constraint `constraint`: *rows (cones: n for LP, n + 1 for SOC, n * n for LMI; equality
- * blocks: their rows) and *columns (cones: m + 1; equality blocks: nvars + 1). Returns 0, or -1 when the batch has no
+ * blocks: their rows) and *columns (cones: m_k + 1 for a cone on m_k variables, m + 1 on all of them; equality
+ * blocks: nvars + 1). Returns 0, or -1 when the batch has no
  * such constraint. The caller of CONEXB200_BatchUpdateConstraintData must pass blocks of exactly these rows. */
 int CONEXB200_BatchConstraintDataShape(void* batch, int constraint, int* rows, int* columns);
 

@@ -27,6 +27,11 @@
 // constraint's data in every program on the device, so that the next instance of a parametric
 // problem is solved without building a new batch.
 //
+// Cones on variable subsets: each runs the cone kernels on its own m_k variables. Before each slack
+// pass one gather copies their slices of y behind each program's y (the cone descriptors' y_offset
+// points there); their Schur blocks go to scratch, and one scatter-add puts them into H, AW, AQc and
+// the scalars after the full cones' kernels (the order of DenseKKTSolver::Assemble).
+//
 // Packed copies of the LMI operators: an update refreshes the lower triangles of the changed
 // matrices only; data that is not symmetric bit for bit drops the cone's packed copy for the life of
 // the batch (the slack passes then read the full matrices), as the constructor does.
@@ -50,8 +55,9 @@ struct BatchResult {
 class BatchProgram {
  public:
   // All programs must have the same number of variables and the same list of constraints: cones
-  // (LP, second-order, dense LMI; type, order) on all variables in order, and equality blocks (rows,
-  // variable subset) at the same positions among them; at least one cone. Throws otherwise.
+  // (LP, second-order, dense LMI; type, order, list of distinct variables — all of them in order, or
+  // any subset in any order) and equality blocks (rows, variable subset) at the same positions among
+  // them; at least one cone. Throws otherwise.
   explicit BatchProgram(const std::vector<Program*>& programs);
   ~BatchProgram();
 
@@ -61,7 +67,8 @@ class BatchProgram {
   // (config.initialization_mode != cold start) throws when the batch has never been solved.
   int Maximize(const double* b, const SolverConfiguration& config, double* y);
   // Replaces columns [first, first + count) of the data of constraint `constraint` (numbered like
-  // GetDualVariable) in every program: cones [A | c] (rows x (m + 1); LMI: vec(A_j) and vec(C)),
+  // GetDualVariable) in every program: cones [A | c] (rows x (m_k + 1) for a cone on m_k variables,
+  // column j for its j-th variable; LMI: vec(A_j) and vec(C)),
   // equality blocks [A | b] (rows x (nvars + 1)). data: B host blocks of rows x count, column-major,
   // program p at data + p * rows * count. Throws on bad arguments before anything is written.
   void UpdateConstraintData(int constraint, int first, int count, const double* data);

@@ -271,10 +271,16 @@ int cxb_affine_update(void* stream, int n, double* dW, const double* dWSW, doubl
  *          SOC (W0, W1)[n + 1] at 0, d[n + 1] at op (op = n + 1 rounded up to 4)
  *          PSD W, T1, T2 (n x n each) at 0, nnp, 2 nnp (nnp = n * n rounded up to 4)
  *   work : SOC (n + 1) * (m + 4) doubles; PSD (m + 2) * n * n doubles; LP none.
+ *   y_offset: where the cone's y starts in the slack kernels' y argument (cxb_small_eigen / cxb_small_prepare and their
+ *          _multi forms): program p reads y[p * ystride + y_offset + j], j < m. 0 for a cone on all variables; a cone
+ *          on a subset of a program's variables reads the slice that cxb_small_gather placed behind the program's y.
+ *          It fills the padding after `m`, so the size and layout of the struct are those of earlier releases, and
+ *          a zero-initialised descriptor reads y from its start.
  * active (device ints, may be NULL) masks programs that must not be touched. */
 enum { CXB_CONE_LP = 0, CXB_CONE_SOC = 1, CXB_CONE_PSD = 2 };
 typedef struct {
   int type, n, m;
+  int y_offset;
   const double* data;
   long data_stride;
   double* state;
@@ -346,6 +352,22 @@ int cxb_small_take_step_multi(void* stream, int batch, int ncones, const cxb_sma
 void cxb_set_small_cone_threads(int threads);
 /* A/B switch: 0 = the *_multi entry points launch their cones one after the other (default 1). */
 void cxb_set_small_fused_launches(int enabled);
+/* Cones on variable subsets in a batch: the gather of their y slices and the scatter-add of their Schur blocks.
+ * cxb_small_gather: y[p * ystride + dst + i] = y[p * ystride + d_idx[i]] for i < count with d_idx[i] >= 0 (entries
+ * < 0 are padding and leave their slot alone). Every d_idx[i] must be < dst: the sources, a program's variables,
+ * lie before the destination slices. One CTA per program. */
+int cxb_small_gather(void* stream, int batch, int count, const int* d_idx, double* dy, long ystride, long dst,
+                     const int* d_active);
+/* The batched counterpart of cxb_scatter_add_lower + cxb_scatter_add_vec: for the subset cones k < ncones in order,
+ * d_cones[3 k ..] = {m_k, first, offset}: the cone's variables are d_idx[first .. first + m_k), and its Schur
+ * block (cxb_small_schur with accumulate = 0) lies at dS + p * sstride + offset as G_k (m_k x m_k lower triangle,
+ * ld = m_k rounded up to 4), then AW_k and AQc_k (ld doubles each), then its two scalars. Adds G_k[i, j], i >= j,
+ * to H[max(v_i, v_j), min(v_i, v_j)], AW_k / AQc_k to AW / AQc at v, the scalars to scal[0..1]. accumulate == 0
+ * first zeroes the leading m x m block of H, AW[0..m), AQc[0..m) and scal[0..1]. One CTA per program; the cones
+ * are added one after the other (no atomics: the result does not depend on scheduling). */
+int cxb_small_scatter_schur(void* stream, int batch, int ncones, const int* d_cones, const int* d_idx, const double* dS,
+                            long sstride, int m, double* dH, long ldh, long hstride, double* dAW, double* dAQc,
+                            long vstride, double* d_scal, long scal_stride, int accumulate, const int* d_active);
 /* Cholesky of `batch` N x N matrices (lower, ld, stride) and solves with nrhs = 1; d_info[p] = 0 or
  * 1 + first non-positive pivot (block_triangular_operations.cc:184-219, :114-182). */
 int cxb_small_potrf(void* stream, int batch, int N, double* dH, long ldh, long hstride, int* d_info,
