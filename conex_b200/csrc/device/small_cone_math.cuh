@@ -1237,5 +1237,150 @@ CXB_HD void SmallLdltSolve(T& t, int N, const double* L, long ld, const int* per
   t.par(N, [&](int i) { x[perm[i]] = sx[i]; });
 }
 
+// =================================================================================================
+// KKT systems whose N x N matrix does not fit in shared memory (cxb_small_potrf / cxb_small_ldlt above the sizes of
+// SmallPotrf / SmallLdlt): the same two factorisations, blocked and right-looking, in place in global memory. Per
+// block column of kKktNb columns: the diagonal block is factored in shared memory with the per-column arithmetic of
+// SmallPotrf / SmallLdlt; the panel below it is solved one row per thread (the row in registers, the block's
+// columns in sequence); the trailing matrix takes A22 -= L21 S L21^T on its lower triangle (`update`: the DMMA tiles
+// of small_cones.cu on the device, KktTrailingUpdateLoop on the host). The scratch does not depend on N.
+// =================================================================================================
+constexpr int kKktNb = 32;
+constexpr int kKktPitch = kKktNb + 1;  // odd pitch of the diagonal block
+// sm: the diagonal block, then per column the scale (Cholesky: sqrt(d); LDL^T: sign / sqrt|d|) and the sign
+CXB_HOST_DEVICE long BlockedKktSmemDoubles() { return (long)kKktNb * kKktPitch + 2 * kKktNb; }
+
+// A22 -= L21 S L21^T on the lower triangle: the trailing R x R matrix at (t0, t0) of A, L21 = the kb columns from k0
+// of its rows, S = s[0..kb). Plain team loop; the product's kernels use DMMA tiles instead.
+struct KktTrailingUpdateLoop {
+  template <class T>
+  CXB_HD void operator()(T& t, double* A, long ld, int k0, int kb, int t0, int R, const double* s) const {
+    const Divider by_R(R);
+    t.par(R * R, [&](int e) {
+      const int c = by_R.quot(e), r = e - c * R;
+      if (r < c) return;
+      double acc = 0;
+      for (int k = 0; k < kb; k++) {
+        const double* col = A + (long)(k0 + k) * ld + t0;
+        acc += col[r] * (s[k] * col[c]);
+      }
+      A[(long)(t0 + c) * ld + t0 + r] -= acc;
+    });
+  }
+};
+
+// The factorisation of A (N x N lower, ld) in place. LDLT == false: Cholesky; returns 0, or 1 + the first column
+// whose pivot is not > 0 (A is then left partly factored). LDLT == true: the regularised L S L^T of SmallLdlt, S
+// written to signs; returns 1 when some pivot was regularised, else 0. Either way the diagonal keeps the
+// (unregularised) pivot until its block column is done, then stores sqrt|reg(d)|.
+template <bool LDLT, class T, class U>
+CXB_HD int BlockedFactor(T& t, int N, double* A, long ld, double* signs, double* sm, const U& update) {
+  constexpr int P = kKktPitch;
+  double* sD = sm;
+  double* sScale = sm + kKktNb * P;
+  double* sSign = sScale + kKktNb;
+  int regularised = 0;
+  for (int k0 = 0; k0 < N; k0 += kKktNb) {
+    const int kb = (N - k0 < kKktNb) ? N - k0 : kKktNb;
+    double* Ak = A + (long)k0 * ld + k0;  // the diagonal block
+    t.par(kb * kb, [&](int e) {
+      const int c = e / kb, r = e - c * kb;
+      if (r >= c) sD[c * P + r] = Ak[(long)c * ld + r];
+    });
+    for (int j = 0; j < kb; j++) {
+      double d = sD[j * P + j];
+      double sign = 1.0;
+      if (LDLT) {
+        if (!(fabs(d) > 1e-9)) regularised = 1;
+        d = RegularisedPivot(d);
+        sign = (d < 0) ? -1.0 : 1.0;
+      } else if (!(d > 0.0)) {
+        return k0 + j + 1;  // d is the same in every thread
+      }
+      const double scale = LDLT ? sign * (1.0 / sqrt(fabs(d))) : sqrt(d);
+      t.par(kb - j, [&](int i) {
+        if (i == 0) {
+          sScale[j] = scale;
+          sSign[j] = sign;
+        } else if (LDLT) {
+          sD[j * P + j + i] *= scale;
+        } else {
+          sD[j * P + j + i] /= scale;
+        }
+      });
+      const int w = kb - j - 1;
+      t.par2(
+          w, w, [&](int i) { return sD[j * P + j + 1 + i]; },
+          [&](int i, int c, double lr) {
+            if (i >= c) sD[(j + 1 + c) * P + j + 1 + i] -= lr * (sign * sD[j * P + j + 1 + c]);
+          });
+    }
+    t.par(kb * kb, [&](int e) {
+      const int c = e / kb, r = e - c * kb;
+      if (r > c) Ak[(long)c * ld + r] = sD[c * P + r];
+      if (r == c) {
+        const double d = LDLT ? RegularisedPivot(sD[c * P + r]) : sD[c * P + r];
+        Ak[(long)c * ld + r] = sqrt(fabs(d));
+        if (LDLT) signs[k0 + r] = (d < 0) ? -1.0 : 1.0;
+      }
+    });
+    // the panel: row i of L21 = row i of A21 solved against the block's columns, the same steps as its entries take
+    // in SmallPotrf / SmallLdlt once the earlier blocks' updates are in
+    const int t0 = k0 + kb, R = N - t0;
+    if (R == 0) break;
+    t.par(R, [&](int i) {
+      double* row = A + (long)k0 * ld + t0 + i;  // entry (t0 + i, k0 + c) at row[c * ld]
+      double x[kKktNb];
+#pragma unroll
+      for (int c = 0; c < kKktNb; c++) x[c] = (c < kb) ? row[(long)c * ld] : 0.0;
+#pragma unroll
+      for (int j = 0; j < kKktNb; j++) {
+        if (j < kb) {
+          x[j] = LDLT ? x[j] * sScale[j] : x[j] / sScale[j];
+          const double sj = sSign[j];
+#pragma unroll
+          for (int c = j + 1; c < kKktNb; c++)
+            if (c < kb) x[c] -= x[j] * (sj * sD[j * P + c]);
+        }
+      }
+#pragma unroll
+      for (int c = 0; c < kKktNb; c++)
+        if (c < kb) row[(long)c * ld] = x[c];
+    });
+    update(t, A, ld, k0, kb, t0, R, sSign);
+  }
+  return LDLT ? regularised : 0;
+}
+
+// Cholesky of H (N x N lower, ld) in place: 0, or 1 + the first column whose pivot is not > 0 (H is then
+// unspecified). sm: BlockedKktSmemDoubles() doubles.
+template <class T, class U>
+CXB_HD int BlockedPotrf(T& t, int N, double* H, long ld, double* sm, const U& update) {
+  return BlockedFactor<false>(t, N, H, ld, nullptr, sm, update);
+}
+
+// SmallLdlt without the N x N shared copy: the pivot order of RldltPivotOrder (warp 0), P K P^T gathered from the
+// lower triangle of K straight into L, then L factored in place. K is not modified. sm: BlockedKktSmemDoubles()
+// doubles; sd: N doubles, at: N ints (shared).
+template <class T, class U>
+CXB_HD int BlockedLdlt(T& t, int N, const double* K, long ldk, double* L, long ldl, int* perm, double* signs,
+                       double* sm, double* sd, int* at, const U& update) {
+  t.par(N, [&](int i) {
+    sd[i] = fabs(K[(long)i * ldk + i]);
+    at[i] = i;
+  });
+  t.warp0([&](auto& w) { RldltPivotOrder(w, N, sd, at); });
+  const Divider by_N(N);
+  t.par(N * N, [&](int e) {
+    const int c = by_N.quot(e), r = e - c * N;
+    if (r >= c) {
+      const int i = at[r], j = at[c];
+      L[(long)c * ldl + r] = (i >= j) ? K[(long)j * ldk + i] : K[(long)i * ldk + j];
+    }
+  });
+  t.par(N, [&](int i) { perm[i] = at[i]; });
+  return BlockedFactor<true>(t, N, L, ldl, signs, sm, update);
+}
+
 }  // namespace small
 }  // namespace cxb

@@ -394,6 +394,113 @@ __global__ void __launch_bounds__(kThreads) LdltSolveKernel(int batch, long per,
                         base + 64);
 }
 
+// ---- KKT systems larger than shared memory: small::BlockedPotrf / BlockedLdlt, one CTA of kThreads per program ----
+// The trailing update A22 -= L21 S L21^T of a block column on the FP64 tensor cores: the lower 32 x 32 tiles of A22
+// go round the warps; per tile the warp stages its two operand panels (kb <= 32 columns each) in its own shared
+// memory, -L21 rows of the tile's row block and S L21 rows of its column block, k-major with a pitch of 4 (mod 16)
+// so that the fragment loads are conflict free, and accumulates on top of the tile read from global memory.
+constexpr int kKktTile = small::kKktNb;
+constexpr int kKktOpPitch = 36;
+constexpr long kKktStageDoubles = 2L * kKktTile * kKktOpPitch;  // per warp
+struct KktTrailingUpdateMma {
+  double* stage;  // kThreads / 32 * kKktStageDoubles doubles of shared memory
+  __device__ void operator()(DeviceTeam& t, double* A, long ld, int k0, int kb, int t0, int R, const double* s) const {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+    const int gid = lane >> 2, tig = lane & 3;
+    double* sa = stage + warp * kKktStageDoubles;  // sa[k * pitch + r] = -L21(r0 + r, k)
+    double* sb = sa + kKktTile * kKktOpPitch;      // sb[k * pitch + c] = s_k L21(c0 + c, k)
+    const int nt = (R + kKktTile - 1) / kKktTile;
+    const int k4 = (kb + 3) & ~3;
+    const double* L21 = A + (long)k0 * ld + t0;
+    double* A22 = A + (long)t0 * ld + t0;
+    for (int w = warp; w < nt * (nt + 1) / 2; w += nwarps) {
+      int ti = (int)((sqrt(8.0 * w + 1.0) - 1.0) * 0.5);  // row-major order of the lower tiles: w -> (ti >= tj)
+      while ((ti + 1) * (ti + 2) / 2 <= w) ti++;
+      while (ti * (ti + 1) / 2 > w) ti--;
+      const int tj = w - ti * (ti + 1) / 2;
+      const int r0 = ti * kKktTile, c0 = tj * kKktTile;
+      for (int e = lane; e < k4 * kKktTile; e += 32) {
+        const int k = e / kKktTile, r = e % kKktTile;
+        const bool in = k < kb;
+        sa[k * kKktOpPitch + r] = (in && r0 + r < R) ? -L21[(long)k * ld + r0 + r] : 0.0;
+        sb[k * kKktOpPitch + r] = (in && c0 + r < R) ? s[k] * L21[(long)k * ld + c0 + r] : 0.0;
+      }
+      __syncwarp();
+      // acc[x][y] = A22(r0 + 8 x + gid, c0 + 8 y + 2 tig + {0, 1}); entries outside A22 stay zero, entries above its
+      // diagonal (diagonal tiles) are not read
+      double acc[4][4][2];
+#pragma unroll
+      for (int x = 0; x < 4; x++)
+#pragma unroll
+        for (int y = 0; y < 4; y++)
+#pragma unroll
+          for (int h = 0; h < 2; h++) {
+            const int r = r0 + 8 * x + gid, c = c0 + 8 * y + 2 * tig + h;
+            acc[x][y][h] = (r < R && c <= r) ? A22[(long)c * ld + r] : 0.0;
+          }
+      const bool diag = ti == tj;
+      for (int k = 0; k < k4; k += 4) {
+        double a[4], b[4];
+#pragma unroll
+        for (int x = 0; x < 4; x++) a[x] = sa[(k + tig) * kKktOpPitch + 8 * x + gid];
+#pragma unroll
+        for (int y = 0; y < 4; y++) b[y] = sb[(k + tig) * kKktOpPitch + 8 * y + gid];
+#pragma unroll
+        for (int x = 0; x < 4; x++)
+#pragma unroll
+          for (int y = 0; y < 4; y++)
+            if (!diag || y <= x) Dmma884(acc[x][y][0], acc[x][y][1], a[x], b[y]);
+      }
+#pragma unroll
+      for (int x = 0; x < 4; x++)
+#pragma unroll
+        for (int y = 0; y < 4; y++)
+#pragma unroll
+          for (int h = 0; h < 2; h++) {
+            const int r = r0 + 8 * x + gid, c = c0 + 8 * y + 2 * tig + h;
+            if (r < R && c <= r) A22[(long)c * ld + r] = acc[x][y][h];
+          }
+      __syncwarp();  // the next tile's staging overwrites sa / sb
+    }
+    __syncthreads();  // the next block column reads the updated trailing matrix
+  }
+};
+
+// Dynamic shared memory (doubles) of the blocked kernels: reduction scratch, the diagonal block, the warps' operand
+// stages and (LDL^T) the pivot order, N doubles and N ints.
+__host__ __device__ inline long BlockedKktSmemDoubles(int N, bool ldlt) {
+  return 64 + small::BlockedKktSmemDoubles() + (kThreads / 32) * kKktStageDoubles + (ldlt ? N + (N + 1) / 2 : 0);
+}
+
+__global__ void __launch_bounds__(kThreads) BlockedPotrfKernel(int N, double* H, long ldh, long hstride, int* info,
+                                                               const int* active) {
+  extern __shared__ double sm[];
+  const int p = blockIdx.x;
+  if (active && !active[p]) return;
+  DeviceTeam t(sm);
+  double* scratch = sm + 64;
+  const KktTrailingUpdateMma update{scratch + small::BlockedKktSmemDoubles()};
+  const int failed = small::BlockedPotrf(t, N, H + p * hstride, ldh, scratch, update);
+  t.single([&]() { info[p] = failed; });
+}
+
+__global__ void __launch_bounds__(kThreads) BlockedLdltKernel(int N, const double* K, long ldk, long kstride, double* L,
+                                                              long ldl, long lstride, int* perm, long pstride,
+                                                              double* signs, long sstride, int* info,
+                                                              const int* active) {
+  extern __shared__ double sm[];
+  const int p = blockIdx.x;
+  if (active && !active[p]) return;
+  DeviceTeam t(sm);
+  double* scratch = sm + 64;
+  double* stage = scratch + small::BlockedKktSmemDoubles();
+  double* sd = stage + (kThreads / 32) * kKktStageDoubles;
+  const KktTrailingUpdateMma update{stage};
+  const int regularised = small::BlockedLdlt(t, N, K + p * kstride, ldk, L + p * lstride, ldl, perm + p * pstride,
+                                             signs + p * sstride, scratch, sd, reinterpret_cast<int*>(sd + N), update);
+  t.single([&]() { info[p] = regularised; });
+}
+
 // The y slices of the subset cones of a batch (cxb_small_gather): one CTA per program.
 __global__ void __launch_bounds__(kThreads) GatherKernel(int count, const int* __restrict__ idx, double* y,
                                                          long ystride, long dst, const int* active) {
@@ -478,9 +585,11 @@ __global__ void __launch_bounds__(kThreads) BatchedDotKernel(int n, const double
   if (threadIdx.x == 0) out[p * ostride] = s;
 }
 
+constexpr size_t kMaxSmemBytes = 227 * 1024;  // dynamic shared memory of one CTA on sm_100
+
 template <typename K>
 int EnsureSmem(K kernel, size_t bytes) {
-  if (bytes > 227 * 1024) return -1;
+  if (bytes > kMaxSmemBytes) return -1;
   if (bytes > 48 * 1024) {
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
     if (e != cudaSuccess) return (int)e;
@@ -854,10 +963,22 @@ int cxb_small_take_step_multi(void* stream, int batch, int ncones, const cxb_sma
   return 0;
 }
 
+int cxb_small_potrf_blocked(void* stream, int batch, int N, double* dH, long ldh, long hstride, int* d_info,
+                            const int* d_active) {
+  if (batch <= 0 || N <= 0) return 0;
+  const size_t smem = sizeof(double) * BlockedKktSmemDoubles(N, false);
+  int rc = EnsureSmem(BlockedPotrfKernel, smem);
+  if (rc) return rc;
+  CountLaunch();
+  BlockedPotrfKernel<<<batch, kThreads, smem, AsStream(stream)>>>(N, dH, ldh, hstride, d_info, d_active);
+  return LaunchStatus();
+}
+
 int cxb_small_potrf(void* stream, int batch, int N, double* dH, long ldh, long hstride, int* d_info,
                     const int* d_active) {
   if (batch <= 0 || N <= 0) return 0;
   const Geometry g = MakeGeometry(batch, sizeof(double) * (64 + (size_t)N * N));
+  if (g.smem > kMaxSmemBytes) return cxb_small_potrf_blocked(stream, batch, N, dH, ldh, hstride, d_info, d_active);
   if (g.warp) {
     int rc = EnsureSmem(PotrfKernel<true>, g.smem);
     if (rc) return rc;
@@ -890,11 +1011,27 @@ int cxb_small_potrs(void* stream, int batch, int N, const double* dL, long ldl, 
   return LaunchStatus();
 }
 
+int cxb_small_ldlt_blocked(void* stream, int batch, int N, const double* dK, long ldk, long kstride, double* dL,
+                           long ldl, long lstride, int* d_perm, long pstride, double* d_signs, long sstride,
+                           int* d_info, const int* d_active) {
+  if (batch <= 0 || N <= 0) return 0;
+  const size_t smem = sizeof(double) * BlockedKktSmemDoubles(N, true);
+  int rc = EnsureSmem(BlockedLdltKernel, smem);
+  if (rc) return rc;
+  CountLaunch();
+  BlockedLdltKernel<<<batch, kThreads, smem, AsStream(stream)>>>(N, dK, ldk, kstride, dL, ldl, lstride, d_perm, pstride,
+                                                                d_signs, sstride, d_info, d_active);
+  return LaunchStatus();
+}
+
 int cxb_small_ldlt(void* stream, int batch, int N, const double* dK, long ldk, long kstride, double* dL, long ldl,
                    long lstride, int* d_perm, long pstride, double* d_signs, long sstride, int* d_info,
                    const int* d_active) {
   if (batch <= 0 || N <= 0) return 0;
   const Geometry g = MakeGeometry(batch, sizeof(double) * (64 + (size_t)LdltSmemDoubles(N)));
+  if (g.smem > kMaxSmemBytes)
+    return cxb_small_ldlt_blocked(stream, batch, N, dK, ldk, kstride, dL, ldl, lstride, d_perm, pstride, d_signs,
+                                  sstride, d_info, d_active);
   if (g.warp) {
     int rc = EnsureSmem(LdltKernel<true>, g.smem);
     if (rc) return rc;

@@ -158,7 +158,8 @@ def mpc_problem(seed, stages=8, stage_vars=6, lp_rows=12, soc_order=6, lmi_order
     """A program shaped like a model-predictive-control horizon: `stages` stages of `stage_vars` variables
     (m = stages * stage_vars). Per stage, an LP block of `lp_rows` rows (A uniform, c = 1) and a Lorentz cone of
     order `soc_order` (A uniform, c = e_0) on the stage's variables; per pair of adjacent stages, a dense LMI of order
-    `lmi_order` (A_i = sym(U[-1,1]), C = I) and an equality block of `eq_rows` rows on the two stages' variables.
+    `lmi_order` (A_i = sym(U[-1,1]), C = I) and an equality block of `eq_rows` rows on the two stages' variables
+    (none with eq_rows = 0; the equality blocks are drawn last, so the cones do not depend on eq_rows).
     Constraint order: stage s's LP and SOC, then (s > 0) the LMI and the equality block coupling s - 1 and s.
     Strictly feasible by construction, like small_multicone_equality_problem: b = sum over cones of AW/2 at W = I plus
     A_eq^T lambda0, and b_eq = A_eq y0[variables] for a y0 at which every cone slack is interior.
@@ -202,7 +203,8 @@ def mpc_problem(seed, stages=8, stage_vars=6, lp_rows=12, soc_order=6, lmi_order
 
     while margin(y0) <= 0.1:
         y0 *= 0.5
-    for position, w in reversed(couplings):  # after each LMI; reversed: earlier positions stay valid
+    # after each LMI; reversed: earlier positions stay valid
+    for position, w in reversed(couplings if eq_rows > 0 else []):
         A_eq = rng.uniform(-1.0, 1.0, size=(eq_rows, len(w)))
         lam0 = rng.uniform(-1.0, 1.0, size=eq_rows)
         np.add.at(b, w, A_eq.T @ lam0)

@@ -212,7 +212,10 @@ void CONEXB200_RldltPivotOrder(int n, const double* diag, int* perm);
  * started from the iterate of the batch's previous solve (-1 when there was none). With equality
  * blocks the KKT systems are factored by a batched regularised LDL^T; iterative_refinement_iterations
  * > 0 is then refused (-1), as is enable_line_search when every constraint is an LP cone or an
- * equality block. */
+ * equality block. The KKT order N (variables + multipliers) has no limit of its own: up to N = 170
+ * (Cholesky) / 169 (LDL^T) a program's KKT matrix is factored in shared memory, above that by blocked
+ * kernels, as long as the batch's 2 N^2 doubles per program (with multipliers, 1 N^2 without) fit in
+ * device memory. LMI cones keep their own limits (order <= 64), which BatchMaximize refuses (-1). */
 void* CONEXB200_CreateBatch(void* const* programs, int count);
 void CONEXB200_DeleteBatch(void* batch);
 int CONEXB200_BatchMaximize(void* batch, const double* b, const CONEX_SolverConfiguration* config, double* y,

@@ -17,7 +17,9 @@
 // Their rows of the KKT matrices and of AQc / AW are constant and written once per batch; the cones'
 // Schur kernels assign only the leading m x m block. A batch with multipliers factors its KKT systems
 // with the batched regularised LDL^T (cxb_small_ldlt, never fails), one without keeps the batched
-// Cholesky — the input decides, as in kkt_solver.cc:172-199.
+// Cholesky — the input decides, as in kkt_solver.cc:172-199. Both take any KKT order N: the device
+// layer factors a program's matrix in shared memory while it fits (N <= 170 / 169) and with blocked
+// kernels above that, so long horizons batch like short ones.
 //
 // A batch lives across many solves. Maximize with initialization_mode = warm start continues every
 // program from the iterate of the previous solve (cone states, including the dual-recovery update,

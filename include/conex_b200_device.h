@@ -369,9 +369,17 @@ int cxb_small_scatter_schur(void* stream, int batch, int ncones, const int* d_co
                             long sstride, int m, double* dH, long ldh, long hstride, double* dAW, double* dAQc,
                             long vstride, double* d_scal, long scal_stride, int accumulate, const int* d_active);
 /* Cholesky of `batch` N x N matrices (lower, ld, stride) and solves with nrhs = 1; d_info[p] = 0 or
- * 1 + first non-positive pivot (block_triangular_operations.cc:184-219, :114-182). */
+ * 1 + first column whose pivot is not > 0, in column order (a NaN pivot fails too; block_triangular_operations.cc:
+ * 184-219, :114-182). After a failure the contents of that program's H are unspecified. d_active[p] == 0 masks
+ * programs that must not be touched. Any N whose matrices fit in device memory: up to N = 170 the whole matrix of a
+ * program is factored in shared memory; above that cxb_small_potrf_blocked is used. */
 int cxb_small_potrf(void* stream, int batch, int N, double* dH, long ldh, long hstride, int* d_info,
                     const int* d_active);
+/* The same contract at any N, blocked: block columns of 32, the diagonal block in shared memory, the trailing update
+ * on the FP64 tensor cores, the matrix factored in place in global memory; shared memory per program does not
+ * depend on N. Not bitwise equal to the shared-memory kernel (the summation order differs). */
+int cxb_small_potrf_blocked(void* stream, int batch, int N, double* dH, long ldh, long hstride, int* d_info,
+                            const int* d_active);
 int cxb_small_potrs(void* stream, int batch, int N, const double* dL, long ldl, long lstride, double* dX,
                     long xstride, const int* d_active);
 /* Regularised LDL^T of `batch` symmetric indefinite N x N matrices (KKT systems with equality multipliers; the
@@ -380,11 +388,17 @@ int cxb_small_potrs(void* stream, int batch, int N, const double* dL, long ldl, 
  * permuted copy P K P^T gathered from the lower triangle of K, and its factorisation L S L^T, S = diag(+-1), with
  * |D|^{1/2} folded into L. Pivots with |d| <= 1e-9 become -1e-9 when d < 0, +1e-9 otherwise; d_info[p] = 1 then,
  * else 0 — it never fails. K is not modified; the lower triangle of L (ldl, lstride), d_perm (ints, perm[i] =
- * original index at pivot position i) and d_signs (S) are written. Shared memory: N^2 + O(N) doubles per program;
- * returns an error code when that does not fit. */
+ * original index at pivot position i) and d_signs (S) are written. d_active[p] == 0 masks programs that must not be
+ * touched. Any N whose matrices fit in device memory: up to N = 169 the permuted copy (N^2 + O(N) doubles) is
+ * factored in shared memory; above that cxb_small_ldlt_blocked is used. */
 int cxb_small_ldlt(void* stream, int batch, int N, const double* dK, long ldk, long kstride, double* dL, long ldl,
                    long lstride, int* d_perm, long pstride, double* d_signs, long sstride, int* d_info,
                    const int* d_active);
+/* The same contract at any N, blocked like cxb_small_potrf_blocked: P K P^T is gathered straight into L, which is
+ * then factored in place; shared memory per program: a fixed amount plus the pivot order (N doubles, N ints). */
+int cxb_small_ldlt_blocked(void* stream, int batch, int N, const double* dK, long ldk, long kstride, double* dL,
+                           long ldl, long lstride, int* d_perm, long pstride, double* d_signs, long sstride,
+                           int* d_info, const int* d_active);
 /* x <- P^T L^{-T} S L^{-1} P x with the factors of cxb_small_ldlt, nrhs = 1. */
 int cxb_small_ldlt_solve(void* stream, int batch, int N, const double* dL, long ldl, long lstride, const int* d_perm,
                          long pstride, const double* d_signs, long sstride, double* dX, long xstride,
