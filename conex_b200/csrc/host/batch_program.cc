@@ -6,8 +6,8 @@
 
 #include "../../../include/conex_b200_device.h"
 #include "dense_lmi_constraint.h"
-#include "divergence.h"
 #include "equality_constraint.h"
+#include "newton_control.h"
 #include "small_cone_constraint.h"
 
 namespace conex {
@@ -443,11 +443,7 @@ void BatchProgram::GetDualVariable(int p, int cone, double* host_out) {
   const int sz = DualVariableSize(cone);
   d.ctx.Download(host_out, c.state.get() + c.state_size * p, sz);
   const BatchResult& r = results_.at(p);
-  if (!r.primal_infeasible && r.num_iterations > 0) {
-    // reference cone_program.h:120-134: W / (sqrt_inv_mu[last] * b_scaling)
-    const double scale = r.inv_sqrt_mu * r.b_scaling;
-    for (int j = 0; j < sz; j++) host_out[j] /= scale;
-  }
+  ScaleDualVariable(r.num_iterations, r.primal_infeasible, r.inv_sqrt_mu, r.b_scaling, host_out, sz);
 }
 
 bool BatchProgram::ConstraintDataShape(int constraint, int* rows, int* columns) const {
@@ -497,21 +493,6 @@ void BatchProgram::UpdateConstraintData(int constraint, int first, int count, co
   d.ctx.Synchronize();  // data is pageable
 }
 
-namespace {
-
-// Host state of one program of the batch: the locals of Solve() (reference cone_program.cc:276-309).
-struct ProgramState {
-  double k = 0, kmax = 0, cx = 1, by = -1, kkt_error = 0;
-  double b_scaling = 1, c_scaling = 1, b_norm = 0, d_inf = 0;
-  int centering_steps = 0, num_iter = 0;
-  bool active = true, failed = false, max_iters_reached = true;
-  bool initial_centering = false, final_centering = false, update_mu = false;
-  bool warmstart_aborted = false;
-  bool restarted = false;  // this iteration: the warm start failed to factor, the cones were reset, nothing else runs
-};
-
-}  // namespace
-
 int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, double* y_out) {
   Impl& d = *impl_;
   const int B = batch_, m = m_, N = d.N;
@@ -541,25 +522,16 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
   }
   void* s = d.s();
   cudaStream_t cs = d.ctx.cuda_stream();
-  std::vector<ProgramState> st(B);
+  std::vector<NewtonControl> st;
   results_.assign(B, BatchResult());
   step_ms_.clear();
 
   // ---- cost vectors; a cold start resets the scalings and the cones (cone_program.cc:350-354) ------------
   for (int p = 0; p < B; p++) {
-    double nrm = 0;
-    for (int i = 0; i < m; i++) {
-      const double v = b_in[static_cast<size_t>(p) * m + i];
-      d.hcoef[p * vs + i] = v;
-      nrm += v * v;
-    }
+    const double* bp = b_in + static_cast<size_t>(p) * m;
+    for (int i = 0; i < m; i++) d.hcoef[p * vs + i] = bp[i];
     for (size_t i = m; i < vs; i++) d.hcoef[p * vs + i] = 0;
-    st[p].b_norm = std::sqrt(nrm);
-    st[p].kmax = cfg.inv_sqrt_mu_max;
-    if (warm) {
-      st[p].b_scaling = d.b_scaling[p];
-      st[p].c_scaling = d.c_scaling[p];
-    }
+    st.emplace_back(cfg, d.rank, bp, m, warm ? d.b_scaling[p] : 1.0, warm ? d.c_scaling[p] : 1.0);
   }
   CudaCheck(cudaMemcpyAsync(d.b.get(), d.hcoef.get(), sizeof(double) * vs * B, cudaMemcpyHostToDevice, cs),
             "H2D cost vectors");
@@ -570,8 +542,6 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
     DeviceCheck(cxb_small_set_identity_multi(s, B, ncones, d.descs.data(), nullptr), "cxb_small_set_identity_multi");
     d.initialised = true;
   }
-  const int initial_centering_steps =
-      warm ? cfg.initial_centering_steps_warmstart : cfg.initial_centering_steps_coldstart;
   cudaEvent_t ev_begin, ev_end, ev_a, ev_b;
   CudaCheck(cudaEventCreate(&ev_begin), "cudaEventCreate");
   CudaCheck(cudaEventCreate(&ev_end), "cudaEventCreate");
@@ -590,28 +560,15 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
   double* cone_out = d.out.get();                                   // B x nc x 4
   double* dots = d.out.get() + static_cast<size_t>(B) * 4 * nc;     // B x 4
   const long ostride = static_cast<long>(4 * nc);
-  const int rank = d.rank;
 
   for (int i = 0; i < cfg.max_iterations; i++) {
     // ---- loop control of every program (reference cone_program.cc:312-336) -----------------------
     int nactive = 0;
+    bool new_scalings = false;
     for (int p = 0; p < B; p++) {
-      ProgramState& q = st[p];
-      d.hmask[p] = 0;
-      if (!q.active) continue;
-      q.restarted = false;
-      q.initial_centering = i < initial_centering_steps;
-      q.final_centering = (q.k >= q.kmax) || (q.kkt_error > cfg.kkt_error_tolerance) ||
-                          (i >= cfg.max_iterations - cfg.final_centering_steps);
-      q.update_mu = (i == 0) || !(q.initial_centering || q.final_centering) || q.warmstart_aborted;
-      q.warmstart_aborted = false;
-      if (q.final_centering && q.centering_steps >= cfg.final_centering_steps) {
-        q.max_iters_reached = (i >= cfg.max_iterations - 1);
-        q.active = false;
-        continue;
-      }
-      d.hmask[p] = 1;
-      nactive++;
+      d.hmask[p] = st[p].Begin(i);
+      nactive += d.hmask[p];
+      new_scalings = new_scalings || (d.hmask[p] && st[p].NeedsAqcNorm());
     }
     if (nactive == 0) break;
     d.UploadMask(0);
@@ -619,9 +576,6 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
 
     // ---- assemble, (rescale,) factor ---------------------------------------------------------------
     d.Assemble(active);
-    const bool rescale = (i == 0) && cfg.enable_rescaling;
-    // a warm start keeps the scalings of the previous solve and only rescales kmax with them (NewtonDriver::Run)
-    const bool new_scalings = rescale && !warm;
     if (new_scalings) {
       DeviceCheck(cxb_batched_dot(s, B, N, d.AQc.get(), vs, d.AQc.get(), vs, dots, 4), "cxb_batched_dot");
     }
@@ -638,37 +592,21 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
     bool any_mu = false;
     bool any_restart = false;
     for (int p = 0; p < B; p++) {
-      ProgramState& q = st[p];
+      NewtonControl& q = st[p];
       d.hmask[B + p] = 0;
       d.hmask[2 * static_cast<size_t>(B) + p] = 0;
-      if (!q.active) continue;
-      if (rescale) {
-        // reference cone_program.cc:343-357
-        if (new_scalings) {
-          q.b_scaling = 1.0 / (1 + q.b_norm);
-          q.c_scaling = 1.0 / (1 + std::sqrt(d.hout[4 * p]));
-        }
-        const double mu_target = (1.0 / (q.kmax * q.kmax)) * (q.b_scaling * q.c_scaling);
-        q.kmax = 1.0 / std::sqrt(mu_target);
-      }
+      if (!q.stepping()) continue;
+      q.Rescale(new_scalings ? d.hout[4 * p] : 0.0);
       if (!d.multipliers && d.hinfo[p] != 0) {
         d.hmask[p] = 0;
         mask_changed = true;
-        if (i == 0 && warm) {
-          // the warm start is abandoned: restart from the identity and skip the rest of this iteration, as
-          // NewtonDriver::Run does for one program
-          q.restarted = true;
-          q.warmstart_aborted = true;
+        if (q.RestartOnFactorizationFailure()) {
           d.hmask[2 * static_cast<size_t>(B) + p] = 1;
           any_restart = true;
-          continue;
         }
-        // Factor() failed: the solve returns unsolved (cone_program.cc:360-371)
-        q.active = false;
-        q.failed = true;
         continue;
       }
-      if (q.update_mu) {
+      if (q.update_mu()) {
         d.hmask[B + p] = 1;
         any_mu = true;
       }
@@ -684,9 +622,9 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
     if (any_mu) {
       d.UploadMask(B);
       for (int p = 0; p < B; p++) {
-        d.hcoef[p] = st[p].c_scaling;
-        d.hcoef[B + p] = -st[p].b_scaling;
-        d.hcoef[3 * static_cast<size_t>(B) + p] = st[p].c_scaling;
+        d.hcoef[p] = st[p].c_scaling();
+        d.hcoef[B + p] = -st[p].b_scaling();
+        d.hcoef[3 * static_cast<size_t>(B) + p] = st[p].c_scaling();
       }
       d.UploadCoef(0, 2 * static_cast<size_t>(B));
       d.UploadCoef(3 * static_cast<size_t>(B), B);
@@ -699,48 +637,20 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
                                         mu_mask),
                   "cxb_small_eigen_multi");
       d.DownloadOut(static_cast<size_t>(B) * 4 * nc);
-      for (int p = 0; p < B; p++) {
-        ProgramState& q = st[p];
-        if (!d.hmask[B + p]) continue;
-        WeightedSlackEigenvalues w;
-        w.frobenius_norm_squared = 0;
-        w.trace = 0;
-        w.lambda_max = -30000;
-        w.lambda_min = 30000;
-        for (size_t k = 0; k < nc; k++) {
-          const double* o = d.hout.get() + (static_cast<size_t>(p) * nc + k) * 4;
-          w.lambda_min = std::min(w.lambda_min, o[0]);
-          w.lambda_max = std::max(w.lambda_max, o[1]);
-          w.frobenius_norm_squared += o[2];
-          w.trace += o[3];
-        }
-        w.rank = rank;
-        double cand = -1;
-        if (cfg.enable_line_search) cand = q.k;  // see NewtonDriver::Run
-        if (cand < 0) {
-          cand = DivergenceUpperBoundInverse(cfg.divergence_upper_bound * rank, w);
-          if (cand == -1) cand = (w.lambda_min > 0) ? 2.0 / (w.lambda_min + w.lambda_max) : -1;
-          if (cand < 0 && w.trace > 1e-12) {
-            const double kstar = w.trace / w.frobenius_norm_squared;
-            double norm_bound = 1.5 * (w.frobenius_norm_squared * kstar * kstar - 2 * w.trace * kstar + rank);
-            norm_bound = std::min(norm_bound, rank * .7);
-            const double qa = w.frobenius_norm_squared, qb = -2 * w.trace, qc = rank - norm_bound;
-            const double disc = qb * qb - 4 * qa * qc;
-            cand = (disc < 0) ? kstar : (-qb + std::sqrt(disc)) / (2 * qa);
-          }
-        }
-        q.k = (cand > 0) ? cand : 0.5 * q.k;
-      }
     }
     for (int p = 0; p < B; p++) {
-      ProgramState& q = st[p];
-      if (!q.active || q.restarted) continue;
-      if (!q.update_mu && !q.initial_centering) q.centering_steps++;
-      q.k = std::max(std::min(q.k, q.kmax), std::sqrt(1.0 / (1e-15 + cfg.maximum_mu)));
-      d.hcoef[p] = q.k * q.b_scaling;
-      d.hcoef[B + p] = q.k * q.c_scaling;
+      NewtonControl& q = st[p];
+      if (!q.stepping()) continue;
+      SlackEigenvalueSum w;
+      for (size_t k = 0; k < nc && q.NeedsEigenvalues(); k++) {
+        const double* o = d.hout.get() + (static_cast<size_t>(p) * nc + k) * 4;
+        w.Add(o[0], o[1], o[2], o[3]);
+      }
+      q.ChooseK(w);
+      d.hcoef[p] = q.k() * q.b_scaling();
+      d.hcoef[B + p] = q.k() * q.c_scaling();
       d.hcoef[2 * static_cast<size_t>(B) + p] = -2.0;
-      d.hcoef[3 * static_cast<size_t>(B) + p] = q.k * q.c_scaling;
+      d.hcoef[3 * static_cast<size_t>(B) + p] = q.k() * q.c_scaling();
     }
 
     // ---- Newton direction: y = H^{-1} (k (b b_s + AQc c_s) - 2 AW) (cone_program.cc:409-414) ------
@@ -754,26 +664,19 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
                                         ostride, active),
                 "cxb_small_prepare_multi");
     d.DownloadOut(static_cast<size_t>(B) * 4 * nc);
-    std::vector<double> normsq(B, 0.0);
     bool any_abort = false;
     for (int p = 0; p < B; p++) {
-      ProgramState& q = st[p];
+      NewtonControl& q = st[p];
       d.hcoef[4 * static_cast<size_t>(B) + p] = 1.0;
       d.hmask[2 * static_cast<size_t>(B) + p] = 0;
-      if (!q.active || q.restarted) continue;
+      if (!q.stepping()) continue;
       double ninf = -1, nsq = 0;
       for (size_t k = 0; k < nc; k++) {
         const double* o = d.hout.get() + (static_cast<size_t>(p) * nc + k) * 4;
         ninf = std::max(ninf, o[0]);
         nsq += o[1];
       }
-      q.d_inf = std::fabs(ninf);
-      normsq[p] = nsq;
-      d.hcoef[4 * static_cast<size_t>(B) + p] = std::min(1.0, 2.0 / (ninf * ninf));
-      if (i == 0 && warm && ninf >= cfg.warmstart_abort_threshold) {
-        // too large a first step from the warm iterate: restart from the identity instead of taking it; the
-        // iteration is completed and logged (NewtonDriver::Run)
-        q.warmstart_aborted = true;
+      if (!q.Step(ninf, nsq, &d.hcoef[4 * static_cast<size_t>(B) + p])) {
         d.hmask[p] = 0;
         d.hmask[2 * static_cast<size_t>(B) + p] = 1;
         any_abort = true;
@@ -801,22 +704,9 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
     cudaEventElapsedTime(&ms, ev_a, ev_b);
     step_ms_.push_back(ms);
     for (int p = 0; p < B; p++) {
-      ProgramState& q = st[p];
-      if (!q.active || q.restarted) continue;
-      const double by_dot = d.hout[4 * p + 0], aqc_dot = d.hout[4 * p + 1];
-      const double wc = d.hout[4 * static_cast<size_t>(B) + 2 * p], cqc = d.hout[4 * static_cast<size_t>(B) + 2 * p + 1];
-      const double k = q.k;
-      const double d_2 = std::sqrt(std::fabs(normsq[p]));
-      q.by = by_dot / (k * q.c_scaling);
-      q.cx = (2 * wc + aqc_dot - k * cqc * q.c_scaling) / (k * q.b_scaling);
-      const double mu = (1.0 / k) * (1.0 / k);
-      const double s_dot_x = mu * (rank - d_2 * d_2) / (q.b_scaling * q.c_scaling);
-      q.kkt_error = std::fabs(q.cx - q.by - s_dot_x) / s_dot_x;
-      q.num_iter = i + 1;
-      if ((q.final_centering || k >= q.kmax) && q.d_inf <= cfg.final_centering_tolerance) {
-        q.max_iters_reached = false;
-        q.active = false;
-      }
+      if (!st[p].stepping()) continue;
+      const double* sc = d.hout.get() + 4 * static_cast<size_t>(B) + 2 * p;
+      st[p].End(d.hout[4 * p + 0], d.hout[4 * p + 1], sc[0], sc[1]);
     }
   }
 
@@ -826,37 +716,20 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
   int solved_count = 0;
   bool any_recover = false;
   for (int p = 0; p < B; p++) {
-    ProgramState& q = st[p];
+    const NewtonControl& q = st[p];
     BatchResult& r = results_[p];
-    r.num_iterations = q.num_iter;
-    r.by = q.by;
-    r.cx = q.cx;
-    r.inv_sqrt_mu = q.k;
-    r.b_scaling = d.b_scaling[p] = q.b_scaling;
-    r.c_scaling = d.c_scaling[p] = q.c_scaling;
-    r.d_inf = q.d_inf;
+    r.by = q.by();
+    r.cx = q.cx();
+    r.inv_sqrt_mu = q.k();
+    r.b_scaling = d.b_scaling[p] = q.b_scaling();
+    r.c_scaling = d.c_scaling[p] = q.c_scaling();
+    r.d_inf = q.d_inf();
     double* yp = y_out + static_cast<size_t>(p) * m;
     for (int j = 0; j < m; j++) yp[j] = d.hout[p * ys + j];
-    d.hmask[p] = 0;
-    if (q.failed) {
-      r.solved = 0;
-      continue;
-    }
-    const double mu_final = (1.0 / q.k) * (1.0 / q.k);
-    if (mu_final > cfg.infeasibility_threshold) {
-      r.solved = 0;
-      r.primal_infeasible = q.cx * q.k <= -.5;
-      r.dual_infeasible = q.by * q.k >= .5;
-    } else {
-      r.solved = 1;
-    }
-    d.hmask[p] = 1;
-    any_recover = true;
-    if (r.solved) {
-      for (int j = 0; j < m; j++) yp[j] = yp[j] / q.k / q.c_scaling;
-      if (q.max_iters_reached) r.solved = 0;
-    }
+    static_cast<ConexStatus&>(r) = q.Finish(yp, m);
     solved_count += r.solved;
+    d.hmask[p] = !q.failed();
+    any_recover = any_recover || !q.failed();
   }
   if (cfg.prepare_dual_variables && any_recover) {
     // reference cone_program.cc:500-516
@@ -864,7 +737,7 @@ int BatchProgram::Maximize(const double* b_in, const SolverConfiguration& cfg, d
     d.Assemble(active);
     d.Factor(active);
     for (int p = 0; p < B; p++) {
-      d.hcoef[p] = st[p].k * st[p].b_scaling;
+      d.hcoef[p] = st[p].k() * st[p].b_scaling();
       d.hcoef[B + p] = -1.0;
     }
     d.UploadCoef(0, 2 * static_cast<size_t>(B));

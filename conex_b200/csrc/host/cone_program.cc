@@ -10,7 +10,7 @@
 
 #include "../../../include/conex_b200_device.h"
 #include "communicator.h"
-#include "divergence.h"
+#include "newton_control.h"
 #include "supernodal_kkt_solver.h"
 
 namespace conex {
@@ -257,10 +257,8 @@ void Program::GetDualVariable(int i, double* host_out) {
     const Ref w = c.constraint.dual_variable();
     const size_t sz = w.size();
     ctx_.Download(host_out, w.data, sz);
-    if (!status_.primal_infeasible && stats.num_iter > 0) {
-      const double scale = stats.sqrt_inv_mu[stats.num_iter - 1] * stats.b_scaling;
-      for (size_t j = 0; j < sz; j++) host_out[j] /= scale;
-    }
+    const double k = stats.num_iter > 0 ? stats.sqrt_inv_mu[stats.num_iter - 1] : 0;
+    ScaleDualVariable(stats.num_iter, status_.primal_infeasible, k, stats.b_scaling, host_out, sz);
     return;
   }
 }
@@ -395,24 +393,8 @@ void PrepareStep(Program& prog, const StepOptions& opt, const Ref& y, StepInfo* 
   }
 }
 
-// reference cone_program.cc:31-57
-void GetWeightedSlackEigenvalues(Program& prog, const Ref& y, double c_weight,
-                                 WeightedSlackEigenvalues* p) {
-  p->frobenius_norm_squared = 0;
-  p->trace = 0;
-  p->lambda_max = -30000;
-  p->lambda_min = 30000;
-  for (auto& c : prog.eqs) {
-    WeightedSlackEigenvalues t;
-    GetWeightedSlackEigenvalues(&c.constraint, GatherVariables(prog, c, y), c_weight, &t);
-    p->lambda_max = std::max(p->lambda_max, t.lambda_max);
-    p->lambda_min = std::min(p->lambda_min, t.lambda_min);
-    p->frobenius_norm_squared += t.frobenius_norm_squared;
-    p->trace += t.trace;
-  }
-}
-
-// State of one solve: the reference keeps these as locals of Solve() (cone_program.cc:276-309).
+// State of one solve besides its NewtonControl: the device vectors of the reference's Solve() locals
+// (cone_program.cc:276-309).
 class NewtonDriver {
  public:
   NewtonDriver(Program& prog, const SolverConfiguration& config)
@@ -422,9 +404,8 @@ class NewtonDriver {
 
  private:
   void UploadCost();
-  double MuFromDivergence();
-  void FormNewtonRightHandSide(double k);
-  void RecoverDualVariables(double k);
+  WeightedSlackEigenvalues MuEigenvalues(const NewtonControl& ctl);
+  void RecoverDualVariables(const NewtonControl& control);
 
   Program& prog_;
   const SolverConfiguration& cfg_;
@@ -434,7 +415,6 @@ class NewtonDriver {
   double* d_y_ = nullptr;  // Newton direction / primal variable
   double* d_y2_ = nullptr;
   std::vector<double> b_;
-  int rank_ = 0;
 };
 
 void NewtonDriver::UploadCost() {
@@ -450,12 +430,10 @@ void NewtonDriver::UploadCost() {
   ctx_.Synchronize();  // b_ is pageable: the copy must have consumed it before we move on
 }
 
-// reference cone_program.cc:166-214
-double NewtonDriver::MuFromDivergence() {
-  auto& st = prog_.stats;
-  void* s = ctx_.stream();
+// The slack eigenvalues the mu rule reads (reference cone_program.cc:31-57, 173-191)
+WeightedSlackEigenvalues NewtonDriver::MuEigenvalues(const NewtonControl& ctl) {
   // y = AQc*c_scaling - b*b_scaling ; y <- H^{-1} y
-  DeviceCheck(cxb_axpbypcz(s, m_, st.c_scaling, prog_.sys.AQc, 0.0, d_y_, -st.b_scaling, d_b_),
+  DeviceCheck(cxb_axpbypcz(ctx_.stream(), m_, ctl.c_scaling(), prog_.sys.AQc, 0.0, d_y_, -ctl.b_scaling(), d_b_),
               "cxb_axpbypcz");
   Ref y(d_y_, m_, 1);
   static const bool trace = std::getenv("CONEX_TRACE_EIGEN") != nullptr;
@@ -467,48 +445,27 @@ double NewtonDriver::MuFromDivergence() {
               << std::chrono::duration<double, std::milli>(std::chrono::high_resolution_clock::now() - t0).count()
               << " ms" << std::endl;
   }
-  WeightedSlackEigenvalues p;
-  GetWeightedSlackEigenvalues(prog_, y, st.c_scaling, &p);
-  p.rank = rank_;
-  double k = DivergenceUpperBoundInverse(cfg_.divergence_upper_bound * rank_, p);
-  if (k == -1) {
-    // maximise the denominator of the bound instead (cone_program.cc:166-172)
-    k = (p.lambda_min > 0) ? 2.0 / (p.lambda_min + p.lambda_max) : -1;
+  SlackEigenvalueSum p;
+  for (auto& c : prog_.eqs) {
+    WeightedSlackEigenvalues t;
+    GetWeightedSlackEigenvalues(&c.constraint, GatherVariables(prog_, c, y), ctl.c_scaling(), &t);
+    p.Add(t.lambda_min, t.lambda_max, t.frobenius_norm_squared, t.trace);
   }
-  if (k < 0 && p.trace > 1e-12) {
-    // last resort: the mu that satisfies a norm bound (cone_program.cc:194-211)
-    const double kstar = p.trace / p.frobenius_norm_squared;
-    double norm_bound = 1.5 * (p.frobenius_norm_squared * kstar * kstar - 2 * p.trace * kstar + rank_);
-    norm_bound = std::min(norm_bound, rank_ * .7);
-    const double qa = p.frobenius_norm_squared, qb = -2 * p.trace, qc = rank_ - norm_bound;
-    const double disc = qb * qb - 4 * qa * qc;
-    k = (disc < 0) ? kstar : (-qb + std::sqrt(disc)) / (2 * qa);
-  }
-  return k;
-}
-
-// y = k (b b_scaling + AQc c_scaling) - 2 AW   (reference cone_program.cc:409-411)
-void NewtonDriver::FormNewtonRightHandSide(double k) {
-  const auto& st = prog_.stats;
-  void* s = ctx_.stream();
-  DeviceCheck(cxb_axpbypcz(s, m_, k * st.b_scaling, d_b_, 0.0, d_y_, k * st.c_scaling, prog_.sys.AQc),
-              "cxb_axpbypcz");
-  DeviceCheck(cxb_axpbypcz(s, m_, -2.0, prog_.sys.AW, 1.0, d_y_, 0.0, nullptr), "cxb_axpbypcz");
+  return p;
 }
 
 // reference cone_program.cc:500-516
-void NewtonDriver::RecoverDualVariables(double k) {
+void NewtonDriver::RecoverDualVariables(const NewtonControl& control) {
   prog_.solver->Assemble();
   AssembleSchurComplementResiduals(prog_);
   prog_.solver->Factor();
-  DeviceCheck(cxb_axpbypcz(ctx_.stream(), m_, k * prog_.stats.b_scaling, d_b_, 0.0, d_y2_, -1.0,
-                           prog_.sys.AW),
+  DeviceCheck(cxb_axpbypcz(ctx_.stream(), m_, control.k() * control.b_scaling(), d_b_, 0.0, d_y2_, -1.0, prog_.sys.AW),
               "cxb_axpbypcz");
   Ref y2(d_y2_, m_, 1);
   prog_.solver->SolveInPlace(&y2);
   StepOptions opt;
   opt.affine = true;
-  opt.inv_sqrt_mu = k;
+  opt.inv_sqrt_mu = control.k();
   opt.e_weight = 0;
   opt.c_weight = 0;
   StepInfo info;
@@ -537,21 +494,9 @@ bool NewtonDriver::Run(double* primal_variable) {
   prog_.solver->SetIterativeRefinementIterations(cfg_.iterative_refinement_iterations);
   prog_.solver->SetSolverMode(cfg_.kkt_solver);
 
-  const bool warm = cfg_.initialization_mode != CONEX_INITIALIZATION_MODE_COLDSTART;
-  const int initial_centering_steps =
-      warm ? cfg_.initial_centering_steps_warmstart : cfg_.initial_centering_steps_coldstart;
-  rank_ = 0;
-  for (auto* c : prog_.constraints_) rank_ += Rank(*c);
-
-  double k = 0;  // inv_sqrt_mu of the current iterate
-  double kmax = cfg_.inv_sqrt_mu_max;
-  double cx = 1, by = -1, kkt_error = 0;
-  int centering_steps = 0;
-  bool warmstart_aborted = false;
-  bool max_iters_reached = true;
-  double b_norm = 0;
-  for (double v : b_) b_norm += v * v;
-  b_norm = std::sqrt(b_norm);
+  int rank = 0;
+  for (auto* c : prog_.constraints_) rank += Rank(*c);
+  NewtonControl control(cfg_, rank, b_.data(), b_.size(), st.b_scaling, st.c_scaling);
 
   // Phase boundaries are CUDA events on the program stream: 0 start | 1 assembled | 2 factored |
   // 3 mu chosen | 4 solved | 5 updated (+ objective dots). Elapsed times are read after the
@@ -568,78 +513,55 @@ bool NewtonDriver::Run(double* primal_variable) {
   auto mark = [&](int i) { CudaCheck(cudaEventRecord(ev.e[i], ctx_.cuda_stream()), "cudaEventRecord"); };
 
   for (int i = 0; i < cfg_.max_iterations; i++) {
-    const bool initial_centering = i < initial_centering_steps;
-    const bool final_centering = (k >= kmax) || (kkt_error > cfg_.kkt_error_tolerance) ||
-                                 (i >= cfg_.max_iterations - cfg_.final_centering_steps);
-    const bool update_mu = (i == 0) || !(initial_centering || final_centering) || warmstart_aborted;
-    warmstart_aborted = false;
-    if (final_centering && centering_steps >= cfg_.final_centering_steps) {
-      max_iters_reached = (i >= cfg_.max_iterations - 1);
-      break;
-    }
+    if (!control.Begin(i)) break;
     mark(0);
     prog_.solver->Assemble();
     AssembleSchurComplementResiduals(prog_);
     mark(1);
-    if (i == 0 && cfg_.enable_rescaling) {
-      if (!warm) {
-        DeviceCheck(cxb_dot(ctx_.stream(), m_, prog_.sys.AQc, prog_.sys.AQc, ctx_.scalars()), "cxb_dot");
-        double aqc2 = 0;
-        ctx_.Download(&aqc2, ctx_.scalars(), 1);
-        st.b_scaling = 1.0 / (1 + b_norm);
-        st.c_scaling = 1.0 / (1 + std::sqrt(aqc2));
-      }
-      // xhat*shat = mu I for the scaled iterates means x*s = mu/(b_scaling*c_scaling): rescale the
-      // target (reference cone_program.cc:349-356).
-      const double mu_target = (1.0 / (kmax * kmax)) * (st.b_scaling * st.c_scaling);
-      kmax = 1.0 / std::sqrt(mu_target);
+    double aqc2 = 0;
+    if (control.NeedsAqcNorm()) {
+      DeviceCheck(cxb_dot(ctx_.stream(), m_, prog_.sys.AQc, prog_.sys.AQc, ctx_.scalars()), "cxb_dot");
+      ctx_.Download(&aqc2, ctx_.scalars(), 1);
     }
+    control.Rescale(aqc2);
+    st.b_scaling = control.b_scaling();
+    st.c_scaling = control.c_scaling();
     if (!prog_.solver->Factor()) {
-      if (i == 0 && warm) {
-        for (auto* c : prog_.constraints_) SetIdentity(c);
-        warmstart_aborted = true;
-        continue;
+      if (!control.RestartOnFactorizationFailure()) {
+        status.solved = 0;
+        return false;
       }
-      status.solved = 0;
-      return false;
+      for (auto* c : prog_.constraints_) SetIdentity(c);
+      continue;
     }
     mark(2);
-    if (update_mu) {
-      double candidate = -1;
-      if (cfg_.enable_line_search) {
-        // PSD / second-order cones provide no PerformLineSearch (reference constraint.h:24-28): the
-        // search fails and the previous value is kept (cone_program.cc:376-384). Programs made of LP
-        // cones only would run the reference's real line search, which is not built here.
-        if (!prog_.LineSearchAlwaysFails()) {
-          throw std::runtime_error("conex-b200: enable_line_search on LP-only programs is not implemented");
-        }
-        candidate = k;
-      }
-      if (candidate < 0) candidate = MuFromDivergence();
-      k = (candidate > 0) ? candidate : 0.5 * k;
-    } else if (!initial_centering) {
-      centering_steps++;
+    if (control.update_mu() && cfg_.enable_line_search && !prog_.LineSearchAlwaysFails()) {
+      // Programs made of LP cones only would run the reference's real line search, which is not built here.
+      throw std::runtime_error("conex-b200: enable_line_search on LP-only programs is not implemented");
     }
-    k = std::max(std::min(k, kmax), std::sqrt(1.0 / (1e-15 + cfg_.maximum_mu)));
+    control.ChooseK(control.NeedsEigenvalues() ? MuEigenvalues(control) : WeightedSlackEigenvalues());
+    const double k = control.k();
     mark(3);
 
+    // y = k (b b_scaling + AQc c_scaling) - 2 AW   (reference cone_program.cc:409-411)
+    DeviceCheck(cxb_axpbypcz(ctx_.stream(), m_, k * control.b_scaling(), d_b_, 0.0, d_y_, k * control.c_scaling(),
+                             prog_.sys.AQc),
+                "cxb_axpbypcz");
+    DeviceCheck(cxb_axpbypcz(ctx_.stream(), m_, -2.0, prog_.sys.AW, 1.0, d_y_, 0.0, nullptr), "cxb_axpbypcz");
     Ref y(d_y_, m_, 1);
-    FormNewtonRightHandSide(k);
     prog_.solver->SolveInPlace(&y);
     mark(4);
     StepOptions opt;
     opt.affine = false;
     opt.inv_sqrt_mu = k;
     opt.e_weight = 1;
-    opt.c_weight = k * st.c_scaling;
+    opt.c_weight = k * control.c_scaling();
     StepInfo info;
     PrepareStep(prog_, opt, y, &info);
-    opt.step_size = std::min(1.0, 2.0 / (info.norminfd * info.norminfd));
-    if (i == 0 && warm && info.norminfd >= cfg_.warmstart_abort_threshold) {
-      for (auto* c : prog_.constraints_) SetIdentity(c);
-      warmstart_aborted = true;
-    } else {
+    if (control.Step(info.norminfd, info.normsqrd, &opt.step_size)) {
       for (auto* c : prog_.constraints_) TakeStep(c, opt);
+    } else {
+      for (auto* c : prog_.constraints_) SetIdentity(c);
     }
     // by, cx need b.y, AQc.y, <w,c>, <c,Qc>: one round trip of four doubles.
     DeviceCheck(cxb_dot(ctx_.stream(), m_, d_b_, d_y_, ctx_.scalars() + 0), "cxb_dot");
@@ -658,47 +580,25 @@ bool NewtonDriver::Run(double* primal_variable) {
     prog_.seconds.solve += 1e-3 * phase_ms[3];
     prog_.seconds.update += 1e-3 * phase_ms[4];
 
-    const double d_2 = std::sqrt(std::fabs(info.normsqrd));
-    const double d_inf = std::fabs(info.norminfd);
-    by = r[0] / (k * st.c_scaling);
-    // k <c,x> = 2 <c,w> + <AQc, y> - k <c,Qc>   (reference cone_program.cc:443-452)
-    cx = (2 * r[2] + r[1] - k * r[3] * st.c_scaling) / (k * st.b_scaling);
-    double mu = (1.0 / k) * (1.0 / k);
-    const double s_dot_x = mu * (rank_ - d_2 * d_2) / (st.b_scaling * st.c_scaling);
-    mu /= (st.c_scaling * st.b_scaling);
-    kkt_error = std::fabs(cx - by - s_dot_x) / s_dot_x;
-    st.num_iter = i + 1;
+    const bool converged = control.End(r[0], r[1], r[2], r[3]);
+    st.num_iter = control.num_iterations();
     st.sqrt_inv_mu[i] = k;
-    prog_.log.push_back({k, mu, d_2, d_inf, by, cx, kkt_error, opt.step_size, ms,
+    prog_.log.push_back({k, control.mu(), control.d_2(), control.d_inf(), control.by(), control.cx(),
+                         control.kkt_error(), opt.step_size, ms,
                          {phase_ms[0], phase_ms[1], phase_ms[2], phase_ms[3], phase_ms[4]},
-                         {2 * r[2], r[1], k * r[3] * st.c_scaling}});
+                         {2 * r[2], r[1], k * r[3] * control.c_scaling()}});
     if (prog_.verbose) {
       std::cout << "i: " << std::setw(2) << i << ", mu: " << std::scientific << std::setprecision(2)
-                << mu << ", d_2: " << d_2 << ", d_inf: " << d_inf << ", by: " << by << ", cx: " << cx
-                << ", kkt_error: " << kkt_error << ", ms: " << std::fixed << ms << std::endl;
+                << control.mu() << ", d_2: " << control.d_2() << ", d_inf: " << control.d_inf()
+                << ", by: " << control.by() << ", cx: " << control.cx() << ", kkt_error: " << control.kkt_error()
+                << ", ms: " << std::fixed << ms << std::endl;
     }
-    if ((final_centering || k >= kmax) && d_inf <= cfg_.final_centering_tolerance) {
-      max_iters_reached = false;
-      break;
-    }
+    if (converged) break;
   }
 
-  status.num_iterations = st.num_iter;
-  const int num_vars = prog_.GetNumberOfVariables();
-  ctx_.Download(primal_variable, d_y_, num_vars);  // yout = y.topRows(m), cone_program.cc:486
-  const double mu_final = (1.0 / k) * (1.0 / k);
-  if (mu_final > cfg_.infeasibility_threshold) {
-    status.solved = 0;
-    status.primal_infeasible = cx * k <= -.5;
-    status.dual_infeasible = by * k >= .5;
-  } else {
-    status.solved = 1;
-  }
-  if (cfg_.prepare_dual_variables) RecoverDualVariables(k);
-  if (status.solved) {
-    for (int j = 0; j < num_vars; j++) primal_variable[j] = primal_variable[j] / k / st.c_scaling;
-    if (max_iters_reached) status.solved = 0;
-  }
+  ctx_.Download(primal_variable, d_y_, prog_.GetNumberOfVariables());  // yout = y.topRows(m), cone_program.cc:486
+  if (cfg_.prepare_dual_variables) RecoverDualVariables(control);
+  status = control.Finish(primal_variable, prog_.GetNumberOfVariables());
   ctx_.Synchronize();
   return status.solved != 0;
 }

@@ -8,9 +8,10 @@
 // phase of the Newton step is ONE launch per cone with one CTA per program (device/small_cones.cu),
 // the B small KKT systems are factored and solved by one launch each, and the per-program control
 // flow of Solve() — centering schedule, mu rule, rescaling, step size, termination, status — runs on
-// the host over arrays of B scalars fetched once per phase. Programs that have terminated are masked
-// out of later launches, so every program follows exactly the iteration sequence it would follow
-// alone.
+// the host over arrays of B scalars fetched once per phase, in one NewtonControl per program
+// (newton_control.h), the class that also drives a single program's solve. Programs that have
+// terminated are masked out of later launches, so every program follows exactly the iteration
+// sequence it would follow alone.
 //
 // Equality constraints (EqualityConstraints blocks, on any subset of the variables) add their
 // multipliers as KKT unknowns m..N-1, in the order the blocks were added (Program::AddConstraint).
@@ -23,7 +24,7 @@
 //
 // A batch lives across many solves. Maximize with initialization_mode = warm start continues every
 // program from the iterate of the previous solve (cone states, including the dual-recovery update,
-// and the b / c scalings), exactly as Program's warm start does for one program: the warm centering
+// and the b / c scalings), with the NewtonControl warm-start logic of a single program: the warm centering
 // schedule, and a restart from the identity for a program whose first factorisation fails or whose
 // first step is too large (warmstart_abort_threshold). UpdateConstraintData replaces columns of a
 // constraint's data in every program on the device, so that the next instance of a parametric
@@ -45,11 +46,7 @@
 
 namespace conex {
 
-struct BatchResult {
-  int solved = 0;
-  int num_iterations = 0;
-  int primal_infeasible = 0;
-  int dual_infeasible = 0;
+struct BatchResult : ConexStatus {
   double by = 0, cx = 0, inv_sqrt_mu = 0;
   double b_scaling = 1, c_scaling = 1, d_inf = 0;
 };
