@@ -42,6 +42,12 @@ int DgemmStructured(cudaStream_t stream, int config, int splits, bool transA, bo
                     bool mirror, int diag_off, GemmStructure structure, bool pack);
 long PackedSymmetricSize(int n);
 
+// ozaki.cu: H (lower, M x N, N <= M) = X^T X for X K x M column-major (K % 16 == 0), FP64 emulated on the 8-bit
+// integer tensor cores; `work` holds GramEmulatedWorkspace(M, K) bytes (the int8 slices of X and its column exponents)
+size_t GramEmulatedWorkspace(int M, long K);
+int GramSlices(cudaStream_t s, int M, long K, const double* X, long ldx, void* work);
+int GramEmulated(cudaStream_t s, int M, int N, long K, const double* X, long ldx, double* H, long ldh, void* work);
+
 // cholesky.cu: factors the block column [j0, j0 + w) x rows [j0, m) in place (w <= 512)
 int PotrfBlockColumn(cudaStream_t s, int m, int j0, int w, double* H, long ldh, int* info);
 

@@ -1,5 +1,5 @@
-// K1 + K2: Schur-complement assembly for one dense LMI block, H_ij = tr(A_i W A_j W), entirely
-// on the FP64 tensor cores.
+// K1 + K2: Schur-complement assembly for one dense LMI block, H_ij = tr(A_i W A_j W), on the tensor
+// cores (FP64, and for the symmetric form's Gram the 8-bit integer ones, see below).
 //
 // Reference (dense_lmi_constraint.cc:62-103): per constraint two n x n x n GEMMs (A_i W, W A_i W)
 // followed by a GEMV against the growing slab Avect[:, 0:i+1] — BLAS-2 and memory bound. Here:
@@ -48,7 +48,8 @@ __global__ void CopyLowerKernel(int n, const double* __restrict__ W, double* L) 
 //       S_i = L^T Y_i + Y_i^T L  symmetric: lower tiles only, both products in one k loop (2 n^3 / 3 flop)
 //           stored as packed 64 x 64 lower tiles with sqrt(2)-scaled off-diagonal tiles, so that the
 //           plain dot product of two packed matrices is their trace inner product (K = 0.54 n^2)
-//   K2  Haug = X^T X (lower)   X = [S_0 .. S_{m-1}, L^T C L, I]: one DMMA SYRK-shaped GEMM
+//   K2  Haug = X^T X (lower)   X = [S_0 .. S_{m-1}, L^T C L, I]: one SYRK-shaped Gram, emulated on the 8-bit integer
+//                              tensor cores (ozaki.cu) at sizes where that pays, one DMMA GEMM below them
 // K1 reads the lower triangle of A_i and C only. Rows m and m+1 of Haug are AQc_j = <L^T C L, S_j> and
 // AW_j = tr(S_j) as before. Executed flops: 1.0 m n^3 + 0.54 m^2 n^2 against 3 m n^3 + m^2 n^2 of the W A_i W form
 // (4 m n^3 + m^2 n^2 dense).
@@ -91,12 +92,39 @@ extern "C" int cxb_schur_dense_lmi_sym_scale(void* stream, int n, int m, const d
   return cxb_pack_symmetric(stream, n, dT, dX + (long)(m + 1) * kp);
 }
 
-extern "C" int cxb_schur_dense_lmi_sym_gram(void* stream, int n, int m, const double* dX, double* dHaug, long ldh) {
+// K2 runs on the 8-bit integer tensor cores (FP64 emulation, ozaki.cu) when there are at least two 128-row tile rows and
+// one full 2^15 K chunk, and on the DMMA Gram otherwise (a handful of CTAs, where slicing X costs as much as the
+// product). _ws: dWork holds cxb_schur_dense_lmi_sym_gram_workspace(n, m) bytes for the slices of X, or is nullptr (the
+// caller could not afford them: DMMA Gram). Without the argument the slices come from the stream-ordered pool for the
+// call, and the DMMA Gram runs if that allocation fails.
+extern "C" size_t cxb_schur_dense_lmi_sym_gram_workspace(int n, int m) {
+  const long kp = cxb::PackedSymmetricSize(n);
+  return (m + 2 >= 256 && kp >= (1L << 15)) ? cxb::GramEmulatedWorkspace(m + 2, kp) : 0;
+}
+
+extern "C" int cxb_schur_dense_lmi_sym_gram_ws(void* stream, int n, int m, const double* dX, double* dHaug, long ldh,
+                                               void* dWork, size_t work_bytes) {
   using namespace cxb;
   if (n < 1 || m < 1 || ldh < m + 2) return -1;
+  cudaStream_t s = AsStream(stream);
   const long kp = PackedSymmetricSize(n);
-  return Dgemm(AsStream(stream), true, false, m + 2, m + 1, (int)kp, 1.0, dX, kp, 0, dX, kp, 0, 0.0, dHaug, ldh, 0, 1,
-               true);
+  const size_t need = cxb_schur_dense_lmi_sym_gram_workspace(n, m);
+  if (need > 0 && dWork != nullptr && work_bytes >= need) {
+    return GramEmulated(s, m + 2, m + 1, kp, dX, kp, dHaug, ldh, dWork);
+  }
+  return Dgemm(s, true, false, m + 2, m + 1, (int)kp, 1.0, dX, kp, 0, dX, kp, 0, 0.0, dHaug, ldh, 0, 1, true);
+}
+
+extern "C" int cxb_schur_dense_lmi_sym_gram(void* stream, int n, int m, const double* dX, double* dHaug, long ldh) {
+  const size_t need = cxb_schur_dense_lmi_sym_gram_workspace(n, m);
+  void* p = nullptr;
+  if (need > 0 && cudaMallocAsync(&p, need, cxb::AsStream(stream)) != cudaSuccess) {
+    cudaGetLastError();
+    p = nullptr;
+  }
+  const int rc = cxb_schur_dense_lmi_sym_gram_ws(stream, n, m, dX, dHaug, ldh, p, need);
+  if (p != nullptr) cudaFreeAsync(p, cxb::AsStream(stream));
+  return rc;
 }
 
 extern "C" int cxb_schur_dense_lmi_sym(void* stream, int n, int m, const double* dAall, const double* dW,

@@ -18,6 +18,7 @@ struct DenseLMIConstraint::Storage {
   DeviceBuffer<double> B;        // n^2 x (m+2): W A_i W, W C W, W        (K1 output / K2 operand)
   DeviceBuffer<double> X;        // symmetric form: packed L^T A_i L, L^T C L, I  ((m+2) x packed size)
   DeviceBuffer<double> Lw;       // symmetric form: Cholesky factor of W
+  DeviceBuffer<unsigned char> slices;  // symmetric form: int8 slices of X for the emulated Gram (empty: DMMA Gram)
   bool symmetric = false;        // assemble through cxb_schur_dense_lmi_sym
   DeviceBuffer<double> T;        // panel scratch for A_i W
   DeviceBuffer<double> scratch;  // Lanczos / Padé / LU work
@@ -349,6 +350,10 @@ void DenseLMIConstraint::EnsureScratch() {
   if (d.symmetric) {
     d.X.Resize(kp * (m_local_ + 2));
     d.Lw.Resize(nn);
+    // K2 on the integer tensor cores needs 8 bytes of slices per packed entry (as much as X); where they do not fit
+    // beside everything else, K2 stays on the DMMA Gram
+    const size_t slice_bytes = cxb_schur_dense_lmi_sym_gram_workspace(n_, m_local_);
+    if (slice_bytes > 0 && sym_bytes + slice_bytes + other <= free_bytes) d.slices.Resize(slice_bytes);
   } else {
     d.B.Resize(d.streamed ? nn * (d.panel + 1) : nn * (m_local_ + 2));
   }
@@ -458,9 +463,12 @@ void ConstructSchurComplementSystem(DenseLMIConstraint* o, bool initialize,
     o->AssembleSharded(sys);
   } else if (d.symmetric) {
     int* flag = o->ctx_->flags() + 4;
-    DeviceCheck(cxb_schur_dense_lmi_sym(s, o->n_, m, d.Aall.get(), o->workspace_.W.data, d.X.get(), d.T.get(),
-                                        d.panel, d.Lw.get(), flag, sys->G.data, sys->G.ld),
-                "cxb_schur_dense_lmi_sym");
+    DeviceCheck(cxb_schur_dense_lmi_sym_scale(s, o->n_, m, d.Aall.get(), o->workspace_.W.data, d.X.get(), d.T.get(),
+                                              d.panel, d.Lw.get(), flag),
+                "cxb_schur_dense_lmi_sym_scale");
+    DeviceCheck(cxb_schur_dense_lmi_sym_gram_ws(s, o->n_, m, d.X.get(), sys->G.data, sys->G.ld, d.slices.get(),
+                                                d.slices.size()),
+                "cxb_schur_dense_lmi_sym_gram_ws");
     int w_not_pd = 0;
     o->ctx_->DownloadInts(&w_not_pd, flag, 1);
     if (w_not_pd != 0) {
@@ -594,8 +602,8 @@ void DenseLMIConstraint::AssembleSharded(SchurComplementSystem* sys) {
                                               d.Lw.get(), flag),
                 "cxb_schur_dense_lmi_sym_scale(local block)");
     release_side_stream();
-    DeviceCheck(cxb_schur_dense_lmi_sym_gram(s, n, ml, d.X.get(), d.Hloc.get(), ldl),
-                "cxb_schur_dense_lmi_sym_gram(local block)");
+    DeviceCheck(cxb_schur_dense_lmi_sym_gram_ws(s, n, ml, d.X.get(), d.Hloc.get(), ldl, d.slices.get(), d.slices.size()),
+                "cxb_schur_dense_lmi_sym_gram_ws(local block)");
   } else {
     DeviceCheck(cxb_schur_dense_lmi(s, n, ml, d.Aall.get(), workspace_.W.data, d.B.get(), d.T.get(),
                                     d.panel, d.Hloc.get(), ldl),

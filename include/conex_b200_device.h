@@ -81,6 +81,22 @@ int cxb_schur_dense_lmi_sym(void* stream, int n, int m, const double* dAall, con
 int cxb_schur_dense_lmi_sym_scale(void* stream, int n, int m, const double* dAall, const double* dW, double* dX,
                                   double* dT, int panel, double* dL, int* d_info);
 int cxb_schur_dense_lmi_sym_gram(void* stream, int n, int m, const double* dX, double* dHaug, long ldh);
+/* K2 is FP64 emulated on the 8-bit integer tensor cores (see cxb_gram_emulated) at sizes where that pays; the _ws form
+ * takes caller-owned scratch for the int8 slices of X, cxb_schur_dense_lmi_sym_gram_workspace(n, m) bytes (0: the sizes
+ * keep the DMMA Gram), and runs the DMMA Gram when dWork is nullptr. The plain form takes the slices from the
+ * stream-ordered pool for the call. */
+size_t cxb_schur_dense_lmi_sym_gram_workspace(int n, int m);
+int cxb_schur_dense_lmi_sym_gram_ws(void* stream, int n, int m, const double* dX, double* dHaug, long ldh, void* dWork,
+                                    size_t work_bytes);
+/* Lower triangle of H = X^T X (M x N, N <= M, ld ldh >= M) for X K x M column-major (ld ldx >= K, K % 16 == 0),
+ * FP64 emulated on the 8-bit integer tensor cores (Ozaki scheme, ozaki.cu: error bound and determinism there).
+ * dWork: cxb_gram_emulated_workspace(M, K) bytes; on return it holds the 8 int8 slices of X in the order the MMAs read
+ * them (128-row blocks, 32-byte k-steps, slices, 128 x 32-byte swizzled rows; ozaki.cu), followed by the M int32 column
+ * exponents. cxb_gram_slices writes that workspace only. */
+size_t cxb_gram_emulated_workspace(int M, long K);
+int cxb_gram_slices(void* stream, int M, long K, const double* dX, long ldx, void* dWork);
+int cxb_gram_emulated(void* stream, int M, int N, long K, const double* dX, long ldx, double* dH, long ldh,
+                      void* dWork);
 
 /* ---- entry-sparse LMI operators (MaxCut, Lovasz theta, ...; sparse_lmi.cu) -----------------------
  * A_i given by their non-zero entries (both triangles listed): entries offsets[i] .. offsets[i+1]-1 of
